@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Msamples/s through iq_tool's resample+shift+filter chain on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2] [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path (convert -> DC block -> multi-stage resample -> FIR ->
 convert) over one HBM-resident synthetic capture of the workload BASELINE.json's metric is
@@ -181,8 +181,10 @@ def run_reference(args):
         ch.process(raw[: 2 * min(n, 1 << 20)], threaded=threaded)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        ch.process(raw, threaded=threaded)
+        out = ch.process(raw, threaded=threaded)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out.view(np.uint8).reshape(-1, wl.config.out_bytes), wl.config.output_format)
     val = n * args.steps / dt / 1e6
     cores = 3 if threaded else 1
     line = {
@@ -330,7 +332,7 @@ def run_file_bench(args):
             k = min(left, len(block))
             f.write(block[:k])
             left -= k
-    steps = max(1, min(args.steps, 5))
+    steps = max(1, args.steps)
     try:
         sampler = ClockSampler(0)
         sampler.start()
@@ -343,6 +345,9 @@ def run_file_bench(args):
         dt = time.perf_counter() - p0
         clocks = sampler.stop(t0, time.time())
         out_bytes = os.path.getsize(dst)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, np.memmap(dst, dtype=np.uint8, mode="r").reshape(-1, cfg.out_bytes),
+                         cfg.output_format)
         value = n * steps / dt / 1e6
         cpu = None
         if not args.no_cpu_baseline:
@@ -376,6 +381,35 @@ def run_file_bench(args):
             "gpu_launches": None, "clocks": clocks}
     print(json.dumps(line))
     return 0
+
+
+DUMP_MAX_FRAMES = 1 << 21       # 2M frames: 16 MB of float32 I/Q (32 MB as float64) + 16 MB of float64 indices
+
+
+def dump_outputs(path, frames, output_format, rank=0, world=1):
+    """--dump-outputs: what the last timed step handed its caller, so two builds can be compared output for output.
+    `frames` holds the output as rows of one frame's bytes (a CUDA tensor, a numpy array or a memory-mapped file).
+    output.npy holds the frames as rows of float32 (float64 for 32-bit integer formats), output_index.npy their frame
+    indices and frames_out.npy the frame count; both are stored as float64, which holds every count exactly.  Above
+    DUMP_MAX_FRAMES a fixed, seeded sample of frames is stored.  With N > 1 every rank writes its own shard, with a
+    _rank<r> suffix."""
+    import numpy as np
+    import torch
+    from iq_tool_b200.configs import NUMPY_DTYPE
+    nf = frames.shape[0]
+    idx = np.arange(nf)
+    if nf > DUMP_MAX_FRAMES:
+        idx = np.sort(np.random.default_rng(20261020).choice(nf, DUMP_MAX_FRAMES, replace=False))
+        frames = frames[torch.from_numpy(idx).to(frames.device)] if torch.is_tensor(frames) else frames[idx]
+    raw = frames.cpu().numpy() if torch.is_tensor(frames) else np.asarray(frames)
+    dt = np.dtype(NUMPY_DTYPE[output_format])
+    vals = raw.view(dt).reshape(len(idx), -1)
+    vals = vals.astype(np.float32 if dt.kind == "f" or dt.itemsize < 4 else np.float64)
+    sfx = "" if world == 1 else f"_rank{rank}"
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, f"output{sfx}.npy"), vals)
+    np.save(os.path.join(path, f"output_index{sfx}.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, f"frames_out{sfx}.npy"), np.array([nf], dtype=np.float64))
 
 
 def pcie_probe(world, dev, nbytes=1 << 30, reps=3):
@@ -428,9 +462,11 @@ def main():
                          "multi-GPU configuration: time shards + the AGC peak all-gather); '' = off")
     ap.add_argument("--stage-leg", default="k1",
                     help="N = 1: a stage workload measured in the same run and reported as `stage_convert_shift` (k1: the "
-                         "stand-alone convert + NCO shift pass, north_star's >= 60 % of HBM target); '' = off")
+                         "stand-alone convert + NCO shift pass, north_star's >= 60 %% of HBM target); '' = off")
     ap.add_argument("--no-pcie-probe", action="store_true")
     ap.add_argument("--train-chunks", type=int, default=64, help="file workloads: reference chunks per chain call")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the output of the last timed step to DIR/*.npy (a seeded sample when large)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
@@ -478,6 +514,9 @@ def main():
     launches_per_step = chain.info().kernel_launches
     produced = run.produced
     value = world * n * args.steps / (ms / 1e3) / 1e6
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, run.out[: produced * cfg.out_bytes].view(produced, cfg.out_bytes), cfg.output_format,
+                     rank, world)
 
     # ---- sustained leg: the same step back to back for >= 2 s (power / clock behaviour of a long run) ----
     sustained = None

@@ -1,0 +1,2 @@
+/* agc.h — see stages.h.  TEST INFRASTRUCTURE. */
+#include "stages.h"

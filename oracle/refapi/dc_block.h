@@ -1,0 +1,2 @@
+/* dc_block.h — see stages.h.  TEST INFRASTRUCTURE. */
+#include "stages.h"

@@ -1,0 +1,2 @@
+/* filter.h — see stages.h.  TEST INFRASTRUCTURE. */
+#include "stages.h"

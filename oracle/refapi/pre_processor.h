@@ -1,0 +1,2 @@
+/* pre_processor.h — see stages.h.  TEST INFRASTRUCTURE. */
+#include "stages.h"

@@ -1,0 +1,2 @@
+/* resampler.h — see stages.h.  TEST INFRASTRUCTURE. */
+#include "stages.h"

@@ -1,0 +1,2 @@
+/* sample_convert.h — see stages.h.  TEST INFRASTRUCTURE. */
+#include "stages.h"
