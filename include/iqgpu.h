@@ -216,9 +216,38 @@ int  iqgpu_chain_get_arb_taps(iqgpu_chain *c, float *taps, uint32_t capacity, ui
  *      `out_first_frame` receives the absolute output-frame index of the first output the chain
  *      will emit.  To reproduce the single-stream result a shard seeks to
  *      (shard_start - halo), processes from there and drops the outputs that precede
- *      shard_start (their count is closed form too); halo from iqgpu_chain_halo_frames. ------ */
+ *      shard_start (their count is closed form too); halo from iqgpu_chain_halo_frames.
+ *      A post-resample FFT filter (every decimating chain with one) is positioned on the single
+ *      stream's blocks: R(first_frame) mod n resampled frames (R = resampler outputs, n = block)
+ *      wait as zeros for a full block and `out_first_frame` = floor(R(first_frame) / n) * n.  A
+ *      pre-resample FFT filter (interpolating or no_resample chains) is refused.  The RMS AGC
+ *      starts from its reset state; iqgpu_chain_agc_rms_resume_device hands the state over.
+ *      The halo covers the resampler's history, a FIR's taps, two FFT blocks (2n / ratio frames)
+ *      and 16 time constants of the DC blocker (the only approximate term). ------------------- */
 int  iqgpu_chain_seek(iqgpu_chain *c, uint64_t first_frame, uint64_t *out_first_frame);
 int  iqgpu_chain_halo_frames(iqgpu_chain *c, size_t *halo_frames);
+/* closed form: chain output frames after `frames_in` input frames since a restart — the resampler's
+ * count, block-quantised by an FFT filter.  The output index of a capture frame, for shard plans. */
+int  iqgpu_chain_outputs_after(iqgpu_chain *c, uint64_t frames_in, uint64_t *frames_out);
+
+/* ---- sharded RMS AGC (liquid agc_crcf, a nonlinear per-sample recurrence in {g, y2'}): each
+ *      shard runs its halo and shard from the reset state at its lead with ONE process_device call
+ *      (one sub-train: raise the subtrain_frames option), then world-1 rounds follow, in each of
+ *      which every rank publishes its end state (8 bytes) and rank g >= 1 resumes from rank g-1's.
+ *      After round k ranks 0..k are exact.
+ *        agc_rms_state_device   copies the end state {g, y2'} (two floats) to device memory on `stream`;
+ *        agc_rms_resume_device  re-runs the AGC of the last call from output frame `first_output` (the
+ *                               shard's first owned output) with the state at `dev_state`, rewrites
+ *                               and re-converts into `dev_out` (the last call's output buffer) only the
+ *                               range that changed, and writes 1 / 0 to `dev_changed` (optional, device
+ *                               int) when the end state did / did not change.  A resume at the same
+ *                               frame from the same state as the previous one does nothing on the device;
+ *                               all of it is queued on `stream` without a host synchronisation;
+ *        get_agc_rms_state      reads {g, y2'} to the host (synchronises). ----------------------------- */
+int  iqgpu_chain_agc_rms_state_device(iqgpu_chain *c, float *dev_state, void *cuda_stream);
+int  iqgpu_chain_agc_rms_resume_device(iqgpu_chain *c, size_t first_output, const float *dev_state, void *dev_out,
+                                       size_t out_capacity_bytes, int *dev_changed, void *cuda_stream);
+int  iqgpu_chain_get_agc_rms_state(iqgpu_chain *c, float *g, float *y2);
 
 /* ---- sharded digital AGC (SURVEY.md 8(e)): the one exchange step of a time-sharded run.
  *      The digital AGC (src/agc.c:105-222) is a scalar state machine over per-chunk peaks, so a

@@ -11,6 +11,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -239,6 +240,13 @@ struct iqgpu_chain {
     size_t agc_quiet_bytes = 0;
     void* d_agc_ws = nullptr;           // RMS-AGC time-parallel workspace (block end states + sweep flags)
     size_t agc_ws_bytes = 0;
+    // RMS AGC of the last call when it was one sub-train: input, parameters and (in d_agc_scratch / d_agc_ws) output and
+    // checkpoints, which iqgpu_chain_agc_rms_resume_device re-runs from a later start state (time shards)
+    const float2* rms_src = nullptr;
+    size_t rms_n = 0;
+    PostParams rms_qp{};
+    bool rms_ready = false, rms_fresh = false;
+    AgcRmsResume* d_rms_resume = nullptr;
     // streams: s_in = pre output; s_stage[d] = output of executed halfband stage d; s_rs = resampler
     // output; s_f = post-filter output (or pre-filter output when the filter is pre-resample)
     DevStream s_in, s_pref, s_arb_in, s_rs, s_f;
@@ -337,7 +345,7 @@ iqgpu_chain::~iqgpu_chain()
     cudaFree(d_lut); cudaFree(d_dc_carry); cudaFree(d_dc_ref); cudaFree(d_run_sums); cudaFree(d_run_start); cudaFree(d_scan_ws); cudaFree(d_bank);
     cudaFree(d_fir_taps); cudaFree(d_fft_H); cudaFree(d_fft_tw); cudaFree(d_fft_scratch); cudaFree(d_agc); cudaFree(d_seg_start);
     cudaFree(d_seg_peak); cudaFree(d_seg_gain); cudaFree(d_agc_scratch); cudaFree(d_agc_ws);
-    cudaFree(d_iq_state); cudaFree(d_iq_probe); cudaFree(d_agc_quiet);
+    cudaFree(d_iq_state); cudaFree(d_iq_probe); cudaFree(d_agc_quiet); cudaFree(d_rms_resume);
     if (h_iq_state) cudaFreeHost(h_iq_state);
     if (ev_iq) cudaEventDestroy(ev_iq);
     if (ev_iq_probe) cudaEventDestroy(ev_iq_probe);
@@ -371,6 +379,17 @@ static bool filter_is_fft(const FilterPlan& f)
 static bool filter_is_fir(const FilterPlan& f)
 {
     return f.impl == IQGPU_FILTER_IMPL_FIR_SYM || f.impl == IQGPU_FILTER_IMPL_FIR_ASYM;
+}
+
+// chain output frames after `k` input frames since a restart: the resampler's count (pipeline.c:523), block-quantised by an
+// FFT filter (filter.c:491-526).  The quantisation carries its remainder from chunk to chunk, so the sum of count_outputs'
+// per-chunk counts from a restart is this closed form at every chunk boundary.
+static uint64_t chain_outputs_after(const iqgpu_chain* c, uint64_t k)
+{
+    if (!filter_is_fft(c->filt)) return resampler_outputs_after(c->rs, k);
+    const uint64_t B = c->filt.block;
+    if (!c->filt.post_resample) return resampler_outputs_after(c->rs, k / B * B);
+    return resampler_outputs_after(c->rs, k) / B * B;
 }
 
 size_t iqgpu_chain::max_out_for(size_t n) const
@@ -588,6 +607,7 @@ int iqgpu_chain::reset_state(bool keep_fft_remainder)
     n_in = 0; n_nco_post = 0; n_out = 0; fft_rem = keep;
     iq_last_attempt_s = -1e18;              // the sample clock restarts with the stream
     fft_rem_carry = pre_fft ? keep : 0;
+    rms_ready = false;
     if (plan_only || !buffers_ready) return IQGPU_OK;
     CK(cudaSetDevice(device));
     cudaStream_t S = last_stream ? last_stream : stream;
@@ -751,6 +771,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
     const size_t total_out = seg[n_chunks];
     launches = 0;
     fir_wrote_output = false;
+    rms_ready = false;
     if (iq_optimize) { int rc_iq = iq_sync_state(); if (rc_iq) return rc_iq; }      // factors the last train's passes left
 
     // ---------------- K1: pre-processor ----------------
@@ -1086,6 +1107,7 @@ int iqgpu_chain::run_back(void* d_outp, size_t skip_chunks, size_t* out_frames, 
             CK(launch_agc_rms(post_src, post_n, qp, d_agc, y, d_agc_ws, st));
             CK(launch_post(y, post_n, qp, nullptr, 0, nullptr, 1, tap2, d_outp, st));
             launches += 2;
+            rms_src = post_src; rms_n = post_n; rms_qp = qp; rms_ready = true; rms_fresh = true;
         } else {
             CK(launch_post(post_src, post_n, qp, nullptr, 0, nullptr, 0, tap2, d_outp, st));
             launches++;
@@ -1455,6 +1477,7 @@ int iqgpu_chain_process_device(iqgpu_chain* c, const void* dev_raw_in, size_t n_
     }
     c->launches = launches + c->prepass_launches;   // pre-pass kernels that really ran on the second stream
     c->prepass_launches = 0;
+    if (subs.size() != 1) c->rms_ready = false;     // an RMS-AGC resume needs the whole call in one sub-train
     *out_frames = total;
     return IQGPU_OK;
 }
@@ -1538,7 +1561,7 @@ int iqgpu_chain_agc_advance_device(iqgpu_chain* c, const float* dev_peaks, uint6
     if (rc) return rc;
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
     if (c->last_stream && st != c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
-    // the chunks' output frame counts are closed form (pipeline.c:523 via count_outputs' arithmetic)
+    // the chunks' output frame counts are closed form (pipeline.c:523 and the FFT filter's blocks, chain_outputs_after)
     const size_t nch = (size_t)((n_frames + c->chunk_frames - 1) / c->chunk_frames);
     const uint32_t* d_seg = nullptr;
     for (const auto& t : c->prefix_tabs)
@@ -1553,11 +1576,11 @@ int iqgpu_chain_agc_advance_device(iqgpu_chain* c, const float* dev_peaks, uint6
             if (!c->ev_seg[sl]) CK(cudaEventCreateWithFlags(&c->ev_seg[sl], cudaEventDisableTiming));
         } else if (c->ev_seg[sl]) CK(cudaEventSynchronize(c->ev_seg[sl]));
         uint32_t* seg = c->seg_pin[sl];
-        uint64_t before = resampler_outputs_after(c->rs, first_frame);
+        uint64_t before = chain_outputs_after(c, first_frame);
         seg[0] = 0;
         for (size_t k = 0; k < nch; k++) {
             const uint64_t end = std::min<uint64_t>(first_frame + n_frames, first_frame + (uint64_t)(k + 1) * c->chunk_frames);
-            const uint64_t after = resampler_outputs_after(c->rs, end);
+            const uint64_t after = chain_outputs_after(c, end);
             seg[k + 1] = seg[k] + (uint32_t)(after - before);       // the scan uses differences only: wrap-around is harmless
             before = after;
         }
@@ -1633,6 +1656,61 @@ int iqgpu_chain_set_agc_state(iqgpu_chain* c, const iqgpu_agc_state* s)
     a.last_strong = s->last_strong_s;
     CK(cudaMemcpyAsync(c->d_agc, &a, sizeof(a), cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));
+    return IQGPU_OK;
+}
+
+// ---- sharded RMS AGC: the end state {g, y2'} of a shard and the resume of its successor from it ----
+int iqgpu_chain_agc_rms_state_device(iqgpu_chain* c, float* dev_state, void* cuda_stream)
+{
+    if (!c || !dev_state) return fail(IQGPU_EINVAL, "null argument");
+    if (c->plan_only) return fail(IQGPU_ENODEVICE, "plan-only chain");
+    if (c->agc_mode != 2) return fail(IQGPU_EINVAL, "the chain has no RMS AGC");
+    CK(cudaSetDevice(c->device));
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
+    if (c->last_stream && st != c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
+    static_assert(offsetof(AgcState, rms_y2) == offsetof(AgcState, rms_g) + sizeof(float), "{g, y2'} must be adjacent");
+    CK(cudaMemcpyAsync(dev_state, &c->d_agc->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return IQGPU_OK;
+}
+
+int iqgpu_chain_agc_rms_resume_device(iqgpu_chain* c, size_t first_output, const float* dev_state, void* dev_out,
+                                      size_t out_capacity_bytes, int* dev_changed, void* cuda_stream)
+{
+    if (!c) return fail(IQGPU_EINVAL, "null chain");
+    if (c->plan_only) return fail(IQGPU_ENODEVICE, "plan-only chain");
+    if (c->agc_mode != 2) return fail(IQGPU_EINVAL, "the chain has no RMS AGC");
+    if (!dev_state || !dev_out) return fail(IQGPU_EINVAL, "null buffer");
+    if (!c->rms_ready)
+        return fail(IQGPU_EINVAL, "nothing to resume: the last call must be a process_device call that fit one sub-train "
+                                  "(raise the subtrain_frames option)");
+    if (c->rms_n * c->out_bps > out_capacity_bytes) return fail(IQGPU_ECAPACITY, "output buffer too small");
+    CK(cudaSetDevice(c->device));
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
+    if (c->last_stream && st != c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
+    c->last_stream = st;
+    if (first_output >= c->rms_n) {            // nothing of the call lies behind the resume point
+        if (dev_changed) CK(cudaMemsetAsync(dev_changed, 0, sizeof(int), st));
+        return IQGPU_OK;
+    }
+    if (!c->d_rms_resume) CK(cudaMalloc(&c->d_rms_resume, sizeof(AgcRmsResume)));
+    CK(launch_agc_rms_resume(c->rms_src, c->rms_n, c->rms_qp, c->d_agc, c->d_agc_scratch, c->d_agc_ws, first_output,
+                             reinterpret_cast<const float2*>(dev_state), c->d_rms_resume, c->rms_fresh, dev_changed, st));
+    c->rms_fresh = false;
+    CK(launch_convert_range(c->d_agc_scratch, c->d_rms_resume, c->cfg.output_format, dev_out, st));
+    c->launches += 2;
+    return IQGPU_OK;
+}
+
+int iqgpu_chain_get_agc_rms_state(iqgpu_chain* c, float* g, float* y2)
+{
+    if (!c || !g || !y2) return fail(IQGPU_EINVAL, "null argument");
+    if (c->plan_only) return fail(IQGPU_ENODEVICE, "plan-only chain");
+    CK(cudaSetDevice(c->device));
+    if (c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
+    CK(cudaStreamSynchronize(c->stream));
+    AgcState a{};
+    CK(cudaMemcpy(&a, c->d_agc, sizeof(a), cudaMemcpyDeviceToHost));
+    *g = a.rms_g; *y2 = a.rms_y2;
     return IQGPU_OK;
 }
 
@@ -1737,6 +1815,7 @@ int iqgpu_chain_process(iqgpu_chain* c, const void* raw_in, size_t n_frames, con
     CK(cudaStreamSynchronize(c->d2h));
     CK(cudaStreamSynchronize(c->stream));
     c->launches = launches;
+    c->rms_ready = false;                            // the output went through the staging slots, not a caller's buffer
     *out_frames = total;
     return IQGPU_OK;
 }
@@ -1787,23 +1866,44 @@ int iqgpu_chain_halo_frames(iqgpu_chain* c, size_t* halo)
     if (filter_is_fir(c->filt) && c->filt.post_resample)
         h += (size_t)std::ceil((double)c->filt.taps.size() / (double)c->ratio) + ((size_t)1 << c->rs.num_halfband);
     else if (filter_is_fir(c->filt)) h += c->filt.taps.size();
+    // post-resample FFT filter: output block b reads the resampled samples [(b-1)n, (b+1)n), so the block before the first one
+    // a shard owns must lie behind the resampler's exact region: 2n output-rate samples = 2n/ratio input frames
+    if (filter_is_fft(c->filt) && c->filt.post_resample)
+        h += (size_t)std::ceil(2.0 * (double)c->filt.block / (double)c->ratio) + ((size_t)1 << c->rs.num_halfband);
     // DC blocker: infinite memory; 16 time constants leave e^-16 ~ 1e-7 of the integrator state
     if (c->dc.enable) h += (size_t)std::ceil(16.0 / (double)c->dc.alpha);
     *halo = h;
     return IQGPU_OK;
 }
 
+int iqgpu_chain_outputs_after(iqgpu_chain* c, uint64_t frames_in, uint64_t* frames_out)
+{
+    if (!c || !frames_out) return fail(IQGPU_EINVAL, "null argument");
+    *frames_out = chain_outputs_after(c, frames_in);
+    return IQGPU_OK;
+}
+
 int iqgpu_chain_seek(iqgpu_chain* c, uint64_t first_frame, uint64_t* out_first_frame)
 {
     if (!c) return fail(IQGPU_EINVAL, "null chain");
-    if (filter_is_fft(c->filt)) return fail(IQGPU_EINVAL, "seek is not supported with an FFT filter (block alignment)");
-    if (c->agc_mode == 2) return fail(IQGPU_EINVAL, "seek is not supported with the RMS AGC (not shardable, SURVEY 8(e))");
+    if (filter_is_fft(c->filt) && !c->filt.post_resample)
+        return fail(IQGPU_EINVAL, "seek is not supported with a pre-resample FFT filter: its blocks are cut from the input "
+                                  "stream behind the remainder that filter_reset carries into the next stream (F5), a "
+                                  "position a shard cannot reproduce; only interpolating or no_resample chains filter there");
     int rc = c->plan_only ? IQGPU_OK : c->ensure_buffers();
     if (rc) return rc;
     rc = c->reset_state();
     if (rc) return rc;
     c->n_in = first_frame;
-    const uint64_t o = resampler_outputs_after(c->rs, first_frame);
+    const uint64_t r = resampler_outputs_after(c->rs, first_frame);
+    uint64_t o = r;
+    if (filter_is_fft(c->filt)) {
+        // the single stream cuts the filter's blocks at multiples of n from its start: R(first_frame) mod n resampled frames
+        // wait for a full block here.  They are halo (dropped by the caller), so they may read as the zeros reset_state
+        // left in the stream's history; the blocks that follow are those of the single stream.
+        c->fft_rem = (uint32_t)(r % c->filt.block);
+        o = r - c->fft_rem;
+    }
     c->n_out = o;
     c->n_nco_post = o;
     if (out_first_frame) *out_first_frame = o;

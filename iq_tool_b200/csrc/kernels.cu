@@ -1217,7 +1217,10 @@ __device__ __forceinline__ double agc_normal_f2d(unsigned bits)
     return __hiloint2double((int)(((mag >> 3) + 0x38000000u) | (bits & 0x80000000u)), (int)(mag << 29));
 }
 
-// generic step (any operand: zero / subnormal / huge): the rare fall-back of agc_rms_step, kept out of line
+// generic step (any operand: zero / subnormal / huge): the rare fall-back of agc_rms_step, kept out of line.
+// V: one instance per kernel (0: agc_rms_parallel_kernel, 1: agc_rms_resume_kernel).  An out-of-line function shared by two
+// kernels is compiled for both callers, and the parallel kernel then re-derives the table's shared-window address in its loop.
+template <int V>
 __device__ __noinline__ AgcRec agc_rms_step_slow(float ay2, float mha, double oma, const AgcLogEntry* __restrict__ ltab, AgcRec r)
 {
     const float y2n = (float)fma(oma, r.y2pd, (double)ay2);
@@ -1239,6 +1242,7 @@ __device__ __noinline__ AgcRec agc_rms_step_slow(float ay2, float mha, double om
 // of the stream, so the step is written for latency: straight-line code for the operand ranges that occur (everything
 // normal, y2' > 1e-6, |t| <= 0.125), conversions by integer arithmetic where they are exact, the three range checks folded
 // into one predicate that is tested once at the end and sends the rare other cases through agc_rms_step_slow.
+template <int V>
 __device__ __forceinline__ float2 agc_rms_step(float2 v, size_t i, const PostParams& p, const float* __restrict__ lut,
                                                const AgcLogEntry* __restrict__ ltab, uint32_t ltab_s,
                                                float alpha, double oma, float mha, AgcRec& r)
@@ -1262,7 +1266,7 @@ __device__ __forceinline__ float2 agc_rms_step(float2 v, size_t i, const PostPar
     if (ok_a && ok_t && y2n > 1e-6f) {
         r.g = gn; r.y2p = y2n; r.y2pd = agc_normal_f2d(yb);
     } else {
-        r = agc_rms_step_slow(ay2, mha, oma, ltab, r);
+        r = agc_rms_step_slow<V>(ay2, mha, oma, ltab, r);
     }
     return make_float2(yr, yi);
 }
@@ -1285,6 +1289,7 @@ __device__ __forceinline__ void st_global_256(float2* p, float2 a, float2 b, flo
                  :: "l"(p), "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y), "f"(c.x), "f"(c.y), "f"(d.x), "f"(d.y) : "memory");
 }
 constexpr int AGC_CK = 256;
+template <int V = 0>
 __device__ __forceinline__ bool agc_rms_block(const float2* __restrict__ x, size_t i0, size_t i1, const PostParams& p,
                                               const float* __restrict__ lut, const AgcLogEntry* __restrict__ ltab,
                                               float& g, float& y2p, float2* __restrict__ y, float2* __restrict__ ck, bool compare,
@@ -1329,7 +1334,7 @@ __device__ __forceinline__ bool agc_rms_block(const float2* __restrict__ x, size
         for (int k = 0; k < 8; k++) v[k] = nx[k];
         if (i + 16 <= i1) load8(i + 8);
 #pragma unroll
-        for (int k = 0; k < 8; k++) v[k] = agc_rms_step(v[k], i + k, p, lut, ltab, ltab_s, alpha, oma, mha, r);
+        for (int k = 0; k < 8; k++) v[k] = agc_rms_step<V>(v[k], i + k, p, lut, ltab, ltab_s, alpha, oma, mha, r);
         if (wide) {
             st_global_256(y + i, v[0], v[1], v[2], v[3]);
             st_global_256(y + i + 4, v[4], v[5], v[6], v[7]);
@@ -1338,7 +1343,7 @@ __device__ __forceinline__ bool agc_rms_block(const float2* __restrict__ x, size
             for (int k = 0; k < 8; k++) y[i + k] = v[k];
         }
     }
-    for (; i < i1; i++) y[i] = agc_rms_step(x[i], i, p, lut, ltab, ltab_s, alpha, oma, mha, r);
+    for (; i < i1; i++) y[i] = agc_rms_step<V>(x[i], i, p, lut, ltab, ltab_s, alpha, oma, mha, r);
     g = r.g; y2p = r.y2p;
     return false;
 }
@@ -1385,6 +1390,93 @@ __global__ void __launch_bounds__(AGC_RMS_THREADS) agc_rms_parallel_kernel(const
         }
     }
     if (b == nblocks - 1) { const float2 f = fin[b]; st->rms_g = f.x; st->rms_y2 = f.y; }
+}
+
+__device__ __forceinline__ bool same_bits(float2 a, float2 b)
+{
+    return __float_as_uint(a.x) == __float_as_uint(b.x) && __float_as_uint(a.y) == __float_as_uint(b.y);
+}
+
+// Resume of the last agc_rms_parallel_kernel run over the same samples from a new start state at sample `first` (a time
+// shard taking over the end state of the shard in front of it).  At that run's fixed point every block's checkpoint row
+// holds the exact trajectory and fin[] the block end states, so this is one more level of the same guess-and-verify
+// scheme: block k (the one holding `first`) runs from `first` — a scalar head up to its next checkpoint, then the usual
+// block walk comparing against the old checkpoints — and stops where the new trajectory meets the old one; a later block
+// runs again only when its predecessor's end state changed (the sweep logic of the parallel kernel, blocks below k idle).
+// The grid is the parallel kernel's (its occupancy sized the workspace plan): at most its 72 registers, 7 CTAs per SM.
+__global__ void __launch_bounds__(AGC_RMS_THREADS, 7) agc_rms_resume_kernel(const float2* __restrict__ x, size_t n, PostParams p,
+                                                                          AgcState* __restrict__ st, float2* __restrict__ y,
+                                                                          size_t B, unsigned nblocks, float2* __restrict__ fin,
+                                                                          unsigned* __restrict__ flags, float2* __restrict__ ckpt,
+                                                                          unsigned ck_per_block, size_t first,
+                                                                          const float2* __restrict__ start_state,
+                                                                          AgcRmsResume* __restrict__ rr, int fresh,
+                                                                          int* __restrict__ changed)
+{
+    cg::grid_group grid = cg::this_grid();
+    __shared__ float lut[1024];
+    __shared__ AgcLogEntry ltab[AGC_LOG_N];
+    const unsigned b = blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned k = (unsigned)min((size_t)nblocks, first / B);
+    const bool active = b < nblocks && b >= k;
+    const size_t i0 = (size_t)b * B, i1 = (i0 + B < n) ? i0 + B : n;
+    // everything the resume overwrites is read before the first grid-wide barrier
+    const float2 s_new = *start_state;
+    const bool same = !fresh && rr->valid && rr->last_first == first && same_bits(rr->last_start, s_new);
+    const float2 old_end = make_float2(st->rms_g, st->rms_y2);
+    float2 start = (b == k) ? s_new : (active ? fin[b - 1] : make_float2(0.f, 0.f));
+    grid.sync();
+    if (b == 0) { rr->last_start = s_new; rr->last_first = first; rr->valid = 1u; rr->lo = first; rr->hi = first; }
+    if (same) {                        // same start as the previous resume: the trajectory in memory is already this one
+        if (b == 0 && changed) *changed = 0;
+        return;
+    }
+    if (p.nco_enable)
+        for (int i = threadIdx.x; i < 1024; i += blockDim.x) lut[i] = p.nco_table[i];
+    for (int i = threadIdx.x; i < AGC_LOG_N; i += blockDim.x) ltab[i] = agc_log_tab_c[i];
+    __syncthreads();
+    float2* ck = ckpt + (size_t)b * ck_per_block;
+    const uint32_t opaque_zero = (uint32_t)(B >> 48);
+    bool run = active && b == k, ran = false;
+    for (unsigned it = 0; it <= nblocks; it++) {
+        if (run) {
+            float g = start.x, y2p = start.y;
+            bool merged = false;
+            // block k (it runs once): the head [first, c) up to its next checkpoint, then [c, i1); other blocks: [i0, i1).
+            // One call site of the block walk: a second inlined copy would not fit the register budget above.
+            size_t a = i0, c = i0;
+            if (b == k) {
+                a = first;
+                c = i0 + (first - i0 + AGC_CK - 1) / AGC_CK * AGC_CK;
+                if (c > i1) c = i1;
+            }
+#pragma unroll 1
+            for (int part = (a < c) ? 0 : 1; part < 2 && !merged; part++) {
+                const size_t s0 = part ? c : a, s1 = part ? i1 : c;
+                if (s0 < s1)
+                    merged = agc_rms_block<1>(x, s0, s1, p, lut, ltab, g, y2p, y, part ? ck + (c - i0) / AGC_CK : &rr->ck_scratch,
+                                           part == 1, opaque_zero);
+            }
+            if (!merged) fin[b] = make_float2(g, y2p);
+            ran = true;
+        }
+        grid.sync();
+        run = false;
+        if (active && b > k) {
+            const float2 ns = fin[b - 1];
+            run = !same_bits(ns, start);
+            start = ns;
+        }
+        if (run) flags[it] = 1u;
+        grid.sync();
+        if (flags[it] == 0u) break;
+    }
+    if (ran) atomicMax(&rr->hi, (unsigned long long)i1);     // a merged run rewrote less: re-converting the rest is harmless
+    if (b == nblocks - 1) {
+        const float2 f = fin[b];
+        st->rms_g = f.x; st->rms_y2 = f.y;
+        if (changed) *changed = same_bits(f, old_end) ? 0 : 1;
+    }
 }
 
 // cf32 -> output sample formats, reference sample_convert.c:40-73, 213-306
@@ -1744,6 +1836,54 @@ cudaError_t launch_post(const float2* x, size_t n, const PostParams& p, const ui
 #undef CALL
     return cudaGetLastError();
 }
+cudaError_t launch_agc_rms_resume(const float2* x, size_t n, const PostParams& p, AgcState* state, float2* y, void* ws,
+                                  size_t first, const float2* start, AgcRmsResume* rr, bool fresh, int* changed,
+                                  cudaStream_t st)
+{
+    if (n == 0 || first >= n) return cudaErrorInvalidValue;
+    size_t B; unsigned nb;
+    agc_rms_plan(n, p.agc_alpha, B, nb);        // the plan of the call being resumed: its workspace layout
+    float2* fin = reinterpret_cast<float2*>(ws);
+    unsigned* flags = reinterpret_cast<unsigned*>(fin + nb);
+    cudaError_t e = cudaMemsetAsync(flags, 0, ((size_t)nb + 2) * sizeof(unsigned), st);
+    if (e != cudaSuccess) return e;
+    PostParams pp = p;
+    float2* ckpt = reinterpret_cast<float2*>(flags + (((size_t)nb + 2 + 1) & ~(size_t)1));
+    unsigned ckb = (unsigned)((B + AGC_CK - 1) / AGC_CK);
+    int fr = fresh ? 1 : 0;
+    void* args[] = {(void*)&x, (void*)&n, (void*)&pp, (void*)&state, (void*)&y, (void*)&B, (void*)&nb, (void*)&fin, (void*)&flags,
+                    (void*)&ckpt, (void*)&ckb, (void*)&first, (void*)&start, (void*)&rr, (void*)&fr, (void*)&changed};
+    const unsigned grid = (nb + AGC_RMS_THREADS - 1) / AGC_RMS_THREADS;
+    return cudaLaunchCooperativeKernel((void*)agc_rms_resume_kernel, dim3(grid), dim3(AGC_RMS_THREADS), args, 0, st);
+}
+
+template <int FMT>
+__global__ void __launch_bounds__(256) convert_range_kernel(const float2* __restrict__ y, const AgcRmsResume* __restrict__ rr,
+                                                            void* __restrict__ out, bool vec_out)
+{
+    const size_t lo = rr->lo, hi = rr->hi;
+    if (lo >= hi) return;
+    // from the group of four holding `lo`: the frames in front of it are converted again to the same bits
+    const size_t stride = (size_t)gridDim.x * blockDim.x * 4;
+    for (size_t i = (lo & ~(size_t)3) + ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * 4; i < hi; i += stride) {
+        float2 v[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) v[k] = (i + k < hi) ? y[i + k] : make_float2(0.f, 0.f);
+        store_out4<FMT>(out, i, hi, v, vec_out);
+    }
+}
+
+cudaError_t launch_convert_range(const float2* y, const AgcRmsResume* rr, int format, void* out, cudaStream_t st)
+{
+    // a fixed grid striding over a range only the device knows; an unchanged resume leaves it empty (a few us)
+    const int grid = 148 * 2;
+    const bool vo = aligned16(out);
+#define CALL(F) convert_range_kernel<F><<<grid, 256, 0, st>>>(y, rr, out, vo)
+    DISPATCH_FMT(format, CALL)
+#undef CALL
+    return cudaGetLastError();
+}
+
 cudaError_t launch_convert_out(const float2* x, size_t n, int format, void* out, cudaStream_t st)
 {
     PostParams p{};

@@ -128,6 +128,23 @@ cudaError_t launch_agc_digital_scan(const uint32_t* seg_start, size_t nseg, cons
 size_t agc_rms_workspace_bytes(size_t n, float alpha);
 cudaError_t launch_agc_rms(const float2* x, size_t n, const PostParams& p, AgcState* state, float2* y, void* ws,
                            cudaStream_t st);
+// Resume of the last launch_agc_rms call (same x, n, p, y, ws — the workspace still holds that call's block end states and
+// checkpoints): the recurrence re-runs from sample `first` with the start state *start ({g, y2'}, device), stops where its
+// trajectory meets the previous one bit for bit, and leaves y and *state exactly as one call from that state at `first`
+// would have.  A resume at the same sample and from the same state as the previous resume (rr->last_first / last_start;
+// `fresh` = no resume since the call) does nothing.  rr receives the rewritten range [lo, hi) of y; *changed (optional) =
+// whether the end state changed.
+struct AgcRmsResume {
+    float2 last_start;
+    float2 ck_scratch;              // checkpoint slot of the unaligned head of the resumed block (never compared)
+    unsigned long long last_first, lo, hi;
+    unsigned valid, pad;
+};
+cudaError_t launch_agc_rms_resume(const float2* x, size_t n, const PostParams& p, AgcState* state, float2* y, void* ws,
+                                  size_t first, const float2* start, AgcRmsResume* rr, bool fresh, int* changed,
+                                  cudaStream_t st);
+// convert y[rr->lo, rr->hi) to `format` into out (the range a resume rewrote; both bounds read on the device)
+cudaError_t launch_convert_range(const float2* y, const AgcRmsResume* rr, int format, void* out, cudaStream_t st);
 // y_cf32 (optional tap) and converted out
 cudaError_t launch_post(const float2* x, size_t n, const PostParams& p, const uint32_t* seg_start,
                         size_t nseg, const float* seg_gain, int nco_already_applied, float2* tap_cf32,

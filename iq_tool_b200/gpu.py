@@ -128,6 +128,10 @@ def _load() -> C.CDLL:
     lib.iqgpu_chain_process_device_finish.argtypes = [vp, sz, vp, sz, C.POINTER(sz), u32p, vp]
     lib.iqgpu_chain_pending_chunk_peaks_device.argtypes = [vp, sz, vp, sz, C.POINTER(sz), vp]
     lib.iqgpu_chain_agc_advance_device.argtypes = [vp, vp, C.c_uint64, C.c_uint64, vp]
+    lib.iqgpu_chain_outputs_after.argtypes = [vp, C.c_uint64, C.POINTER(C.c_uint64)]
+    lib.iqgpu_chain_agc_rms_state_device.argtypes = [vp, vp, vp]
+    lib.iqgpu_chain_agc_rms_resume_device.argtypes = [vp, sz, vp, vp, sz, vp, vp]
+    lib.iqgpu_chain_get_agc_rms_state.argtypes = [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     lib.iqgpu_chain_get_agc_state.argtypes = [vp, C.POINTER(AgcStateC)]
     lib.iqgpu_chain_set_agc_state.argtypes = [vp, C.POINTER(AgcStateC)]
     lib.iqgpu_agc_digital_initial_state.argtypes = [C.POINTER(AgcStateC)]
@@ -164,7 +168,8 @@ def _load() -> C.CDLL:
                  "iqgpu_chain_process_device_begin", "iqgpu_chain_pending_chunk_peaks",
                  "iqgpu_chain_process_device_finish", "iqgpu_chain_get_agc_state", "iqgpu_chain_set_agc_state",
                  "iqgpu_chain_pending_chunk_peaks_device", "iqgpu_chain_agc_advance_device",
-                 "iqgpu_agc_digital_advance", "iqgpu_convert_block_to_cf32",
+                 "iqgpu_agc_digital_advance", "iqgpu_convert_block_to_cf32", "iqgpu_chain_outputs_after",
+                 "iqgpu_chain_agc_rms_state_device", "iqgpu_chain_agc_rms_resume_device", "iqgpu_chain_get_agc_rms_state",
                  "iqgpu_convert_cf32_to_block", "iqgpu_iq_optimize"):
         getattr(lib, name).restype = C.c_int
     return lib
@@ -269,6 +274,32 @@ class Chain:
         o = C.c_uint64(0)
         _check(lib.iqgpu_chain_resampler_outputs_after(self._h, frames_in, C.byref(o)))
         return o.value
+
+    def outputs_after(self, frames_in: int) -> int:
+        """Closed form: chain output frames after `frames_in` input frames since a restart (the resampler's count,
+        block-quantised by an FFT filter): the output index of a capture frame."""
+        o = C.c_uint64(0)
+        _check(lib.iqgpu_chain_outputs_after(self._h, frames_in, C.byref(o)))
+        return o.value
+
+    # ---- sharded RMS AGC: end-state hand-over between time shards (include/iqgpu.h) ----
+    def agc_rms_state_device(self, dev_state_ptr: int, stream: int = 0) -> None:
+        """Copy the RMS AGC's state {g, y2'} (two float32) to device memory, asynchronously on `stream`."""
+        _check(lib.iqgpu_chain_agc_rms_state_device(self._h, dev_state_ptr, C.c_void_p(stream) if stream else None))
+
+    def agc_rms_resume_device(self, first_output: int, dev_state_ptr: int, dev_out_ptr: int, out_capacity_bytes: int,
+                              dev_changed_ptr: int = 0, stream: int = 0) -> None:
+        """Re-run the RMS AGC of the last process_device call from output frame `first_output` with the state at
+        `dev_state_ptr` and re-convert the outputs that changed into `dev_out_ptr` (that call's output buffer).
+        `dev_changed_ptr` (optional, int32 in device memory) receives whether the end state changed."""
+        _check(lib.iqgpu_chain_agc_rms_resume_device(self._h, first_output, dev_state_ptr, dev_out_ptr, out_capacity_bytes,
+                                                     dev_changed_ptr or None, C.c_void_p(stream) if stream else None))
+
+    def get_agc_rms_state(self):
+        """(g, y2') of the RMS AGC, read to the host."""
+        g, y2 = C.c_float(0), C.c_float(0)
+        _check(lib.iqgpu_chain_get_agc_rms_state(self._h, C.byref(g), C.byref(y2)))
+        return g.value, y2.value
 
     # ---- sharded digital AGC: process_device split at the peak exchange (include/iqgpu.h) ----
     def process_device_begin(self, dev_in_ptr: int, n_frames: int, stream: int = 0) -> None:

@@ -4,14 +4,21 @@ A capture of `total_frames` input frames is cut into contiguous shards whose sta
 multiples of the reference chunk (16384 frames, include/constants.h:123), so that chunk
 boundaries — and with them the per-chunk digital-AGC blocks — are those of the single stream.
 Everything that positions a shard is closed-form integer arithmetic (NCO phase, halfband
-pairing, polyphase phase, output index: `iqgpu_chain_seek`); finite-memory filter state is
-rebuilt by re-processing a halo in front of the shard and dropping its outputs.
+pairing, polyphase phase, FFT-filter block position, output index: `iqgpu_chain_seek`,
+`iqgpu_chain_outputs_after`); finite-memory filter state is rebuilt by re-processing a halo in
+front of the shard and dropping its outputs.
 
-There is exactly one data-dependent exchange: the digital AGC (src/agc.c:105-222) is a scalar
-state machine over per-chunk peaks, so a shard needs the state left by all earlier chunks.
-The ranks all-gather their per-chunk peaks (4 bytes per 16384 input frames) and each replays the
-state machine on the host over the chunks that precede its shard (`exchange_agc_state`).  No
-sample data crosses GPUs.
+The AGC is the only data-dependent exchange, and no sample data crosses GPUs:
+- the digital AGC (src/agc.c:105-222) is a scalar state machine over per-chunk peaks, so a shard
+  needs the state left by all earlier chunks.  The ranks all-gather their per-chunk peaks
+  (4 bytes per 16384 input frames) and each replays the state machine over the chunks that
+  precede its shard (`exchange_agc_state`, or on the device);
+- the RMS AGC (liquid agc_crcf) is a per-sample recurrence in {g, y2'}.  Every shard runs it from
+  the reset state at its lead, then `world - 1` rounds follow: the ranks all-gather their end
+  states (8 bytes each) and rank g >= 1 resumes its AGC at its first owned output from rank
+  g-1's end state.  After round k ranks 0..k are exact; a resume whose start state did not change
+  is a no-op on the device, so once the shards are longer than the recurrence's merge time the
+  later rounds cost only their collectives.
 """
 from __future__ import annotations
 
@@ -21,7 +28,7 @@ from typing import List, Optional, Tuple
 import numpy as np
 
 from . import gpu
-from .configs import AGC_DIGITAL, CHUNK_SAMPLES
+from .configs import AGC_DIGITAL, AGC_DX, AGC_LOCAL, CHUNK_SAMPLES
 
 
 @dataclass
@@ -68,9 +75,9 @@ def plan_shards(chain: "gpu.Chain", total_frames: int, world: int, halo_frames: 
         lead = max(0, start - halo)
         shards.append(Shard(rank=r, world=world, start=start, frames=end - start, lead=lead,
                             skip_chunks=(start - lead) // chunk,
-                            out_lead=chain.resampler_outputs_after(lead),
-                            out_start=chain.resampler_outputs_after(start),
-                            out_end=chain.resampler_outputs_after(end)))
+                            out_lead=chain.outputs_after(lead),
+                            out_start=chain.outputs_after(start),
+                            out_end=chain.outputs_after(end)))
         c0 += nc
     return shards
 
@@ -168,24 +175,28 @@ class ShardedChain:
         opts = dict(options)
         self.cfg = cfg
         self.digital_agc = bool(cfg.agc_enable and cfg.agc_profile == AGC_DIGITAL)
+        self.rms_agc = bool(cfg.agc_enable and cfg.agc_profile in (AGC_DX, AGC_LOCAL))
+        self.device = device
         self._probe = gpu.Chain(cfg, -1)
         halo = self._probe.halo_frames()
         halo += (-halo) % CHUNK_SAMPLES
         self.halo = halo
-        if self.digital_agc and shard_frames_hint:
-            # the begun call must be one sub-train: the resampled stream is kept on the device across the exchange
+        if (self.digital_agc or self.rms_agc) and shard_frames_hint:
+            # the shard's call must be one sub-train: the AGC's input (and for the RMS AGC its output and checkpoints) is
+            # kept on the device across the exchange
             opts["subtrain_frames"] = max(int(opts.get("subtrain_frames", 0)), shard_frames_hint + halo + CHUNK_SAMPLES)
         self.chain = gpu.Chain(cfg, device, **opts)
         self.agc_target = cfg.agc_target_level_arg if cfg.agc_target_level_arg > 0 else 0.9   # agc.c:108-110, constants.h:184
         self.target_rate = float(np.float32(cfg.target_rate_hz))
         # input frames (whole chunks) after which the digital AGC is certainly locked: more than 2 s of output samples
-        # (agc.c:145-149) plus two chunks of slack
+        # (agc.c:145-149) plus two chunks of slack.  Output counts are the chain's (outputs_after): an FFT filter's block
+        # lag (n output frames, several chunks at cfg3's rates) is part of them.
         lock_out = int(2.0 * self.target_rate) + 2
         k = 0
         if self.digital_agc:
             step = max(1, int(lock_out / max(cfg.ratio, 1e-9)) // CHUNK_SAMPLES)
-            while self._probe.resampler_outputs_after(k * CHUNK_SAMPLES) <= lock_out:
-                k += step if self._probe.resampler_outputs_after((k + step) * CHUNK_SAMPLES) <= lock_out else 1
+            while self._probe.outputs_after(k * CHUNK_SAMPLES) <= lock_out:
+                k += step if self._probe.outputs_after((k + step) * CHUNK_SAMPLES) <= lock_out else 1
         self.lock_frames = (k + 2) * CHUNK_SAMPLES
 
     def plan(self, total_frames: int, world: int) -> List[Shard]:
@@ -265,6 +276,49 @@ class ShardedChain:
             mark()                                            # own scan + scale + convert
             return produced
 
+    def rms_resume(self, shard: Shard, gathered_ptr: int, dev_out_ptr: int, out_capacity_bytes: int, stream: int = 0,
+                   changed_ptr: int = 0) -> None:
+        """One round of the RMS-AGC hand-over on this rank, after the all-gather: `gathered_ptr` holds every rank's end
+        state ({g, y2'} float32 pairs in rank order, device memory); rank g >= 1 resumes from rank g-1's."""
+        if shard.rank and shard.read_frames:
+            self.chain.agc_rms_resume_device(shard.drop, gathered_ptr + 8 * (shard.rank - 1), dev_out_ptr,
+                                             out_capacity_bytes, changed_ptr, stream)
+
+    def _rms_rounds(self, shard: Shard, dev_out_ptr: int, out_capacity_bytes: int, stream: int, group, device) -> None:
+        """The `world - 1` rounds of the RMS-AGC hand-over.  On a CUDA communication device everything is queued on the
+        chain's stream without a host synchronisation (8-byte all-gathers over NCCL); otherwise the states travel through
+        the host over any torch.distributed group.  A rank with an empty shard sends zeros (it is the last with data
+        behind it) and takes part in every collective."""
+        import torch
+        import torch.distributed as dist
+
+        ch, world = self.chain, shard.world
+        if str(device).startswith("cuda"):
+            key = (world, str(device))
+            bufs = getattr(self, "_rms_bufs", None)
+            if bufs is None or bufs[0] != key:
+                bufs = (key, torch.zeros(2, dtype=torch.float32, device=device),
+                        torch.zeros(2 * world, dtype=torch.float32, device=device))
+                self._rms_bufs = bufs
+            mine, gathered = bufs[1], bufs[2]
+            with self._on_stream(stream):
+                for _ in range(world - 1):
+                    if shard.read_frames:
+                        ch.agc_rms_state_device(mine.data_ptr(), stream)
+                    else:
+                        mine.zero_()
+                    dist.all_gather_into_tensor(gathered, mine, group=group)
+                    self.rms_resume(shard, gathered.data_ptr(), dev_out_ptr, out_capacity_bytes, stream)
+            return
+        for _ in range(world - 1):
+            mine = torch.tensor(ch.get_agc_rms_state() if shard.read_frames else (0.0, 0.0), dtype=torch.float32)
+            got = [torch.zeros_like(mine) for _ in range(world)]
+            dist.all_gather(got, mine, group=group)
+            # kept alive on the object: the resume reads it asynchronously on the chain's stream
+            self._rms_host_state = torch.cat(got).to(torch.device("cuda", self.device))
+            torch.cuda.synchronize(self.device)           # a copy from pageable memory may still be in flight on return
+            self.rms_resume(shard, self._rms_host_state.data_ptr(), dev_out_ptr, out_capacity_bytes, stream)
+
     def process_device(self, shard: Shard, dev_in_ptr: int, dev_out_ptr: int, out_capacity_bytes: int,
                        stream: int = 0, group=None, comm_device="cpu") -> Tuple[int, int]:
         """Returns (frames written, frames to drop from the front)."""
@@ -272,6 +326,10 @@ class ShardedChain:
         out_lead = ch.seek(shard.lead)
         assert out_lead == shard.out_lead
         n = shard.read_frames
+        if self.rms_agc and shard.world > 1:
+            produced = ch.process_device(dev_in_ptr, n, dev_out_ptr, out_capacity_bytes, stream) if n else 0
+            self._rms_rounds(shard, dev_out_ptr, out_capacity_bytes, stream, group, comm_device)
+            return produced, shard.drop
         exchange = self.digital_agc and shard.world > 1
         plan = getattr(self, "_plans", {}).get((shard.world, shard.rank, shard.start, shard.frames))
         sizes = getattr(self, "_table_sizes", {}).get((shard.world, shard.rank, shard.start, shard.frames))
