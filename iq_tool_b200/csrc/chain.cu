@@ -475,7 +475,7 @@ int iqgpu_chain::init_device()
     if (!rs.passthrough && !rs.is_interp && !pre_filter0) {
         ResamplerDesc rd{};
         rd.S = rs.num_halfband; rd.zeta = rs.zeta; rd.step = rs.step;
-        bool ok = rs.num_halfband <= (unsigned)FUSED_MAX_STAGES;
+        bool ok = rs.num_halfband <= (unsigned)W2_MAXS;
         for (unsigned d = 0; ok && d < rs.num_halfband; d++) {
             const unsigned g = rs.num_halfband - 1 - d;
             rd.m_exec[d] = rs.stages[g].m;

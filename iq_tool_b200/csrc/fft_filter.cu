@@ -17,7 +17,6 @@
 #include <algorithm>
 #include <cstdio>
 #include <cmath>
-#include <cstdlib>
 
 #include "fft_core.cuh"
 #include "fft_filter2.cuh"
@@ -154,13 +153,12 @@ static cudaError_t launch_smem(const float2* src, float2* dst, unsigned M, unsig
 
 // v2 (radix-16 register butterflies, fft_filter2.cuh) serves every transform that fits one CTA
 static bool v2_capable(unsigned nfft) { return nfft >= 64 && nfft <= fft2::MAX_POINTS; }
-static bool use_v2(unsigned nfft) { return v2_capable(nfft) && !getenv("IQGPU_FFT_V1"); }
 static size_t v2_smem_bytes(unsigned nfft) { return (size_t)(fft2::pad(nfft) + 8) * sizeof(float2); }
 
 size_t fft_twiddle_entries(unsigned nfft)
 {
     size_t n = nfft;
-    if (v2_capable(nfft)) {      // (whatever IQGPU_FFT_V1 says now: the kernel choice is made at launch time)
+    if (v2_capable(nfft)) {
         const fft2::Plan P = fft2::make_plan(nfft);
         unsigned L = nfft;
         for (unsigned k = 0; k < P.n16; k++, L >>= 4) n += 4 * (size_t)(L >> 4);
@@ -189,7 +187,7 @@ void fft_fill_twiddles(unsigned nfft, float2* host)
 cudaError_t launch_fft_forward(const float2* in, unsigned nfft, const float2* twiddle, float2* out, cudaStream_t st)
 {
     if (!is_pow2(nfft) || nfft < 2 || nfft > FFT_MAX_POINTS) return cudaErrorInvalidValue;
-    if (use_v2(nfft)) {
+    if (v2_capable(nfft)) {
         cudaError_t ea = cudaFuncSetAttribute(fft2::fft2_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                               (int)(fft2::SMEM_F2 * sizeof(float2)));
         if (ea != cudaSuccess) return ea;
@@ -213,7 +211,7 @@ cudaError_t launch_fftfilt(const float2* x, size_t nblocks, unsigned B, const fl
     if (!fftfilt_supported(B)) return cudaErrorInvalidValue;
     const unsigned N = 2 * B;
     const float scale = 1.0f / (float)N;
-    if (use_v2(N)) {
+    if (v2_capable(N)) {
         cudaError_t ea = cudaFuncSetAttribute(fft2::fftfilt2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                               (int)(fft2::SMEM_F2 * sizeof(float2)));
         if (ea != cudaSuccess) return ea;
@@ -225,7 +223,7 @@ cudaError_t launch_fftfilt(const float2* x, size_t nblocks, unsigned B, const fl
             cudaGetDevice(&dev);
             cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
             cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fft2::fftfilt2_kernel, fft2::THREADS, v2_smem_bytes(fft2::MAX_POINTS));
-            wave = getenv("IQGPU_FFT_NO_PREFETCH") ? 0 : std::max(1, sms * std::max(1, per_sm));
+            wave = std::max(1, sms * std::max(1, per_sm));
         }
         const unsigned w = (N == fft2::MAX_POINTS) ? (unsigned)wave : 0u;     // smaller transforms run several CTAs per SM
         fft2::fftfilt2_kernel<<<(unsigned)nblocks, fft2::THREADS, v2_smem_bytes(N), st>>>(x, y, N, twiddle, H, scale, w);

@@ -8,17 +8,12 @@
 // pre-resample filter) + resampler_execute (src/resampler.c:49 -> liquid msresamp_crcf_execute)
 // in ONE pass over HBM: 4 B/sample in (cs16), 8*r B/sample out.
 //
-// Execution model.  The sub-train is cut into blocks of B0 raw frames aligned to the ABSOLUTE
-// stream index.  A CTA owns a contiguous run of blocks and streams through it: per block it
-// (P0) loads + pre-processes B0 frames into shared memory (even/odd planes, padded so that
-// R-consecutive-output register windows are bank-conflict free), then runs the halfband
-// stages level by level through shared memory, then the polyphase stage, writing only the
-// resampled output to global memory.  Filter histories live in shared memory and slide from
-// block to block; a CTA warms its histories up by re-computing `warm_blocks` blocks before its
-// first own block (the filter-length halo).  Frames older than the call (previous call /
-// sub-train) come from a small cf32 "tail" of the pre-processed stream kept in HBM, so nothing
-// depends on how the host cuts the stream into calls.  All indices are absolute; the halfband
-// pairing, the 24-bit polyphase phase and the NCO phase are closed forms of the index.
+// The kernel is the warp-streaming one of fused_front2.cuh, instantiated here.  This file matches
+// the cascade to one of its compiled plans (S = 0..W2_MAXS halfband stages, semi-lengths
+// 3...3,5,10; any other cascade runs the stage-by-stage kernels), sizes and launches it, and runs
+// the DC pre-pass.
+// Frames older than the call (previous call / sub-train) come from a small cf32 "tail" of the
+// pre-processed stream kept in HBM, so nothing depends on how the host cuts the stream into calls.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -31,318 +26,7 @@
 
 namespace iqgpu {
 
-constexpr int FF_THREADS = 256;
-constexpr int FF_WARPS = FF_THREADS / 32;
-constexpr int FF_ARB_HIST = 16;   // >= 13 decimated samples of look-back
-constexpr int FF_BANK_STRIDE = 15; // odd row stride: scattered polyphase rows spread over banks
-constexpr int FF_NOPAD = 31;       // padding shift meaning "no padding"
-
-struct FusedPlan {
-    int S, B0, DB;                      // stages, raw frames per block, decimated frames per block
-    int m[FUSED_MAX_STAGES], R[FUSED_MAX_STAGES];
-    int sh[FUSED_MAX_STAGES];           // padding shift of level d's planes (= log2 R[d], or FF_NOPAD)
-    int Hh[FUSED_MAX_STAGES];           // history entries per plane of level d
-    int e_off[FUSED_MAX_STAGES], o_off[FUSED_MAX_STAGES];   // float2 offsets of level d's planes
-    int taps_off[FUSED_MAX_STAGES];     // float offset of depth d's taps inside the taps area
-    int flat_off;                       // level S (polyphase input), float2 offset
-    int levels_end;                     // float2 count of all level buffers (zeroed at start)
-    int taps_base, taps_total;          // float2 offset / float count
-    int bank_base;                      // float2 offset of the polyphase bank (256 x FF_BANK_STRIDE floats)
-    int lut_base;                       // float2 offset of the NCO table
-    int misc_base;                      // float2 offset of 2 x int64 scratch
-    int smem_bytes;
-    int warm_blocks, H_tail;
-    float zeta;
-    uint32_t step;
-};
-
-struct FusedArgs {
-    FusedPlan plan;
-    const void* raw;
-    long long n0, N1;                   // absolute index range of raw
-    const float2* tail_in;
-    float2* tail_out;
-    PreParams pre;
-    DcDev dc;
-    const double2* dc_table;            // v at absolute multiples of 256, starting at A0
-    long long A0;
-    const float* taps;                  // device, concatenated h1 by depth
-    const float* bank;                  // device, [256][14]
-    long long O0, O1;
-    float2* y;
-    long long blk_first, blk_last;
-    int blocks_per_cta;
-    int raw_aligned;
-};
-
-__device__ __forceinline__ int ff_phys(int p, int sh) { return p + (p >> sh); }
-
-template <int FMT>
-__device__ __forceinline__ void ff_load_quad(const void* __restrict__ raw, long long rel, long long n, float sc,
-                                             float gain, bool aligned, float2 (&x)[4])
-{
-    if (rel >= 0 && rel + 4 <= n) {
-        load_quad<FMT>(raw, (size_t)rel, (size_t)n, sc, gain, aligned, x);
-        return;
-    }
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-        const long long i = rel + k;
-        x[k] = (i >= 0 && i < n) ? load_frame<FMT>(raw, (size_t)i, sc, gain) : make_float2(0.f, 0.f);
-    }
-}
-
-// ---- P0: load + pre-process one block into level 0 -------------------------------------------
-template <int FMT, bool DC>
-__device__ __forceinline__ void ff_p0(const FusedArgs& A, float2* __restrict__ sm, const float* __restrict__ lut,
-                                      long long block_start, int warp, int lane)
-{
-    const FusedPlan& P = A.plan;
-    const PreParams& p = A.pre;
-    const float sc = in_scale<FMT>(p.gain);
-    const long long n = A.N1 - A.n0;
-    const float lanepow = DC ? A.dc.lanepow[lane] : 0.f;
-    float2* E = sm + P.e_off[0];
-    float2* O = sm + P.o_off[0];
-    float2* flat = sm + P.flat_off;
-    const int sh0 = P.sh[0], Hh0 = P.Hh[0];
-    for (int run = warp; run < P.B0 / 256; run += FF_WARPS) {
-        const long long rs = block_start + (long long)run * 256;
-        const bool active = (rs + 256 > A.n0) && (rs < A.N1);
-        double vr = 0.0, vi = 0.0;
-        if (DC && active) {
-            const double2 v = A.dc_table[(rs - A.A0) >> 8];
-            vr = v.x; vi = v.y;
-        }
-#pragma unroll
-        for (int rr = 0; rr < 2; rr++) {
-            const long long a = rs + rr * 128 + lane * 4;
-            float2 x[4];
-            if (active) {
-                ff_load_quad<FMT>(A.raw, a - A.n0, n, sc, p.gain, A.raw_aligned != 0, x);
-                if (DC) {
-                    float2 Ex, T;
-                    dc_row_scan(x, A.dc, lane, Ex, T);
-                    float wr = fmaf(lanepow, (float)vr, Ex.x), wi = fmaf(lanepow, (float)vi, Ex.y);
-#pragma unroll
-                    for (int k = 0; k < 4; k++) {
-                        const float xr = x[k].x, xi = x[k].y;
-                        x[k].x = fmaf(-A.dc.a, wr, xr);
-                        x[k].y = fmaf(-A.dc.a, wi, xi);
-                        wr = fmaf(A.dc.c, wr, xr);
-                        wi = fmaf(A.dc.c, wi, xi);
-                    }
-                    vr = fma(A.dc.c128, vr, (double)T.x);
-                    vi = fma(A.dc.c128, vi, (double)T.y);
-                }
-                if (p.iq_enable) {
-#pragma unroll
-                    for (int k = 0; k < 4; k++) {
-                        const float re = x[k].x;
-                        x[k].x = __fmul_rn(re, p.iq_magp1);
-                        x[k].y = __fadd_rn(x[k].y, __fmul_rn(p.iq_phase, re));
-                    }
-                }
-                if (p.nco_enable) {
-#pragma unroll
-                    for (int k = 0; k < 4; k++) {
-                        const uint32_t th = p.nco_theta0 + (uint32_t)(a + k - A.n0) * p.nco_dtheta;
-                        x[k] = nco_mix(x[k], th, p.nco_sign, lut);
-                    }
-                }
-            } else {
-#pragma unroll
-                for (int k = 0; k < 4; k++) x[k] = make_float2(0.f, 0.f);
-            }
-            if (a < A.n0) {   // frames of an earlier call: already pre-processed, kept in the tail
-#pragma unroll
-                for (int k = 0; k < 4; k++) {
-                    if (a + k < A.n0) {
-                        const long long j = a + k - (A.n0 - P.H_tail);
-                        x[k] = (j >= 0) ? A.tail_in[j] : make_float2(0.f, 0.f);
-                    }
-                }
-            }
-            if (a + 4 > A.N1 - P.H_tail && a < A.N1) {
-#pragma unroll
-                for (int k = 0; k < 4; k++) {
-                    const long long j = a + k - (A.N1 - P.H_tail);
-                    if (j >= 0 && a + k < A.N1) A.tail_out[j] = x[k];
-                }
-            }
-            const int q = (int)(a - block_start);   // block-relative index, multiple of 4
-            if (P.S == 0) {
-#pragma unroll
-                for (int k = 0; k < 4; k++) flat[FF_ARB_HIST + q + k] = x[k];
-            } else {
-                const int pe = (q >> 1) + Hh0;
-                E[ff_phys(pe, sh0)] = x[0];
-                O[ff_phys(pe, sh0)] = x[1];
-                E[ff_phys(pe + 1, sh0)] = x[2];
-                O[ff_phys(pe + 1, sh0)] = x[3];
-            }
-        }
-    }
-}
-
-// ---- one halfband decimator level: liquid resamp2_crcf_decim_execute over a block -------------
-//   y[q] = sum_{j<2M} h1[j] * E[q-2M+1+j] + O[q-M]        (plane-local, before the history offset)
-template <int M, int R>
-__device__ __forceinline__ void ff_stage(const float2* __restrict__ E, const float2* __restrict__ O, int Hh,
-                                         const float* __restrict__ h1, int n_out, float scale, bool next_flat,
-                                         float2* __restrict__ nE, float2* __restrict__ nO, int nsh, int nHh,
-                                         float2* __restrict__ nflat, int tid)
-{
-    constexpr int SH = (R == 4) ? 2 : (R == 2 ? 1 : FF_NOPAD);
-    for (int q0 = tid * R; q0 < n_out; q0 += FF_THREADS * R) {
-        float2 acc[R], win[R];
-        const int base = q0 - 2 * M + 1 + Hh;
-#pragma unroll
-        for (int r = 0; r < R; r++) {
-            acc[r] = make_float2(0.f, 0.f);
-            win[r] = E[ff_phys(base + r, SH)];
-        }
-#pragma unroll
-        for (int j = 0; j < 2 * M; j++) {
-            const float h = h1[j];
-#pragma unroll
-            for (int r = 0; r < R; r++) {
-                const float2 v = win[(r + j) % R];
-                acc[r].x = fmaf(h, v.x, acc[r].x);
-                acc[r].y = fmaf(h, v.y, acc[r].y);
-            }
-            if (j + 1 < 2 * M) win[j % R] = E[ff_phys(base + j + R, SH)];
-        }
-#pragma unroll
-        for (int r = 0; r < R; r++) {
-            const int q = q0 + r;
-            const float2 c = O[ff_phys(q - M + Hh, SH)];
-            const float2 v = make_float2((c.x + acc[r].x) * scale, (c.y + acc[r].y) * scale);
-            if (next_flat) nflat[FF_ARB_HIST + q] = v;
-            else {
-                float2* pl = (q & 1) ? nO : nE;
-                pl[ff_phys((q >> 1) + nHh, nsh)] = v;
-            }
-        }
-    }
-}
-
-__device__ __forceinline__ void ff_run_stage(const FusedPlan& P, float2* __restrict__ sm, const float* __restrict__ staps,
-                                             int d, int tid)
-{
-    const float2* E = sm + P.e_off[d];
-    const float2* O = sm + P.o_off[d];
-    const bool last = (d + 1 == P.S);
-    float2* nE = last ? nullptr : sm + P.e_off[d + 1];
-    float2* nO = last ? nullptr : sm + P.o_off[d + 1];
-    const int nsh = last ? FF_NOPAD : P.sh[d + 1], nHh = last ? 0 : P.Hh[d + 1];
-    float2* nflat = sm + P.flat_off;
-    const int n_out = P.B0 >> (d + 1);
-    const float scale = last ? P.zeta : 1.0f;
-    const float* h1 = staps + P.taps_off[d];
-    const int key = P.m[d] * 8 + P.R[d];
-#define FF_CASE(MM, RR) case (MM) * 8 + (RR): ff_stage<MM, RR>(E, O, P.Hh[d], h1, n_out, scale, last, nE, nO, nsh, nHh, nflat, tid); break;
-    switch (key) {
-        FF_CASE(3, 4) FF_CASE(3, 2) FF_CASE(3, 1)
-        FF_CASE(5, 4) FF_CASE(5, 2) FF_CASE(5, 1)
-        FF_CASE(10, 4) FF_CASE(10, 2) FF_CASE(10, 1)
-        default: break;
-    }
-#undef FF_CASE
-}
-
-// move the last Hh entries of each plane of level d to the history slots
-__device__ __forceinline__ void ff_slide_planes(const FusedPlan& P, float2* __restrict__ sm, int d, int tid)
-{
-    const int Hh = P.Hh[d], sh = P.sh[d], nh = P.B0 >> (d + 1);
-    if (tid < 2 * Hh) {
-        float2* pl = sm + ((tid < Hh) ? P.e_off[d] : P.o_off[d]);
-        const int i = (tid < Hh) ? tid : tid - Hh;
-        pl[ff_phys(i, sh)] = pl[ff_phys(i + nh, sh)];
-    }
-}
-
-// ---- polyphase arbitrary-rate stage: liquid resamp_crcf (fixed-point phase) over a block ------
-__device__ __forceinline__ void ff_arb(const FusedArgs& A, const float2* __restrict__ flat, const float* __restrict__ sbank,
-                                       long long kA, long long oa, long long ob, int tid)
-{
-    const uint32_t step = A.plan.step;
-    for (long long o = oa + tid; o < ob; o += FF_THREADS) {
-        const unsigned long long Pp = (unsigned long long)o * step;
-        const long long k = (long long)(Pp >> 24);
-        const unsigned idx = (unsigned)((Pp & 0xffffffull) >> 16);
-        const float2* __restrict__ w = flat + (int)(k - kA) + FF_ARB_HIST - 13;
-        const float* __restrict__ b = sbank + idx * FF_BANK_STRIDE;
-        float sr = 0.f, si = 0.f;
-#pragma unroll
-        for (int i = 0; i < 14; i++) {
-            const float2 v = w[i];
-            const float h = b[i];
-            sr = fmaf(h, v.x, sr);
-            si = fmaf(h, v.y, si);
-        }
-        A.y[o - A.O0] = make_float2(sr, si);
-    }
-}
-
-template <int FMT, bool DC>
-__global__ void __launch_bounds__(FF_THREADS, 3) fused_front_kernel(const __grid_constant__ FusedArgs A)
-{
-    extern __shared__ __align__(16) float2 sm[];
-    const FusedPlan& P = A.plan;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    float* staps = reinterpret_cast<float*>(sm + P.taps_base);
-    float* sbank = reinterpret_cast<float*>(sm + P.bank_base);
-    float* lut = reinterpret_cast<float*>(sm + P.lut_base);
-    long long* misc = reinterpret_cast<long long*>(sm + P.misc_base);
-
-    const long long seg_first = A.blk_first + (long long)blockIdx.x * A.blocks_per_cta;
-    if (seg_first > A.blk_last) return;
-    long long seg_last = seg_first + A.blocks_per_cta - 1;
-    if (seg_last > A.blk_last) seg_last = A.blk_last;
-
-    for (int i = tid; i < P.levels_end; i += FF_THREADS) sm[i] = make_float2(0.f, 0.f);
-    for (int i = tid; i < P.taps_total; i += FF_THREADS) staps[i] = A.taps[i];
-    for (int i = tid; i < 256 * 14; i += FF_THREADS) sbank[(i / 14) * FF_BANK_STRIDE + (i % 14)] = A.bank[i];
-    if (A.pre.nco_enable)
-        for (int i = tid; i < 1024; i += FF_THREADS) lut[i] = A.pre.nco_table[i];
-    __syncthreads();
-
-    const int S = P.S;
-    float2* flat = sm + P.flat_off;
-    for (long long blk = seg_first - P.warm_blocks; blk <= seg_last; blk++) {
-        const long long block_start = blk * P.B0;
-        const bool emit = blk >= seg_first;
-        if (tid == 0 && emit) {
-            // outputs whose polyphase push index k lies in this block: o in [ceil(kA 2^24/step), ceil(kB 2^24/step))
-            const unsigned long long kA = (unsigned long long)(block_start >> S), kB = kA + P.DB;
-            long long oa = (long long)(((kA << 24) + A.plan.step - 1) / A.plan.step);
-            long long ob = (long long)(((kB << 24) + A.plan.step - 1) / A.plan.step);
-            misc[0] = oa > A.O0 ? oa : A.O0;
-            misc[1] = ob < A.O1 ? ob : A.O1;
-        }
-        ff_p0<FMT, DC>(A, sm, lut, block_start, warp, lane);
-        __syncthreads();
-        for (int d = 0; d < S; d++) {
-            if (d > 0) ff_slide_planes(P, sm, d - 1, tid);
-            ff_run_stage(P, sm, staps, d, tid);
-            __syncthreads();
-        }
-        if (S > 0) ff_slide_planes(P, sm, S - 1, tid);
-        if (emit) ff_arb(A, flat, sbank, block_start >> S, misc[0], misc[1], tid);
-        __syncthreads();
-        if (tid < FF_ARB_HIST) flat[tid] = flat[tid + P.DB];
-        if (S == 0) __syncthreads();
-    }
-}
-
-// =============================================================================================
-// host side
-// =============================================================================================
 struct FusedFront {
-    FusedPlan plan{};
-    float* d_taps = nullptr;
-    const float* d_bank = nullptr;
     float2* d_tail[2] = {nullptr, nullptr};
     int tail_cur = 0;
     // DC pre-pass products, double buffered so that the (HBM-bound) pre-pass of the next sub-train can
@@ -353,16 +37,14 @@ struct FusedFront {
     size_t dc_cap[2] = {0, 0};
     bool dc_ready[2] = {false, false};  // slot holds the table of the sub-train about to be launched
     int num_sms = 148;
-    int ctas_per_sm = 3;
     int format = 0;
-    // v2 (warp-streaming kernel, fused_front2.cuh): used when the cascade matches a compiled plan
-    bool v2 = false;
+    // the compiled plan of the warp-streaming kernel (fused_front2.cuh) that matches the cascade
     int v2_S = 0, v2_warps = 0, v2_sup = 1, v2_warm_sup = 0, v2_warp_f2 = 0;
     size_t v2_smem = 0;
     float v2_taps[W2_MAX_TAPS] = {0};
     float v2_zeta = 1.f;
     uint32_t v2_step = 0;
-    int H_tail = 0;                     // cf32 tail length of the kernel in use
+    int H_tail = 0;                     // cf32 tail length of the plan
     float2* d_bank_image = nullptr;     // polyphase bank in the v2 shared-memory layout (w2_bank_row)
     float2* d_bank_image_q = nullptr;   // ... and in the layout of the four-output variant (w2_qbank_chunk, rotation arb_tz)
     int arb_tz = 0, arb_b2 = 0, arb_b3 = 0, arb_skew_sh = 31;
@@ -408,7 +90,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 static EncodeTiledFn tensor_map_encoder()
 {
     static EncodeTiledFn fn = []() -> EncodeTiledFn {
-        if (getenv("IQGPU_NO_RAW_TMA")) return nullptr;
         void* p = nullptr;
         cudaDriverEntryPointQueryResult q{};
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
@@ -436,7 +117,6 @@ static bool encode_raw_map(CUtensorMap* map, const void* raw, size_t n_frames)
 
 static bool v2_setup(FusedFront* f, const ResamplerDesc& r, bool nco)
 {
-    if (getenv("IQGPU_FUSED_V1")) return false;
     bool ok = false;
 #define V2_TRY(SS) if (!ok && v2_plan_matches<SS>(r)) { v2_fill<SS>(f); ok = true; }
     V2_TRY(0) V2_TRY(1) V2_TRY(2) V2_TRY(3) V2_TRY(4) V2_TRY(5) V2_TRY(6)
@@ -467,49 +147,8 @@ bool fused_supported(int format, const ResamplerDesc& r)
         case IQGPU_FMT_CF32: break;
         default: return false;
     }
-    if (r.S > FUSED_MAX_STAGES) return false;
-    for (unsigned d = 0; d < r.S; d++)
-        if (r.m_exec[d] != 3 && r.m_exec[d] != 5 && r.m_exec[d] != 10) return false;
-    return true;
-}
-
-static void build_plan(FusedPlan& P, const ResamplerDesc& r, bool nco)
-{
-    memset(&P, 0, sizeof(P));
-    P.S = (int)r.S;
-    P.B0 = 2048;
-    while ((P.B0 >> P.S) < 64) P.B0 <<= 1;
-    P.DB = P.B0 >> P.S;
-    P.zeta = r.zeta;
-    P.step = r.step;
-    int off = 0, toff = 0;
-    long long halo = 0;
-    for (int d = 0; d < P.S; d++) {
-        P.m[d] = (int)r.m_exec[d];
-        const int n_out = P.B0 >> (d + 1);
-        P.R[d] = (n_out >= 4 * FF_THREADS) ? 4 : (n_out >= 2 * FF_THREADS ? 2 : 1);
-        P.sh[d] = P.R[d] == 4 ? 2 : (P.R[d] == 2 ? 1 : FF_NOPAD);
-        P.Hh[d] = 2 * P.m[d];
-        const int plane = P.Hh[d] + n_out;                 // entries per plane (level d holds B0>>d frames)
-        const int phys = plane + (P.R[d] > 1 ? (plane >> P.sh[d]) : 0) + 2;
-        P.e_off[d] = off; off += (phys + 1) & ~1;
-        P.o_off[d] = off; off += (phys + 1) & ~1;
-        P.taps_off[d] = toff; toff += 2 * P.m[d];
-        halo += (long long)(4 * P.m[d]) << d;
-    }
-    halo += (long long)FF_ARB_HIST << P.S;
-    P.flat_off = off; off += FF_ARB_HIST + P.DB + 2;
-    off = (off + 1) & ~1;
-    P.levels_end = off;
-    P.taps_base = off; P.taps_total = toff; off += (toff + 1) / 2 + 1;
-    off = (off + 1) & ~1;
-    P.bank_base = off; off += (256 * FF_BANK_STRIDE + 1) / 2 + 1;
-    off = (off + 1) & ~1;
-    P.lut_base = off; if (nco) off += 512;
-    P.misc_base = off; off += 2;
-    P.smem_bytes = off * (int)sizeof(float2);
-    P.warm_blocks = (int)((halo + P.B0 - 1) / P.B0);
-    P.H_tail = (P.warm_blocks + 1) * P.B0;
+    return v2_plan_matches<0>(r) || v2_plan_matches<1>(r) || v2_plan_matches<2>(r) || v2_plan_matches<3>(r) ||
+           v2_plan_matches<4>(r) || v2_plan_matches<5>(r) || v2_plan_matches<6>(r);
 }
 
 FusedFront* fused_create(int format, const ResamplerDesc& r, bool nco, const float* d_bank, int num_sms, std::string& err)
@@ -517,61 +156,49 @@ FusedFront* fused_create(int format, const ResamplerDesc& r, bool nco, const flo
     FusedFront* f = new FusedFront();
     f->format = format;
     f->num_sms = num_sms;
-    f->d_bank = d_bank;
-    build_plan(f->plan, r, nco);
-    f->H_tail = f->plan.H_tail;
-    f->v2 = v2_setup(f, r, nco);
-    if (!f->v2 && f->plan.smem_bytes > 200 * 1024) { err = "fused front: shared memory plan too large"; delete f; return nullptr; }
-    std::vector<float> taps;
-    for (unsigned d = 0; d < r.S; d++) taps.insert(taps.end(), r.h1_exec[d], r.h1_exec[d] + 2 * r.m_exec[d]);
-    if (taps.empty()) taps.push_back(0.f);
-    if (cudaMalloc(&f->d_taps, taps.size() * sizeof(float)) != cudaSuccess ||
-        cudaMemcpy(f->d_taps, taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMalloc(&f->d_tail[0], (size_t)f->H_tail * sizeof(float2)) != cudaSuccess ||
+    if (!v2_setup(f, r, nco)) { err = "fused front: no compiled plan fits this cascade"; delete f; return nullptr; }
+    if (cudaMalloc(&f->d_tail[0], (size_t)f->H_tail * sizeof(float2)) != cudaSuccess ||
         cudaMalloc(&f->d_tail[1], (size_t)f->H_tail * sizeof(float2)) != cudaSuccess) {
         err = "fused front: device allocation failed";
         fused_destroy(f);
         return nullptr;
     }
-    f->ctas_per_sm = std::max(1, std::min(4, (int)((220 * 1024) / f->plan.smem_bytes)));
-    if (f->v2) {
-        // lay the bank out the way the kernel reads it, so one TMA bulk copy stages it per CTA
-        std::vector<float> hb(256 * 14);
-        std::vector<float2> img(W2_BANK_F2, make_float2(0.f, 0.f));
-        if (cudaMemcpy(hb.data(), d_bank, hb.size() * sizeof(float), cudaMemcpyDeviceToHost) != cudaSuccess ||
-            cudaMalloc(&f->d_bank_image, img.size() * sizeof(float2)) != cudaSuccess) {
-            err = "fused front: bank image allocation failed";
-            fused_destroy(f);
-            return nullptr;
-        }
-        f->h_bank = hb;
-        for (int idx = 0; idx < 256; idx++)
-            for (int i = 0; i < 7; i++) img[w2_bank_row(idx) + i] = make_float2(hb[idx * 14 + 2 * i], hb[idx * 14 + 2 * i + 1]);
-        if (cudaMemcpy(f->d_bank_image, img.data(), img.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) {
+    // lay the bank out the way the kernel reads it, so one TMA bulk copy stages it per CTA
+    std::vector<float> hb(256 * 14);
+    std::vector<float2> img(W2_BANK_F2, make_float2(0.f, 0.f));
+    if (cudaMemcpy(hb.data(), d_bank, hb.size() * sizeof(float), cudaMemcpyDeviceToHost) != cudaSuccess ||
+        cudaMalloc(&f->d_bank_image, img.size() * sizeof(float2)) != cudaSuccess) {
+        err = "fused front: bank image allocation failed";
+        fused_destroy(f);
+        return nullptr;
+    }
+    f->h_bank = hb;
+    for (int idx = 0; idx < 256; idx++)
+        for (int i = 0; i < 7; i++) img[w2_bank_row(idx) + i] = make_float2(hb[idx * 14 + 2 * i], hb[idx * 14 + 2 * i + 1]);
+    if (cudaMemcpy(f->d_bank_image, img.data(), img.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) {
+        err = "fused front: bank image upload failed";
+        fused_destroy(f);
+        return nullptr;
+    }
+    // four-output variant: rows of 16 floats, rotated / chunk-permuted for this rate (fused_front2.cuh)
+    f->arb_b2 = (int)((2ull * r.step) >> 24);
+    f->arb_b3 = (int)((3ull * r.step) >> 24);
+    f->arb_quad_ok = ((f->arb_b2 == 2 && (f->arb_b3 == 3 || f->arb_b3 == 4)) || (f->arb_b2 == 3 && (f->arb_b3 == 4 || f->arb_b3 == 5)));
+    if (f->arb_quad_ok) {
+        f->arb_tz = (int)w2_pick_qbank_tz(r.step);
+        f->arb_skew_sh = 31;
+        if (f->v2_S <= 2)       // W2Plan<S>::quad_skew: only the shallow plans have room for a skewed level
+            f->arb_skew_sh = w2_pick_flat_skew(r.step);
+        std::vector<float> q((size_t)W2_BANK_F2 * 2, 0.f);
+        for (unsigned idx = 0; idx < 256; idx++)
+            for (unsigned j = 0; j < 4; j++)
+                for (unsigned t = 0; t < 4; t++)
+                    if (4 * j + t < 14) q[w2_qbank_chunk(idx, (unsigned)f->arb_tz, j) + t] = hb[idx * 14 + 4 * j + t];
+        if (cudaMalloc(&f->d_bank_image_q, q.size() * sizeof(float)) != cudaSuccess ||
+            cudaMemcpy(f->d_bank_image_q, q.data(), q.size() * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess) {
             err = "fused front: bank image upload failed";
             fused_destroy(f);
             return nullptr;
-        }
-        // four-output variant: rows of 16 floats, rotated / chunk-permuted for this rate (fused_front2.cuh)
-        f->arb_b2 = (int)((2ull * r.step) >> 24);
-        f->arb_b3 = (int)((3ull * r.step) >> 24);
-        f->arb_quad_ok = ((f->arb_b2 == 2 && (f->arb_b3 == 3 || f->arb_b3 == 4)) || (f->arb_b2 == 3 && (f->arb_b3 == 4 || f->arb_b3 == 5)));
-        if (f->arb_quad_ok) {
-            f->arb_tz = (int)w2_pick_qbank_tz(r.step);
-            f->arb_skew_sh = 31;
-            if (f->v2_S <= 2)       // W2Plan<S>::quad_skew: only the shallow plans have room for a skewed level
-                f->arb_skew_sh = getenv("IQGPU_ARB_SKEW") ? atoi(getenv("IQGPU_ARB_SKEW")) : w2_pick_flat_skew(r.step);
-            std::vector<float> q((size_t)W2_BANK_F2 * 2, 0.f);
-            for (unsigned idx = 0; idx < 256; idx++)
-                for (unsigned j = 0; j < 4; j++)
-                    for (unsigned t = 0; t < 4; t++)
-                        if (4 * j + t < 14) q[w2_qbank_chunk(idx, (unsigned)f->arb_tz, j) + t] = hb[idx * 14 + 4 * j + t];
-            if (cudaMalloc(&f->d_bank_image_q, q.size() * sizeof(float)) != cudaSuccess ||
-                cudaMemcpy(f->d_bank_image_q, q.data(), q.size() * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess) {
-                err = "fused front: bank image upload failed";
-                fused_destroy(f);
-                return nullptr;
-            }
         }
     }
     return f;
@@ -580,7 +207,7 @@ FusedFront* fused_create(int format, const ResamplerDesc& r, bool nco, const flo
 void fused_destroy(FusedFront* f)
 {
     if (!f) return;
-    cudaFree(f->d_taps); cudaFree(f->d_tail[0]); cudaFree(f->d_tail[1]);
+    cudaFree(f->d_tail[0]); cudaFree(f->d_tail[1]);
     for (int i = 0; i < 2; i++) { cudaFree(f->d_dc_table[i]); cudaFree(f->d_dc_sums[i]); cudaFree(f->d_dc_ws[i]); }
     cudaFree(f->d_bank_image);
     cudaFree(f->d_bank_image_q);
@@ -599,41 +226,19 @@ cudaError_t fused_reset(FusedFront* f, cudaStream_t st)
 
 uint32_t fused_halo_frames(const FusedFront* f)
 {
-    return f->v2 ? (uint32_t)(f->v2_warm_sup * f->v2_sup * W2_T0) : (uint32_t)(f->plan.warm_blocks * f->plan.B0);
+    return (uint32_t)(f->v2_warm_sup * f->v2_sup * W2_T0);
 }
-int fused_version(const FusedFront* f) { return f->v2 ? 2 : 1; }
 
 // DC blocker state v just before absolute frame `pos` of the sub-train that fused_launch() last ran from frame n0 with table
 // slot `slot` (device pointer into the tick table), or nullptr when the launch kept no table entry for that frame (local DC
-// state, v1 kernel, frame not on a tick boundary)
+// state, frame not on a tick boundary)
 const double2* fused_dc_state_at(const FusedFront* f, int slot, int64_t n0, int64_t pos)
 {
-    if (!f->v2 || slot < 0 || slot > 1 || !f->d_dc_table[slot] || pos < n0) return nullptr;
+    if (slot < 0 || slot > 1 || !f->d_dc_table[slot] || pos < n0) return nullptr;
     const int64_t A0 = (n0 / W2_T0) * W2_T0;
     if ((pos - A0) % W2_T0) return nullptr;
     const size_t idx = (size_t)((pos - A0) / W2_T0);
     return idx < f->dc_cap[slot] ? f->d_dc_table[slot] + idx : nullptr;
-}
-
-// DC pre-pass on the virtual range [A0, N1): frames below n0 read as zero, the carry is rewound to A0
-static cudaError_t fused_dc_prepass(FusedFront* f, int slot, const void* raw, long long n0, long long N1, const PreParams& pre,
-                                    double2* d_carry, long long A0, cudaStream_t st);
-
-template <int FMT>
-static cudaError_t launch_fmt(const FusedFront* f, const FusedArgs& A, int grid, bool dc, cudaStream_t st)
-{
-    const int smem = f->plan.smem_bytes;
-    cudaError_t e;
-    if (dc) {
-        e = cudaFuncSetAttribute(fused_front_kernel<FMT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-        fused_front_kernel<FMT, true><<<grid, FF_THREADS, smem, st>>>(A);
-    } else {
-        e = cudaFuncSetAttribute(fused_front_kernel<FMT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-        fused_front_kernel<FMT, false><<<grid, FF_THREADS, smem, st>>>(A);
-    }
-    return cudaGetLastError();
 }
 
 __global__ void dc_rewind_kernel(double2* carry, double c, long long k)
@@ -643,12 +248,12 @@ __global__ void dc_rewind_kernel(double2* carry, double c, long long k)
     *carry = make_double2(carry->x * f, carry->y * f);
 }
 
+// DC pre-pass on the virtual range [A0, N1): frames below n0 read as zero, the carry is rewound to A0
 static cudaError_t fused_dc_prepass(FusedFront* f, int slot, const void* raw, long long n0, long long N1, const PreParams& pre,
                                     double2* d_carry, long long A0, cudaStream_t st)
 {
     const size_t nv = (size_t)(N1 - A0);
-    const bool ticks = f->v2;                       // v2 keeps one table entry per 512-frame tick
-    const size_t n_runs = ticks ? (nv + 511) / 512 : (nv + 255) / 256;
+    const size_t n_runs = (nv + 511) / 512;          // one table entry per 512-frame tick
     if (n_runs + 2 > f->dc_cap[slot]) {
         cudaDeviceSynchronize();        // rare (first use / larger sub-train): nothing may still read the old buffers
         cudaFree(f->d_dc_table[slot]); cudaFree(f->d_dc_sums[slot]); cudaFree(f->d_dc_ws[slot]);
@@ -665,23 +270,18 @@ static cudaError_t fused_dc_prepass(FusedFront* f, int slot, const void* raw, lo
     const long long back = n0 - A0;
     const char* vraw = reinterpret_cast<const char*>(raw) - back * (long long)bps;
     if (back) dc_rewind_kernel<<<1, 1, 0, st>>>(d_carry, (double)pre.dc_c, back);
-    if (ticks) {
-        cudaError_t e = launch_dc_tick_sums(vraw, nv, (size_t)back, pre, f->d_dc_sums[slot], st);
-        if (e != cudaSuccess) return e;
-        return launch_dc_scan(f->d_dc_sums[slot], n_runs, 512, nv, pre.dc_c, d_carry, f->d_dc_table[slot], f->d_dc_ws[slot], st, 512);
-    }
-    cudaError_t e = launch_dc_run_sums_masked(vraw, nv, (size_t)back, pre, 256, f->d_dc_sums[slot], st);
+    cudaError_t e = launch_dc_tick_sums(vraw, nv, (size_t)back, pre, f->d_dc_sums[slot], st);
     if (e != cudaSuccess) return e;
-    return launch_dc_scan(f->d_dc_sums[slot], n_runs, 256, nv, pre.dc_c, d_carry, f->d_dc_table[slot], f->d_dc_ws[slot], st);
+    return launch_dc_scan(f->d_dc_sums[slot], n_runs, 512, nv, pre.dc_c, d_carry, f->d_dc_table[slot], f->d_dc_ws[slot], st, 512);
 }
 
 // DC pre-pass of the sub-train [n0, n0+n) into table slot `slot`, on stream `st` (which may differ from the
 // stream of the front kernel: the caller orders them with events).  fused_launch() then skips its own pre-pass.
 // local DC state + closed-form correction instead of the pre-pass: the blocker must be followed directly by the (real-tap,
 // linear, time-invariant) cascade — no I/Q apply and no table NCO in between
-static bool v2_dc_local(const FusedFront* f, const PreParams& pre)
+static bool v2_dc_local(const PreParams& pre)
 {
-    return f->v2 && pre.dc_enable && !pre.nco_enable && !pre.iq_enable && !getenv("IQGPU_DC_TABLE");
+    return pre.dc_enable && !pre.nco_enable && !pre.iq_enable && !getenv("IQGPU_DC_TABLE");
 }
 
 // gains of the cascade for the sequence c^n (see fused_front2.cuh): Atot over the halfband stages, G per polyphase row
@@ -719,9 +319,8 @@ cudaError_t fused_prepare_dc(FusedFront* f, int slot, const void* raw, int64_t n
                              double2* d_dc_carry, uint32_t* launches, cudaStream_t st)
 {
     if (n == 0 || !pre.dc_enable) return cudaSuccess;
-    if (v2_dc_local(f, pre)) return cudaSuccess;        // no pre-pass in this mode
-    const long long align = f->v2 ? W2_T0 : 256;
-    const long long A0 = (n0 / align) * align;
+    if (v2_dc_local(pre)) return cudaSuccess;        // no pre-pass in this mode
+    const long long A0 = (n0 / W2_T0) * W2_T0;
     cudaError_t e = fused_dc_prepass(f, slot, raw, n0, n0 + (long long)n, pre, d_dc_carry, A0, st);
     if (e != cudaSuccess) return e;
     f->dc_ready[slot] = true;
@@ -747,11 +346,12 @@ static cudaError_t launch_v2_s(const FusedFront* f, const Fused2Args& A, int gri
     return cudaGetLastError();
 }
 
-static cudaError_t fused_launch_v2(FusedFront* f, const void* raw, int64_t n0, size_t n, const PreParams& pre,
-                                   double2* d_dc_carry, int64_t O0, size_t n_out, float2* y, uint32_t* launches, int dc_slot,
-                                   cudaStream_t st, DcFold* fold)
+cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, const PreParams& pre, double2* d_dc_carry,
+                         int64_t O0, size_t n_out, float2* y, uint32_t* launches, int dc_slot, cudaStream_t st, DcFold* fold)
 {
     if (fold) fold->corr = nullptr;
+    if (n == 0) return cudaSuccess;
+    if (dc_slot < 0 || dc_slot > 1) dc_slot = 0;
     Fused2Args A{};
     A.raw = raw; A.n0 = n0; A.N1 = n0 + (long long)n;
     A.tail_in = f->d_tail[f->tail_cur];
@@ -769,7 +369,7 @@ static cudaError_t fused_launch_v2(FusedFront* f, const void* raw, int64_t n0, s
         if (f->lut_dtheta != pre.nco_dtheta || !f->lut_picked) {
             w2_pick_lut_swizzle(pre.nco_dtheta, f->lut_sh, f->lut_mask);
             f->lut_rot_c = 0;
-            if (!getenv("IQGPU_LUT_NO_ROT") && (pre.format == IQGPU_FMT_CS16 || pre.format == IQGPU_FMT_SC16Q11)) w2_pick_lut_rotation(pre.nco_dtheta, f->lut_sh, f->lut_mask, f->lut_rot_sh, f->lut_rot_c);
+            if (pre.format == IQGPU_FMT_CS16 || pre.format == IQGPU_FMT_SC16Q11) w2_pick_lut_rotation(pre.nco_dtheta, f->lut_sh, f->lut_mask, f->lut_rot_sh, f->lut_rot_c);
             if (getenv("IQGPU_VERBOSE"))
                 fprintf(stderr, "iqgpu: NCO table layout: fold sh %u mask %u, rotation sh %u c %u\n", f->lut_sh, f->lut_mask, f->lut_rot_sh, f->lut_rot_c);
             f->lut_dtheta = pre.nco_dtheta; f->lut_picked = true;
@@ -803,7 +403,7 @@ static cudaError_t fused_launch_v2(FusedFront* f, const void* raw, int64_t n0, s
                             cudaMemcpyDeviceToDevice, st);
         if (e != cudaSuccess) return e;
     }
-    const bool dc_local = v2_dc_local(f, pre);
+    const bool dc_local = v2_dc_local(pre);
     W2DcGeom geo{};
     if (dc_local) {
         e = v2_dc_gains(f, pre.dc_c, st);
@@ -923,69 +523,6 @@ cudaError_t fused_dc_correct_range(const DcFold& fold, float2* y, size_t first, 
     w2_dc_correct_kernel<<<std::max(cgrid, 1), 256, 0, st>>>(y + first, Oa, Oa + (long long)count, fold.step, fold.S, fold.geo,
                                                            fold.corr, fold.G, nullptr, 0, 0, 0);
     return cudaGetLastError();
-}
-
-cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, const PreParams& pre, double2* d_dc_carry,
-                         int64_t O0, size_t n_out, float2* y, uint32_t* launches, int dc_slot, cudaStream_t st, DcFold* fold)
-{
-    if (fold) fold->corr = nullptr;
-    if (n == 0) return cudaSuccess;
-    if (dc_slot < 0 || dc_slot > 1) dc_slot = 0;
-    if (f->v2) return fused_launch_v2(f, raw, n0, n, pre, d_dc_carry, O0, n_out, y, launches, dc_slot, st, fold);
-    const FusedPlan& P = f->plan;
-    FusedArgs A{};
-    A.plan = P;
-    A.raw = raw; A.n0 = n0; A.N1 = n0 + (long long)n;
-    A.tail_in = f->d_tail[f->tail_cur];
-    A.tail_out = f->d_tail[f->tail_cur ^ 1];
-    A.pre = pre;
-    A.dc = make_dc_dev(pre.dc_enable ? pre.dc_c : 0.f, pre.dc_a);
-    A.A0 = (n0 / 256) * 256;
-    A.taps = f->d_taps; A.bank = f->d_bank;
-    A.O0 = O0; A.O1 = O0 + (long long)n_out; A.y = y;
-    A.blk_first = n0 / P.B0;
-    A.blk_last = (A.N1 - 1) / P.B0;
-    const long long nblk = A.blk_last - A.blk_first + 1;
-    int grid = f->num_sms * f->ctas_per_sm;
-    long long per = (nblk + grid - 1) / grid;
-    // do not let the warm-up dominate: at least 4 warm-up lengths of own work per CTA
-    const long long min_per = std::max<long long>(1, 4LL * P.warm_blocks);
-    if (per < min_per) per = min_per;
-    grid = (int)((nblk + per - 1) / per);
-    A.blocks_per_cta = (int)per;
-    const size_t bps = (pre.format == IQGPU_FMT_CS8 || pre.format == IQGPU_FMT_CU8) ? 2 : (pre.format == IQGPU_FMT_CF32 ? 8 : 4);
-    (void)bps;
-    A.raw_aligned = ((reinterpret_cast<size_t>(raw) & 15) == 0) && (n0 % 4 == 0);
-    cudaError_t e;
-    // frames of the new tail that precede this call come from the old tail
-    if ((long long)n < P.H_tail) {
-        const size_t keep = (size_t)P.H_tail - n;
-        e = cudaMemcpyAsync(f->d_tail[f->tail_cur ^ 1], f->d_tail[f->tail_cur] + n, keep * sizeof(float2),
-                            cudaMemcpyDeviceToDevice, st);
-        if (e != cudaSuccess) return e;
-    }
-    if (pre.dc_enable) {
-        if (!f->dc_ready[dc_slot]) {
-            e = fused_dc_prepass(f, dc_slot, raw, n0, A.N1, pre, d_dc_carry, A.A0, st);
-            if (e != cudaSuccess) return e;
-            if (launches) *launches += 2;
-        }
-        f->dc_ready[dc_slot] = false;
-        A.dc_table = f->d_dc_table[dc_slot];
-    }
-    const bool dc = pre.dc_enable != 0;
-    switch (pre.format) {
-        case IQGPU_FMT_CS16:    e = launch_fmt<IQGPU_FMT_CS16>(f, A, grid, dc, st); break;
-        case IQGPU_FMT_SC16Q11: e = launch_fmt<IQGPU_FMT_SC16Q11>(f, A, grid, dc, st); break;
-        case IQGPU_FMT_CU16:    e = launch_fmt<IQGPU_FMT_CU16>(f, A, grid, dc, st); break;
-        case IQGPU_FMT_CS8:     e = launch_fmt<IQGPU_FMT_CS8>(f, A, grid, dc, st); break;
-        case IQGPU_FMT_CU8:     e = launch_fmt<IQGPU_FMT_CU8>(f, A, grid, dc, st); break;
-        case IQGPU_FMT_CF32:    e = launch_fmt<IQGPU_FMT_CF32>(f, A, grid, dc, st); break;
-        default: return cudaErrorInvalidValue;
-    }
-    if (launches) *launches += 1;
-    f->tail_cur ^= 1;
-    return e;
 }
 
 }  // namespace iqgpu

@@ -1,9 +1,9 @@
-// fused_front2.cuh — "warp-streaming" fused front (v2): the same computation as fused_front.cu's
-// block-synchronous kernel (convert -> [DC] -> [I/Q] -> [NCO] -> S halfband decimators -> 256-arm
-// polyphase stage, reference src/pre_processor.c:10-55 + src/resampler.c:49), restructured around
-// what ncu showed about v1 (profiles/r01a_fused_front_full_cfg2.md): the kernel is instruction-issue
-// bound (54 % issue active, 15 % FMA pipe, 7 % DRAM) with most issue slots going to address
-// arithmetic, run-time plan lookups and block barriers.
+// fused_front2.cuh — the "warp-streaming" fused front kernel (v2; host side in fused_front.cu):
+// convert -> [DC] -> [I/Q] -> [NCO] -> S halfband decimators -> 256-arm polyphase stage, reference
+// src/pre_processor.c:10-55 + src/resampler.c:49.  Its shape answers what ncu showed about the
+// block-synchronous kernel it replaced (profiles/r01a_fused_front_full_cfg2.md): that kernel was
+// instruction-issue bound (54 % issue active, 15 % FMA pipe, 7 % DRAM) with most issue slots going
+// to address arithmetic, run-time plan lookups and block barriers.
 //
 //   * Every WARP owns a contiguous run of the stream and a private set of level FIFOs in shared
 //     memory; nothing is shared between warps except read-only tables, so the kernel has no
@@ -40,7 +40,6 @@ constexpr int W2_T0 = 512;          // raw frames per warp tick
 #define W2_MAX_WARPS_DEF 20
 #endif
 constexpr int W2_MAX_WARPS = W2_MAX_WARPS_DEF;   // warps per CTA (one CTA per SM): bounded by 64K registers / (32 x registers per thread)
-constexpr int W2_MAXS = 6;          // deepest cascade with a compiled plan
 constexpr int W2_ARB_HIST = 16;     // >= 13 decimated samples of look-back
 // polyphase bank image in shared memory: row `idx` (14 taps = 7 float2) starts at float2 offset
 // 9*idx + (idx >> 2).  The odd stride plus the slow skew keeps the 16 lanes of a half-warp, whose

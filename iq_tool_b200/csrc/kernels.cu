@@ -22,7 +22,7 @@ namespace cg = cooperative_groups;
 namespace iqgpu {
 
 template <int FMT>
-__global__ void __launch_bounds__(256) dc_run_sums_kernel(const void* __restrict__ raw, size_t n, size_t lo, float gain,
+__global__ void __launch_bounds__(256) dc_run_sums_kernel(const void* __restrict__ raw, size_t n, float gain,
                                                           DcDev d, uint32_t run_len, size_t n_runs, bool aligned,
                                                           double2* __restrict__ run_sums)
 {
@@ -36,13 +36,7 @@ __global__ void __launch_bounds__(256) dc_run_sums_kernel(const void* __restrict
         double vr = 0.0, vi = 0.0;
         for (size_t i0 = base; i0 < end; i0 += 128) {
             float2 x[4], E, T;
-            const size_t i = i0 + lane * 4;
-            if (i >= lo) load_quad<FMT>(raw, i, n, sc, gain, aligned, x);
-            else {
-#pragma unroll
-                for (int k = 0; k < 4; k++)
-                    x[k] = (i + k >= lo && i + k < n) ? load_frame<FMT>(raw, i + k, sc, gain) : make_float2(0.f, 0.f);
-            }
+            load_quad<FMT>(raw, i0 + lane * 4, n, sc, gain, aligned, x);
             dc_row_scan(x, d, lane, E, T);
             vr = fma(d.c128, vr, (double)T.x);
             vi = fma(d.c128, vi, (double)T.y);
@@ -51,7 +45,7 @@ __global__ void __launch_bounds__(256) dc_run_sums_kernel(const void* __restrict
     }
 }
 
-// DC pre-pass for the fused front v2: one weighted sum per 512-frame tick, S_t = sum_k c^(511-k) x[k].
+// DC pre-pass for the fused front: one weighted sum per 512-frame tick, S_t = sum_k c^(511-k) x[k].
 // A lane owns 16 consecutive frames (4 x LDG.128 issued back to back for cs16), folds them serially and
 // the warp combines the 32 partial sums with a weighted shuffle tree; frames below `lo` and at or beyond
 // `n` read as zero.
@@ -346,18 +340,12 @@ static inline int grid_for_warps(size_t warps_needed, int threads)
 cudaError_t launch_dc_run_sums(const void* raw, size_t n, const PreParams& p, uint32_t run_len,
                                double2* run_sums, cudaStream_t st)
 {
-    return launch_dc_run_sums_masked(raw, n, 0, p, run_len, run_sums, st);
-}
-
-cudaError_t launch_dc_run_sums_masked(const void* raw, size_t n, size_t lo, const PreParams& p, uint32_t run_len,
-                                      double2* run_sums, cudaStream_t st)
-{
     if (n == 0) return cudaSuccess;
     const size_t n_runs = (n + run_len - 1) / run_len;
     const DcDev d = make_dc_dev(p.dc_c, p.dc_a);
     const bool aligned = (reinterpret_cast<size_t>(raw) & 15) == 0;
     const int grid = grid_for_warps(n_runs, 256);
-#define CALL(F) dc_run_sums_kernel<F><<<grid, 256, 0, st>>>(raw, n, lo, p.gain, d, run_len, n_runs, aligned, run_sums)
+#define CALL(F) dc_run_sums_kernel<F><<<grid, 256, 0, st>>>(raw, n, p.gain, d, run_len, n_runs, aligned, run_sums)
     DISPATCH_FMT(p.format, CALL)
 #undef CALL
     return cudaGetLastError();
@@ -744,13 +732,13 @@ __global__ void __launch_bounds__(FIR_THREADS) fir_param_kernel(const float2* __
 bool fir_can_fold_dc(unsigned ntaps_padded, int complex_taps, bool have_host_taps)
 {
     const unsigned nfloats = ntaps_padded * (complex_taps ? 2u : 1u);
-    return have_host_taps && nfloats <= FIR_PARAM_TAPS && !getenv("IQGPU_FIR_SMEM_TAPS") && !getenv("IQGPU_NO_DC_FOLD");
+    return have_host_taps && nfloats <= FIR_PARAM_TAPS && !getenv("IQGPU_NO_DC_FOLD");
 }
 
 bool fir_can_convert_out(int out_format, unsigned ntaps_padded, int complex_taps)
 {
     const unsigned nfloats = ntaps_padded * (complex_taps ? 2u : 1u);
-    if (nfloats > FIR_PARAM_TAPS || getenv("IQGPU_FIR_SMEM_TAPS") || getenv("IQGPU_FIR_NO_CONVERT")) return false;
+    if (nfloats > FIR_PARAM_TAPS || getenv("IQGPU_FIR_NO_CONVERT")) return false;
     return out_format == IQGPU_FMT_CS16 || out_format == IQGPU_FMT_CU8 || out_format == IQGPU_FMT_CS8;
 }
 
@@ -763,7 +751,7 @@ cudaError_t launch_fir(const float2* x, size_t n, const float* hrev, unsigned nt
     if (out_conv && !(hrev_host && fir_can_convert_out(out_format, ntaps_padded, complex_taps))) return cudaErrorInvalidValue;
     const bool folding = fold && fold->corr;
     if (folding && !fir_can_fold_dc(ntaps_padded, complex_taps, hrev_host != nullptr)) return cudaErrorInvalidValue;
-    if (hrev_host && nfloats <= FIR_PARAM_TAPS && !getenv("IQGPU_FIR_SMEM_TAPS")) {
+    if (hrev_host && nfloats <= FIR_PARAM_TAPS) {
         static thread_local FirTaps T;      // 16 KB: copied into the launch's parameter buffer
         memcpy(T.h, hrev_host, nfloats * sizeof(float));
         const bool vo = (reinterpret_cast<size_t>(out_conv) & 15) == 0;
@@ -1772,7 +1760,7 @@ static void agc_rms_plan(size_t n, float alpha, size_t& B, unsigned& nblocks)
     // blocks of ~20 time constants the second sweep already starts every block within ~e^-20 of the truth, so two
     // or three full sweeps plus a short tail of partial ones reach the fixed point; shorter blocks need one full
     // sweep per block length of convergence (measured: 25 sweeps at 493 samples, alpha = 1e-2).
-    static const double tc = getenv("IQGPU_AGC_BLOCK_TC") ? atof(getenv("IQGPU_AGC_BLOCK_TC")) : 30.0;     // measured on cfg4: 40 -> 3.65 ms, 30 -> 3.51, 20 -> 3.79, 10 -> 4.82
+    constexpr double tc = 30.0;     // measured on cfg4: 40 -> 3.65 ms, 30 -> 3.51, 20 -> 3.79, 10 -> 4.82
     const size_t floorB = (size_t)std::min(65536.0, std::max(256.0, tc / std::max((double)alpha, 1e-6)));
     if (B < floorB) B = floorB;
     B = (B + 3) & ~(size_t)3;           // whole 32-byte groups per block: the 256-bit accesses of agc_rms_block stay aligned

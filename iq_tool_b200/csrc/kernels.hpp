@@ -27,16 +27,13 @@ struct PreParams {
 // DC pass 1: per-run weighted sums S_r = sum_k c^(len-1-k) x[k] (converted samples)
 cudaError_t launch_dc_run_sums(const void* raw, size_t n, const PreParams& p, uint32_t run_len,
                                double2* run_sums, cudaStream_t st);
-// same, frames below `lo` read as zero (virtual, absolute-aligned ranges)
-cudaError_t launch_dc_run_sums_masked(const void* raw, size_t n, size_t lo, const PreParams& p, uint32_t run_len,
-                                      double2* run_sums, cudaStream_t st);
 // DC pass 2: v at the start of every run from the carried state; updates the carry in place
 // scan_ws: device workspace of dc_scan_workspace_doubles(n_runs) doubles
 // row_len: granularity the sums were zero-padded to (128 for launch_dc_run_sums rows, 512 for tick sums)
 cudaError_t launch_dc_scan(const double2* run_sums, size_t n_runs, uint32_t run_len, size_t n,
                            float dc_c, double2* carry_inout, double2* run_start, double* scan_ws, cudaStream_t st,
                            uint32_t row_len = 128);
-// DC pre-pass of the fused front v2: one weighted sum per 512-frame tick (frames below lo / beyond n read as zero)
+// DC pre-pass of the fused front: one weighted sum per 512-frame tick (frames below lo / beyond n read as zero)
 cudaError_t launch_dc_tick_sums(const void* raw, size_t n, size_t lo, const PreParams& p, double2* sums, cudaStream_t st);
 size_t dc_scan_workspace_doubles(size_t n_runs);
 // convert + (DC apply) + I/Q + NCO -> cf32
@@ -164,11 +161,13 @@ cudaError_t launch_iq_optimize_train(const float2* probes, int n_probes, IqOptSt
 float iq_direction_host(unsigned seed, unsigned long long pass, unsigned k);
 
 // ---- fused front: raw -> [convert, DC, I/Q, NCO] -> halfband cascade -> polyphase stage -------
-constexpr int FUSED_MAX_STAGES = 10;
+// The kernel (fused_front2.cuh) is compiled for the cascades S = 0..W2_MAXS with semi-lengths 3...3,5,10; fused_supported()
+// says whether a cascade is one of them.  Any other cascade runs the stage-by-stage kernels above.
+constexpr int W2_MAXS = 6;          // deepest cascade with a compiled plan
 struct ResamplerDesc {
     unsigned S;                                // halfband stages
-    unsigned m_exec[FUSED_MAX_STAGES];         // semi-length by EXECUTION depth (depth 0 = full input rate)
-    const float* h1_exec[FUSED_MAX_STAGES];    // host pointers to the 2m dot-product taps per depth
+    unsigned m_exec[W2_MAXS];                  // semi-length by EXECUTION depth (depth 0 = full input rate)
+    const float* h1_exec[W2_MAXS];             // host pointers to the 2m dot-product taps per depth
     float zeta;
     uint32_t step;
 };
@@ -195,7 +194,6 @@ FusedFront* fused_create(int format, const ResamplerDesc& r, bool nco, const flo
 void fused_destroy(FusedFront* f);
 cudaError_t fused_reset(FusedFront* f, cudaStream_t st);
 uint32_t fused_halo_frames(const FusedFront* f);
-int fused_version(const FusedFront* f);   // 1 = block-synchronous kernel, 2 = warp-streaming kernel
 const double2* fused_dc_state_at(const FusedFront* f, int slot, int64_t n0, int64_t pos);
 // raw[0] has absolute index n0; produces outputs [O0, O0+n_out) into y; d_dc_carry is the DC state at n0
 // (updated to the state at n0+n).  *launches is incremented by the kernels launched.

@@ -102,7 +102,7 @@ def have_ref(fast: bool = False) -> bool:
 
 
 def dropin_path() -> str:
-    return os.path.join(os.path.dirname(HERE), "tests", "native", "_build", "libiqdropin_harness.so")
+    return os.path.join(os.path.dirname(HERE), "iq_tool_b200", "host", "_build", "libiqdropin_harness.so")
 
 
 def get_lib(kind: str):

@@ -1,7 +1,7 @@
 """The drop-in host layer (iq_tool_b200/host/): the reference's stage/module prototypes backed by
 libiqgpu.so.  Driven by oracle/ref_harness.c — the SAME driver that walks chunks through the
 reference's own stage code — linked against the drop-in objects instead
-(tests/native/_build/libiqdropin_harness.so, built by `make -C iq_tool_b200/host harness`).
+(iq_tool_b200/host/_build/libiqdropin_harness.so, built by `make -C iq_tool_b200/host harness`).
 
 CPU tests: the library loads, exports the reference's prototypes, designs/validates exactly like
 the reference does, and fails loudly without a GPU.  GPU tests: chunk-by-chunk and threaded runs

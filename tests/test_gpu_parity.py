@@ -691,6 +691,54 @@ def test_fused_front_every_cascade_depth(S, gpu, monkeypatch):
         assert ym.size == ya.size and np.array_equal(ym.view(np.uint32), ya.view(np.uint32))
 
 
+@pytest.mark.parametrize("S", [7, 8, 9])
+def test_deep_cascades_run_the_stage_kernels(S, gpu):
+    """Cascades deeper than the fused front's compiled plans (S = 7..9 halfband stages, down to the 0.001 ratio floor;
+    S = 8 is 20 Msps -> 48 kHz) run the stage-by-stage kernels even where the fused front is allowed: NCO pre-shift
+    (and the DC blocker for S = 8), per-chunk counts equal to the oracle's, the north_star bar against the oracle, ragged
+    calls (incl. an empty one) == one call."""
+    rng = np.random.Generator(np.random.PCG64(200 + S))
+    fs = 20e6
+    target = fs * 0.61 / (1 << S)
+    n = (1 << 20) + (20000 << S) + 77
+    t = np.arange(n)
+    # a tone that the pre-shift moves into the output band, plus wideband noise
+    x = 0.3 * np.exp(2j * np.pi * ((123e3 + 0.1 * target) / fs) * t) + \
+        0.05 * (rng.standard_normal(n) + 1j * rng.standard_normal(n))
+    raw = np.empty(2 * n, dtype=np.int16)
+    raw[0::2] = np.clip(np.round(x.real * 32767), -32768, 32767)
+    raw[1::2] = np.clip(np.round(x.imag * 32767), -32768, 32767)
+    cfg = ChainConfig(input_format="cs16", output_format="cf32", input_rate_hz=fs, target_rate_hz=target,
+                      freq_shift_hz=-123e3, dc_block=(S == 8))
+    g = gpu.Chain(cfg, 0, fused=1)
+    y, counts = g.process(raw, return_chunk_counts=True)
+    info = g.info()
+    assert info.fused_front == 0 and info.num_halfband == S
+    o = CpuChain(cfg, _oracle_kind())
+    o.trace(n // 16384 + 4)
+    ref = o.process(raw)
+    assert np.array_equal(counts, o.traced())
+    _check_final(cfg, y.view(np.float32), ref)
+    g = gpu.Chain(cfg, 0, fused=1, subtrain_frames=1 << 24)      # one chunk per call, the last one up to 9.1e6 frames
+    parts, pos = [], 0
+    for m in (1, 0, 511, 513, 4096 << S, 16385, 100000, n):
+        m = min(m, n - pos)
+        if m == 0 and pos:
+            parts.append(g.process(raw[:0]))
+            continue
+        if m <= 0:
+            break
+        parts.append(g.process(raw[2 * pos:2 * (pos + m)], chunk_frames=[m]))
+        pos += m
+    many = np.concatenate(parts)
+    assert many.size == y.size
+    if cfg.dc_block:
+        # the DC scan of the stage path restarts its runs at every call: two fp32 evaluation orders of the same arithmetic
+        assert rel_rms_fullscale(many.view(np.complex64), y.view(np.complex64)) <= 1e-7
+    else:
+        assert np.array_equal(many.view(np.uint32), y.view(np.uint32))
+
+
 @pytest.mark.parametrize("S", [1, 4, 6])
 @pytest.mark.parametrize("rate", [0.505, 0.55, 0.66, 0.7, 0.8, 0.97])
 def test_polyphase_variants_are_bit_identical_at_every_rate_class(S, rate, gpu, monkeypatch):
