@@ -240,9 +240,15 @@ int  iqgpu_chain_outputs_after(iqgpu_chain *c, uint64_t frames_in, uint64_t *fra
  *                               shard's first owned output) with the state at `dev_state`, rewrites
  *                               and re-converts into `dev_out` (the last call's output buffer) only the
  *                               range that changed, and writes 1 / 0 to `dev_changed` (optional, device
- *                               int) when the end state did / did not change.  A resume at the same
+ *                               int) when the end state did / did not change.  Any sequence of resumes
+ *                               of one call is allowed: each leaves the outputs in front of `first_output`
+ *                               as they are and makes the outputs from it on and the end state those of
+ *                               the AGC run from `dev_state` at `first_output`.  A resume at the same
  *                               frame from the same state as the previous one does nothing on the device;
- *                               all of it is queued on `stream` without a host synchronisation;
+ *                               one in front of an earlier resume's frame first re-runs the whole call
+ *                               (and converts all of it again); one at the call's end (`first_output` =
+ *                               its output count) only sets the end state; beyond it, nothing happens.
+ *                               All of it is queued on `stream` without a host synchronisation;
  *        get_agc_rms_state      reads {g, y2'} to the host (synchronises). ----------------------------- */
 int  iqgpu_chain_agc_rms_state_device(iqgpu_chain *c, float *dev_state, void *cuda_stream);
 int  iqgpu_chain_agc_rms_resume_device(iqgpu_chain *c, size_t first_output, const float *dev_state, void *dev_out,

@@ -4,15 +4,16 @@
 //
 // Both functions evaluate in double to a relative error of a few 1e-16 and round once to float, i.e. they return the
 // correctly rounded float result except when the exact value lies within ~1e-15 (relative) of a float rounding boundary —
-// which is what a good libm returns (checked against glibc's logf / expf by tests/native/agc_math_check.cpp, run from
-// tests/test_host_logic.py: plain C++, the same IEEE double operations the GPU executes).
+// which is what a good libm returns (checked against long double by tests/native/agc_math_check.cpp, run from
+// tests/test_agc_rms_exact.py: plain C++, the same IEEE double operations the GPU executes).  The serial reference of the
+// RMS AGC (tests/native/agc_rms_serial.cpp) evaluates the recurrence with these same functions on the CPU.
 //
 //   logf:  glibc-style table method, 128 intervals over [0.699, 1.398): z = x / 2^k, r = z * invc - 1 (|r| < 0.008, exact
 //          for the two intervals around 1 where c = 1), log x = k ln2 + log c + log1p(r), log1p by a degree-7 polynomial
 //          in Estrin form: 6 dependent double operations after the table lookup (the Horner evaluation of an atanh series
 //          it replaces had 20).
 //   expf:  |t| <= 0.125 (t = -alpha/2 * log y2', alpha <= 1e-2: always): degree-10 Taylor polynomial in Estrin form,
-//          5 dependent operations instead of 14.
+//          5 dependent operations instead of 14; agc_exp_small covers 0.125 < |t| <= 0.5 off the fast path.
 #pragma once
 #include <math.h>
 #include <stdint.h>
@@ -127,4 +128,16 @@ AGC_HD double agc_exp_tiny(double t, const double* __restrict__ K)
     const double b2 = fma(t2, K[15], a4);
     const double c1 = fma(t4, b2, b1);
     return fma(t4, c1, b0);
+}
+
+// exp(t) in double, |t| <= 0.5: degree-13 Taylor polynomial in Horner form.  Off the fast path: 0.125 < |t| needs
+// y2' > e^25 at alpha = 1e-2 (a full-scale burst after a gain held at its 1e6 clamp), so latency does not matter here.
+AGC_HD double agc_exp_small(double t)
+{
+    double p = 1.0 / 6227020800.0;
+    p = fma(p, t, 1.0 / 479001600.0); p = fma(p, t, 1.0 / 39916800.0); p = fma(p, t, 1.0 / 3628800.0);
+    p = fma(p, t, 1.0 / 362880.0);    p = fma(p, t, 1.0 / 40320.0);    p = fma(p, t, 1.0 / 5040.0);
+    p = fma(p, t, 1.0 / 720.0);       p = fma(p, t, 1.0 / 120.0);      p = fma(p, t, 1.0 / 24.0);
+    p = fma(p, t, 1.0 / 6.0);         p = fma(p, t, 0.5);              p = fma(p, t, 1.0);
+    return fma(p, t, 1.0);
 }

@@ -247,6 +247,11 @@ struct iqgpu_chain {
     PostParams rms_qp{};
     bool rms_ready = false, rms_fresh = false;
     AgcRmsResume* d_rms_resume = nullptr;
+    // d_rms_rerun[0]: {g, y2'} the last call started from (its rms_g / rms_y2), [1]: the state of a re-run of that call
+    // (which so leaves d_agc alone); rms_resume_max: the latest resume frame since the call or its last re-run.  A resume
+    // in front of that frame first re-runs the call (iqgpu_chain_agc_rms_resume_device).
+    AgcState* d_rms_rerun = nullptr;
+    size_t rms_resume_max = 0;
     // streams: s_in = pre output; s_stage[d] = output of executed halfband stage d; s_rs = resampler
     // output; s_f = post-filter output (or pre-filter output when the filter is pre-resample)
     DevStream s_in, s_pref, s_arb_in, s_rs, s_f;
@@ -345,7 +350,7 @@ iqgpu_chain::~iqgpu_chain()
     cudaFree(d_lut); cudaFree(d_dc_carry); cudaFree(d_dc_ref); cudaFree(d_run_sums); cudaFree(d_run_start); cudaFree(d_scan_ws); cudaFree(d_bank);
     cudaFree(d_fir_taps); cudaFree(d_fft_H); cudaFree(d_fft_tw); cudaFree(d_fft_scratch); cudaFree(d_agc); cudaFree(d_seg_start);
     cudaFree(d_seg_peak); cudaFree(d_seg_gain); cudaFree(d_agc_scratch); cudaFree(d_agc_ws);
-    cudaFree(d_iq_state); cudaFree(d_iq_probe); cudaFree(d_agc_quiet); cudaFree(d_rms_resume);
+    cudaFree(d_iq_state); cudaFree(d_iq_probe); cudaFree(d_agc_quiet); cudaFree(d_rms_resume); cudaFree(d_rms_rerun);
     if (h_iq_state) cudaFreeHost(h_iq_state);
     if (ev_iq) cudaEventDestroy(ev_iq);
     if (ev_iq_probe) cudaEventDestroy(ev_iq_probe);
@@ -458,6 +463,7 @@ int iqgpu_chain::init_device()
     CK(cudaMalloc(&d_dc_carry, sizeof(double2)));
     CK(cudaMalloc(&d_dc_ref, sizeof(float2)));
     CK(cudaMalloc(&d_agc, sizeof(AgcState)));
+    if (agc_mode == 2) CK(cudaMalloc(&d_rms_rerun, 2 * sizeof(AgcState)));
     if (!rs.passthrough) {
         d_hb_taps.resize(rs.num_halfband, nullptr);
         for (unsigned i = 0; i < rs.num_halfband; i++) {
@@ -596,6 +602,14 @@ int iqgpu_chain::ensure_buffers()
 }
 
 __global__ void agc_state_init_kernel(AgcState* st, AgcState v) { *st = v; }
+// RMS-AGC resume at the end of the call: the end state becomes *s; *changed (optional) = whether it moved
+__global__ void agc_rms_set_end_kernel(AgcState* st, const float2* s, int* changed)
+{
+    const float2 v = *s;
+    if (changed)
+        *changed = (__float_as_uint(v.x) != __float_as_uint(st->rms_g) || __float_as_uint(v.y) != __float_as_uint(st->rms_y2)) ? 1 : 0;
+    st->rms_g = v.x; st->rms_y2 = v.y;
+}
 
 // Stream discontinuity.  All device state lives behind the stream the chain last ran on, so the reset is QUEUED there
 // (memsets + one tiny kernel, no host synchronisation: the host may go on enqueueing the next train while the previous
@@ -1104,10 +1118,12 @@ int iqgpu_chain::run_back(void* d_outp, size_t skip_chunks, size_t* out_frames, 
                 CK(cudaMalloc(&d_agc_ws, ws_need * 2));
                 agc_ws_bytes = ws_need * 2;
             }
+            static_assert(offsetof(AgcState, rms_y2) == offsetof(AgcState, rms_g) + sizeof(float), "{g, y2'} must be adjacent");
+            CK(cudaMemcpyAsync(&d_rms_rerun->rms_g, &d_agc->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
             CK(launch_agc_rms(post_src, post_n, qp, d_agc, y, d_agc_ws, st));
             CK(launch_post(y, post_n, qp, nullptr, 0, nullptr, 1, tap2, d_outp, st));
             launches += 2;
-            rms_src = post_src; rms_n = post_n; rms_qp = qp; rms_ready = true; rms_fresh = true;
+            rms_src = post_src; rms_n = post_n; rms_qp = qp; rms_ready = true; rms_fresh = true; rms_resume_max = 0;
         } else {
             CK(launch_post(post_src, post_n, qp, nullptr, 0, nullptr, 0, tap2, d_outp, st));
             launches++;
@@ -1688,16 +1704,38 @@ int iqgpu_chain_agc_rms_resume_device(iqgpu_chain* c, size_t first_output, const
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
     if (c->last_stream && st != c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
     c->last_stream = st;
-    if (first_output >= c->rms_n) {            // nothing of the call lies behind the resume point
+    if (first_output == c->rms_n) {            // at the end of the call: no output changes, the end state is the given one
+        agc_rms_set_end_kernel<<<1, 1, 0, st>>>(c->d_agc, reinterpret_cast<const float2*>(dev_state), dev_changed);
+        CK(cudaGetLastError());
+        c->rms_fresh = true;                    // the trajectory in memory no longer ends in the end state
+        c->launches += 1;
+        return IQGPU_OK;
+    }
+    if (first_output > c->rms_n) {             // beyond the call: nothing to do
         if (dev_changed) CK(cudaMemsetAsync(dev_changed, 0, sizeof(int), st));
         return IQGPU_OK;
     }
     if (!c->d_rms_resume) CK(cudaMalloc(&c->d_rms_resume, sizeof(AgcRmsResume)));
+    // A resume compares its trajectory with the checkpoints of the one in memory and stops where the two meet.  Behind an
+    // earlier resume's frame that trajectory is the earlier resume's, while the rows in front of the frame still hold the
+    // call's own: a resume in front of it would meet the call's trajectory and stop, and leave the earlier resume's
+    // outputs behind.  So it first re-runs the call from the state the call started from (outputs, checkpoints and block
+    // end states as the call left them; *d_agc keeps the end state the resume compares with for `dev_changed`), and then
+    // converts the whole call again.  Resumes at the same or a later frame, the time-shard hand-over, need none of this.
+    const bool rerun = first_output < c->rms_resume_max;
+    if (rerun) {
+        AgcState* s = c->d_rms_rerun + 1;         // [0] keeps the start state for the next re-run
+        CK(cudaMemcpyAsync(&s->rms_g, &c->d_rms_rerun->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        CK(launch_agc_rms(c->rms_src, c->rms_n, c->rms_qp, s, c->d_agc_scratch, c->d_agc_ws, st));
+    }
     CK(launch_agc_rms_resume(c->rms_src, c->rms_n, c->rms_qp, c->d_agc, c->d_agc_scratch, c->d_agc_ws, first_output,
-                             reinterpret_cast<const float2*>(dev_state), c->d_rms_resume, c->rms_fresh, dev_changed, st));
+                             reinterpret_cast<const float2*>(dev_state), c->d_rms_resume, c->rms_fresh || rerun, dev_changed,
+                             st));
     c->rms_fresh = false;
-    CK(launch_convert_range(c->d_agc_scratch, c->d_rms_resume, c->cfg.output_format, dev_out, st));
-    c->launches += 2;
+    c->rms_resume_max = rerun ? first_output : std::max(c->rms_resume_max, first_output);
+    if (rerun) CK(launch_post(c->d_agc_scratch, c->rms_n, c->rms_qp, nullptr, 0, nullptr, 1, nullptr, dev_out, st));
+    else CK(launch_convert_range(c->d_agc_scratch, c->d_rms_resume, c->cfg.output_format, dev_out, st));
+    c->launches += rerun ? 3 : 2;
     return IQGPU_OK;
 }
 

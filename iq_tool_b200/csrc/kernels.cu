@@ -1179,16 +1179,8 @@ __global__ void __launch_bounds__(AGC_SCAN_THREADS) agc_digital_scan_kernel(cons
 // log(y) and exp(t) in double with short dependency chains (the recurrence is latency bound: one thread
 // walks its block sample by sample).  Both are accurate to ~1 ulp of double, so rounding them to float
 // gives the correctly rounded logf/expf result (checked against libm on 2e7 arguments; the rounding can
-// differ only when the exact value lies within 1e-15 of a float rounding boundary).
-__device__ __forceinline__ double agc_exp_small(double t)   // |t| <= 0.5 (t = -alpha/2 * log(y2'), alpha <= 1e-2)
-{
-    double p = 1.0 / 6227020800.0;
-    p = fma(p, t, 1.0 / 479001600.0); p = fma(p, t, 1.0 / 39916800.0); p = fma(p, t, 1.0 / 3628800.0);
-    p = fma(p, t, 1.0 / 362880.0);    p = fma(p, t, 1.0 / 40320.0);    p = fma(p, t, 1.0 / 5040.0);
-    p = fma(p, t, 1.0 / 720.0);       p = fma(p, t, 1.0 / 120.0);      p = fma(p, t, 1.0 / 24.0);
-    p = fma(p, t, 1.0 / 6.0);         p = fma(p, t, 0.5);              p = fma(p, t, 1.0);
-    return fma(p, t, 1.0);
-}
+// differ only when the exact value lies within 1e-15 of a float rounding boundary).  The functions are in agc_math.h,
+// shared with the serial reference the tests compare against (tests/native/agc_rms_serial.cpp).
 
 __constant__ AgcLogEntry agc_log_tab_c[AGC_LOG_N];
 __constant__ double agc_coef_c[AGC_NCOEF] = AGC_COEF_LIST;
