@@ -196,6 +196,19 @@ int  iqgpu_chain_process_device(iqgpu_chain *c, const void *dev_raw_in, size_t n
                                 const uint32_t *chunk_frames, size_t n_chunks,
                                 void *dev_out, size_t out_capacity_bytes, size_t *out_frames,
                                 uint32_t *per_chunk_out, void *cuda_stream);
+/* Several channels out of one capture: K chains consume the same host-memory train, which is copied H2D once per
+ * sub-train (into chains[0]'s staging) and processed by every chain, each on its own streams, into its own output.
+ * out[k] / out_capacity_bytes[k] / out_frames[k] / per_chunk_out[k] (the array or an entry may be NULL) belong to
+ * chains[k]; channel k's output, per-chunk counts and state are those of iqgpu_chain_process on chains[k] alone.
+ * The train is cut into sub-trains of the smallest subtrain_frames of the chains.  Before any work is queued the call
+ * refuses (IQGPU_EINVAL, the message names the channel and the field) zero chains, a NULL or repeated handle, chains
+ * on different devices, a different input_format or input_rate_hz, a different chunk_frames option when the chunk
+ * lengths are implicit, and a chain with a begun process_device call pending; then plan-only chains
+ * (IQGPU_ENODEVICE) and a channel whose output does not fit (IQGPU_ECAPACITY).  iqgpu_chain_process is the K = 1
+ * case. */
+int  iqgpu_chain_process_multi(iqgpu_chain *const *chains, size_t n_chains, const void *raw_in, size_t n_frames,
+                               const uint32_t *chunk_frames, size_t n_chunks, void *const *out,
+                               const size_t *out_capacity_bytes, size_t *out_frames, uint32_t *const *per_chunk_out);
 /* closed form: resampler output frames after `frames_in` input frames since reset
  * (msresamp_crcf_execute's cumulative *num_written, src/resampler.c:49) */
 int  iqgpu_chain_resampler_outputs_after(iqgpu_chain *c, uint64_t frames_in, uint64_t *frames_out);
@@ -313,6 +326,12 @@ typedef struct {
 int         iqgpu_rawfile_run(const iqgpu_chain_config *cfg, int device, const char *in_path, const char *out_path,
                               size_t train_chunks /* reference chunks per chain call, 0 = 64 */,
                               iqgpu_rawfile_stats *stats /* optional */);
+/* Several channels out of one raw file (see iqgpu_chain_process_multi): the file is read once, chain k is built from
+ * cfgs[k] and writes out_paths[k]; stats (optional) receives one record per channel.  Every output is opened before
+ * anything is read: if one cannot be, the call fails naming its path and removes the outputs it had opened. */
+int         iqgpu_rawfile_run_channels(const iqgpu_chain_config *cfgs, size_t n_channels, int device, const char *in_path,
+                                       const char *const *out_paths, size_t train_chunks,
+                                       iqgpu_rawfile_stats *stats /* [n_channels] or NULL */);
 const char *iqgpu_rawfile_last_error(void);
 
 /* ---- WAV / RF64 containers around the path (SURVEY.md 8(f) rank 4): the WAV input module
@@ -380,6 +399,13 @@ int  iqgpu_wav_build_header(int container, int output_format, int sample_rate_hz
 int  iqgpu_wavfile_run(const iqgpu_chain_config *cfg, int device, const char *in_path, int in_container,
                        const char *out_path, int out_container, float center_target_hz, size_t train_chunks,
                        iqgpu_rawfile_stats *stats /* optional */, iqgpu_wav_info *in_info /* optional */);
+/* The same with several channels out of one input (iqgpu_rawfile_run_channels): a WAV / RF64 input gives every
+ * channel its format and rate, a non-zero center_target_hz[k] turns its centre frequency into channel k's shift, and
+ * each container output carries its own channel's rate.  iqgpu_wavfile_run is the one-channel case. */
+int  iqgpu_wavfile_run_channels(const iqgpu_chain_config *cfgs, size_t n_channels, int device, const char *in_path,
+                                int in_container, const char *const *out_paths, const int *out_containers,
+                                const float *center_target_hz /* [n_channels] or NULL */, size_t train_chunks,
+                                iqgpu_rawfile_stats *stats /* [n_channels] or NULL */, iqgpu_wav_info *in_info /* optional */);
 
 /* ---- sample_convert.h (include/sample_convert.h:19,35,50) — host buffers ------------- */
 size_t iqgpu_get_bytes_per_sample(int format);

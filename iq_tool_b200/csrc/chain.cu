@@ -1795,66 +1795,127 @@ int iqgpu_chain_process(iqgpu_chain* c, const void* raw_in, size_t n_frames, con
                         void* out, size_t out_capacity_bytes, size_t* out_frames, uint32_t* per_chunk_out)
 {
     if (!c || !out_frames) return fail(IQGPU_EINVAL, "null argument");
-    if (c->plan_only) return fail(IQGPU_ENODEVICE, "chain was created without a device (plan only)");
-    *out_frames = 0;
+    return iqgpu_chain_process_multi(&c, 1, raw_in, n_frames, chunk_frames, n_chunks, &out, &out_capacity_bytes, out_frames,
+                                     &per_chunk_out);
+}
+
+int iqgpu_chain_process_multi(iqgpu_chain* const* chains, size_t K, const void* raw_in, size_t n_frames,
+                              const uint32_t* chunk_frames, size_t n_chunks, void* const* out, const size_t* out_capacity_bytes,
+                              size_t* out_frames, uint32_t* const* per_chunk_out)
+{
+    if (!chains || !out || !out_capacity_bytes || !out_frames) return fail(IQGPU_EINVAL, "null argument");
+    if (K == 0) return fail(IQGPU_EINVAL, "n_chains must be at least 1");
+    // every check that needs no device runs first, so that it fails the same way without one
+    auto chan = [K](size_t k) { return K == 1 ? std::string() : "channel " + std::to_string(k) + ": "; };
+    auto bad = [&](size_t k, const std::string& m) { return fail(IQGPU_EINVAL, chan(k) + m); };
+    iqgpu_chain* const c0 = chains[0];
+    for (size_t k = 0; k < K; k++) {
+        iqgpu_chain* c = chains[k];
+        if (!c) return bad(k, "null chain handle");
+        for (size_t j = 0; j < k; j++)
+            if (chains[j] == c) return bad(k, "chain handle already listed as channel " + std::to_string(j));
+        if (c->device != c0->device) return bad(k, "device differs from channel 0's");
+        if (c->cfg.input_format != c0->cfg.input_format) return bad(k, "input_format differs from channel 0's");
+        if (c->cfg.input_rate_hz != c0->cfg.input_rate_hz) return bad(k, "input_rate_hz differs from channel 0's");
+        if (!chunk_frames && c->chunk_frames != c0->chunk_frames) return bad(k, "chunk_frames option differs from channel 0's");
+        if (c->pend.active) return bad(k, "a begun process_device call is still pending (call process_device_finish)");
+    }
+    for (size_t k = 0; k < K; k++)
+        if (chains[k]->plan_only) return fail(IQGPU_ENODEVICE, "chain was created without a device (plan only)");
+    for (size_t k = 0; k < K; k++) out_frames[k] = 0;
     if (n_frames == 0) return IQGPU_OK;
-    if (!raw_in || !out) return fail(IQGPU_EINVAL, "null buffer");
-    CK(cudaSetDevice(c->device));
-    int rc = c->ensure_buffers();
-    if (rc) return rc;
+    if (!raw_in) return fail(IQGPU_EINVAL, "null buffer");
+    for (size_t k = 0; k < K; k++)
+        if (!out[k]) return bad(k, "null buffer");
+    CK(cudaSetDevice(c0->device));
+    int rc;
+    size_t sub = SIZE_MAX;          // the sub-train partition every chain can take
+    for (size_t k = 0; k < K; k++) {
+        rc = chains[k]->ensure_buffers();
+        if (rc) return rc;
+        sub = std::min(sub, chains[k]->subtrain_frames);
+    }
     std::vector<uint32_t> chunks;
-    rc = build_chunks(c, n_frames, chunk_frames, n_chunks, chunks);
+    rc = build_chunks(c0, n_frames, chunk_frames, n_chunks, chunks);
     if (rc) return rc;
     for (auto f : chunks)
-        if (f > c->subtrain_frames) return fail(IQGPU_EINVAL, "a chunk exceeds subtrain_frames");
-    if (c->count_outputs(chunks.data(), chunks.size(), nullptr) * c->out_bps > out_capacity_bytes)
-        return fail(IQGPU_ECAPACITY, "output buffer too small");
-    // staging slots sized for one sub-train
-    const size_t raw_need = (c->subtrain_frames + 16) * c->in_bps, out_need = c->max_out_for(c->subtrain_frames) * c->out_bps;
-    if (c->d_raw_bytes < raw_need || c->d_out_bytes < out_need) {
-        for (int i = 0; i < 2; i++) {
-            cudaFree(c->d_raw[i]); cudaFree(c->d_out[i]);
-            CK(cudaMalloc(&c->d_raw[i], raw_need));
-            CK(cudaMalloc(&c->d_out[i], out_need));
-        }
-        c->d_raw_bytes = raw_need; c->d_out_bytes = out_need;
+        if (f > sub) return fail(IQGPU_EINVAL, "a chunk exceeds subtrain_frames");
+    for (size_t k = 0; k < K; k++) {
+        iqgpu_chain* c = chains[k];
+        if (c->count_outputs(chunks.data(), chunks.size(), nullptr) * c->out_bps > out_capacity_bytes[k])
+            return fail(IQGPU_ECAPACITY, chan(k) + "output buffer too small");
     }
-    rc = c->order_after_reset(c->stream);
-    if (rc) return rc;
-    c->last_stream = c->stream;
-    for (auto& t : c->tap) t.len = 0;
-    size_t ci = 0, in_off = 0, out_off = 0, total = 0;
-    uint32_t launches = 0;
+    // staging slots sized for one sub-train: the raw input in channel 0's, each channel's output in its own
+    const size_t raw_need = (sub + 16) * c0->in_bps;
+    if (c0->d_raw_bytes < raw_need) {
+        c0->d_raw_bytes = 0;
+        for (int i = 0; i < 2; i++) {
+            cudaFree(c0->d_raw[i]);
+            c0->d_raw[i] = nullptr;
+            CK(cudaMalloc(&c0->d_raw[i], raw_need));
+        }
+        c0->d_raw_bytes = raw_need;
+    }
+    for (size_t k = 0; k < K; k++) {
+        iqgpu_chain* c = chains[k];
+        const size_t out_need = c->max_out_for(sub) * c->out_bps;
+        if (c->d_out_bytes < out_need) {
+            c->d_out_bytes = 0;
+            for (int i = 0; i < 2; i++) {
+                cudaFree(c->d_out[i]);
+                c->d_out[i] = nullptr;
+                CK(cudaMalloc(&c->d_out[i], out_need));
+            }
+            c->d_out_bytes = out_need;
+        }
+        rc = c->order_after_reset(c->stream);
+        if (rc) return rc;
+        c->last_stream = c->stream;
+        for (auto& t : c->tap) t.len = 0;
+    }
+    std::vector<size_t> out_off(K, 0), total(K, 0);
+    std::vector<uint32_t> launches(K, 0);
+    size_t ci = 0, in_off = 0;
     int slot = 0;
     bool used[2] = {false, false};
     while (ci < chunks.size()) {
         size_t cj = ci, n = 0;
-        while (cj < chunks.size() && n + chunks[cj] <= c->subtrain_frames) { n += chunks[cj]; cj++; }
-        // H2D of this sub-train (waits until the slot's previous D2H finished)
-        if (used[slot]) CK(cudaStreamWaitEvent(c->h2d, c->ev_d2h[slot], 0));
-        CK(cudaMemcpyAsync(c->d_raw[slot], (const char*)raw_in + in_off * c->in_bps, n * c->in_bps, cudaMemcpyHostToDevice, c->h2d));
-        CK(cudaEventRecord(c->ev_h2d[slot], c->h2d));
-        CK(cudaStreamWaitEvent(c->stream, c->ev_h2d[slot], 0));
-        size_t produced = 0;
-        c->dc_slot = 0; c->dc_prepared = false;      // host path is PCIe bound: DC pre-pass inline on the compute stream
-        rc = c->run_subtrain(c->d_raw[slot], n, chunks.data() + ci, cj - ci, c->d_out[slot], &produced,
-                             per_chunk_out ? per_chunk_out + ci : nullptr, c->stream);
-        if (rc) return rc;
-        launches += c->launches;
-        CK(cudaEventRecord(c->ev_done[slot], c->stream));
-        CK(cudaStreamWaitEvent(c->d2h, c->ev_done[slot], 0));
-        if (produced)
-            CK(cudaMemcpyAsync((char*)out + out_off, c->d_out[slot], produced * c->out_bps, cudaMemcpyDeviceToHost, c->d2h));
-        CK(cudaEventRecord(c->ev_d2h[slot], c->d2h));
+        while (cj < chunks.size() && n + chunks[cj] <= sub) { n += chunks[cj]; cj++; }
+        // H2D of this sub-train: the raw slot is rewritten only after every channel's D2H out of this slot index finished,
+        // which follows that channel's compute on the slot's previous contents
+        if (used[slot])
+            for (size_t k = 0; k < K; k++) CK(cudaStreamWaitEvent(c0->h2d, chains[k]->ev_d2h[slot], 0));
+        CK(cudaMemcpyAsync(c0->d_raw[slot], (const char*)raw_in + in_off * c0->in_bps, n * c0->in_bps, cudaMemcpyHostToDevice, c0->h2d));
+        CK(cudaEventRecord(c0->ev_h2d[slot], c0->h2d));
+        for (size_t k = 0; k < K; k++) {
+            iqgpu_chain* c = chains[k];
+            CK(cudaStreamWaitEvent(c->stream, c0->ev_h2d[slot], 0));
+            size_t produced = 0;
+            c->dc_slot = 0; c->dc_prepared = false;      // host path is PCIe bound: DC pre-pass inline on the compute stream
+            uint32_t* pc = per_chunk_out ? per_chunk_out[k] : nullptr;
+            rc = c->run_subtrain(c0->d_raw[slot], n, chunks.data() + ci, cj - ci, c->d_out[slot], &produced,
+                                 pc ? pc + ci : nullptr, c->stream);
+            if (rc) return rc;
+            launches[k] += c->launches;
+            CK(cudaEventRecord(c->ev_done[slot], c->stream));
+            CK(cudaStreamWaitEvent(c->d2h, c->ev_done[slot], 0));
+            if (produced)
+                CK(cudaMemcpyAsync((char*)out[k] + out_off[k], c->d_out[slot], produced * c->out_bps, cudaMemcpyDeviceToHost, c->d2h));
+            CK(cudaEventRecord(c->ev_d2h[slot], c->d2h));
+            out_off[k] += produced * c->out_bps; total[k] += produced;
+        }
         used[slot] = true;
-        in_off += n; out_off += produced * c->out_bps; total += produced;
+        in_off += n;
         ci = cj; slot ^= 1;
     }
-    CK(cudaStreamSynchronize(c->d2h));
-    CK(cudaStreamSynchronize(c->stream));
-    c->launches = launches;
-    c->rms_ready = false;                            // the output went through the staging slots, not a caller's buffer
-    *out_frames = total;
+    for (size_t k = 0; k < K; k++) {
+        iqgpu_chain* c = chains[k];
+        CK(cudaStreamSynchronize(c->d2h));
+        CK(cudaStreamSynchronize(c->stream));
+        c->launches = launches[k];
+        c->rms_ready = false;                        // the output went through the staging slots, not a caller's buffer
+        out_frames[k] = total[k];
+    }
     return IQGPU_OK;
 }
 

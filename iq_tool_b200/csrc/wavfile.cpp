@@ -631,15 +631,30 @@ int iqgpu_wav_build_header(int container, int output_format, int sample_rate_hz,
     return IQGPU_OK;
 }
 
-int iqgpu_wavfile_run(const iqgpu_chain_config* cfg_in, int device, const char* in_path, int in_container, const char* out_path,
+int iqgpu_wavfile_run(const iqgpu_chain_config* cfg, int device, const char* in_path, int in_container, const char* out_path,
                       int out_container, float center_target_hz, size_t train_chunks, iqgpu_rawfile_stats* stats, iqgpu_wav_info* in_info)
 {
-    if (!cfg_in || !in_path || !out_path) return fail("null argument");
-    if (in_container < IQGPU_CONTAINER_RAW || in_container > IQGPU_CONTAINER_RF64 || out_container < IQGPU_CONTAINER_RAW || out_container > IQGPU_CONTAINER_RF64)
-        return fail("unknown container");
-    if (stats) memset(stats, 0, sizeof(*stats));
+    return iqio::wavfile_run(cfg, 1, device, in_path, in_container, &out_path, &out_container, &center_target_hz, train_chunks,
+                             stats, in_info, iqio::process_one);
+}
+
+}  // extern "C"
+
+int iqio::wavfile_run(const iqgpu_chain_config* cfgs_in, size_t n, int device, const char* in_path, int in_container,
+                      const char* const* out_paths, const int* out_containers, const float* center_target_hz, size_t train_chunks,
+                      iqgpu_rawfile_stats* stats, iqgpu_wav_info* in_info, ProcessFn process)
+{
+    if (!cfgs_in || !in_path || !out_paths || !out_containers) return fail("null argument");
+    if (n == 0) return fail("n_channels must be at least 1");
+    if (in_container < IQGPU_CONTAINER_RAW || in_container > IQGPU_CONTAINER_RF64) return fail("unknown container");
+    for (size_t k = 0; k < n; k++) {
+        if (!out_paths[k]) return fail(channel_prefix(k, n) + "null argument");
+        if (out_containers[k] < IQGPU_CONTAINER_RAW || out_containers[k] > IQGPU_CONTAINER_RF64) return fail(channel_prefix(k, n) + "unknown container");
+    }
+    if (stats) memset(stats, 0, n * sizeof(*stats));
     if (in_info) memset(in_info, 0, sizeof(*in_info));
-    iqgpu_chain_config cfg = *cfg_in;
+    std::vector<iqgpu_chain_config> cfgs(cfgs_in, cfgs_in + n);
+    auto target = [&](size_t k) { return center_target_hz ? center_target_hz[k] : 0.0f; };
 
     FILE* fin = fopen(in_path, "rb");
     if (!fin) return fail(std::string("Error opening input file: ") + in_path);
@@ -647,49 +662,66 @@ int iqgpu_wavfile_run(const iqgpu_chain_config* cfg_in, int device, const char* 
     if (in_container != IQGPU_CONTAINER_RAW) {
         iqgpu_wav_info wi;
         int rc = probe_stream(fin, in_path, &wi);
-        if (!rc) rc = iqgpu_wav_center_target_shift(&wi, center_target_hz, cfg.freq_shift_hz, &cfg.freq_shift_hz);
+        for (size_t k = 0; k < n && !rc; k++) {
+            rc = iqgpu_wav_center_target_shift(&wi, target(k), cfgs[k].freq_shift_hz, &cfgs[k].freq_shift_hz);
+            if (rc && n > 1) iqio::set_last_error(channel_prefix(k, n) + iqgpu_rawfile_last_error());
+        }
         if (in_info) *in_info = wi;
         if (rc) { fclose(fin); return rc; }
-        cfg.input_format = wi.sample_format;                    // src/input_wav.c:575-577
-        cfg.input_rate_hz = (double)wi.sample_rate_hz;          // :597
+        for (auto& cfg : cfgs) {
+            cfg.input_format = wi.sample_format;                // src/input_wav.c:575-577
+            cfg.input_rate_hz = (double)wi.sample_rate_hz;      // :597
+        }
         in_limit = wi.data_bytes;
         if (fseeko(fin, (off_t)wi.data_offset, SEEK_SET) != 0) { fclose(fin); return fail(std::string("cannot seek in ") + in_path); }
-    } else if (center_target_hz != 0.0f) {
-        fclose(fin);
-        return fail("Option --wav-center-target-freq needs a WAV input");
+    } else {
+        for (size_t k = 0; k < n; k++)
+            if (target(k) != 0.0f) { fclose(fin); return fail(channel_prefix(k, n) + "Option --wav-center-target-freq needs a WAV input"); }
     }
-    // setup.c:99: with --no-resample the target rate IS the source rate (known only now for a WAV input)
-    if (cfg.no_resample) cfg.target_rate_hz = (double)(int)cfg.input_rate_hz;
-    // output side: wav_common_validate_options + wav_common_initialize (src/output_wav_common.c:46-118)
-    unsigned char header[80];
-    const size_t header_bytes = iqgpu_wav_header_bytes(out_container);
-    if (header_bytes) {
-        const int rc = iqgpu_wav_build_header(out_container, cfg.output_format, (int)cfg.target_rate_hz, 0, header, sizeof(header));
-        if (rc) { fclose(fin); return rc; }
+    // output side: wav_common_validate_options + wav_common_initialize (src/output_wav_common.c:46-118), one header per channel
+    std::vector<unsigned char> headers(80 * n);
+    std::vector<size_t> header_bytes(n);
+    for (size_t k = 0; k < n; k++) {
+        iqgpu_chain_config& cfg = cfgs[k];
+        // setup.c:99: with --no-resample the target rate IS the source rate (known only now for a WAV input)
+        if (cfg.no_resample) cfg.target_rate_hz = (double)(int)cfg.input_rate_hz;
+        header_bytes[k] = iqgpu_wav_header_bytes(out_containers[k]);
+        if (header_bytes[k]) {
+            const int rc = iqgpu_wav_build_header(out_containers[k], cfg.output_format, (int)cfg.target_rate_hz, 0, &headers[80 * k], 80);
+            if (rc) {
+                if (n > 1) iqio::set_last_error(channel_prefix(k, n) + iqgpu_rawfile_last_error());
+                fclose(fin);
+                return rc;
+            }
+        }
     }
 
-    iqgpu_chain* chain = nullptr;
-    int rc = iqgpu_chain_create(&cfg, device, &chain);
-    if (rc) { iqio::set_last_error(iqgpu_last_error()); fclose(fin); return rc; }
-    FILE* fout = fopen(out_path, "wb");
-    if (!fout) { fclose(fin); iqgpu_chain_destroy(chain); return fail(std::string("Error opening output WAV file ") + out_path); }
-
+    Channels ch;
+    ch.process = process;
     std::string err;
-    iqgpu_rawfile_stats st;
-    memset(&st, 0, sizeof(st));
-    if (header_bytes && fwrite(header, 1, header_bytes, fout) != header_bytes) { rc = IQGPU_EINVAL; err = "write error on the output file"; }
-    if (!rc) rc = iqio::run_stream(chain, &cfg, fin, in_limit, fout, train_chunks, &st, err);
-    if (!rc && header_bytes) {
+    int rc = ch.open(cfgs.data(), n, device, out_paths, "Error opening output WAV file ", err);
+    if (rc) { fclose(fin); iqio::set_last_error(err); return rc; }
+    std::vector<iqgpu_rawfile_stats> st(n);
+    memset(st.data(), 0, n * sizeof(st[0]));
+    for (size_t k = 0; k < n && !rc; k++)
+        if (header_bytes[k] && fwrite(&headers[80 * k], 1, header_bytes[k], ch.fouts[k]) != header_bytes[k]) {
+            rc = IQGPU_EINVAL;
+            err = channel_prefix(k, n) + "write error on the output file";
+        }
+    if (!rc) rc = iqio::run_stream(ch, cfgs.data(), fin, in_limit, train_chunks, st.data(), err);
+    for (size_t k = 0; k < n && !rc; k++) {
+        if (!header_bytes[k]) continue;
         // what sf_close does: the sizes now that they are known
-        iqgpu_wav_build_header(out_container, cfg.output_format, (int)cfg.target_rate_hz, st.bytes_written, header, sizeof(header));
-        if (fseeko(fout, 0, SEEK_SET) != 0 || fwrite(header, 1, header_bytes, fout) != header_bytes) { rc = IQGPU_EINVAL; err = "cannot finalise the output header"; }
+        iqgpu_wav_build_header(out_containers[k], cfgs[k].output_format, (int)cfgs[k].target_rate_hz, st[k].bytes_written, &headers[80 * k], 80);
+        if (fseeko(ch.fouts[k], 0, SEEK_SET) != 0 || fwrite(&headers[80 * k], 1, header_bytes[k], ch.fouts[k]) != header_bytes[k]) {
+            rc = IQGPU_EINVAL;
+            err = channel_prefix(k, n) + "cannot finalise the output header";
+        }
     }
-    if (fclose(fout) != 0 && !rc) { rc = IQGPU_EINVAL; err = "write error on the output file"; }
+    const int rc_close = ch.close(err);
+    if (!rc) rc = rc_close;
     fclose(fin);
-    iqgpu_chain_destroy(chain);
-    if (stats) *stats = st;
+    if (stats) memcpy(stats, st.data(), n * sizeof(st[0]));
     if (rc) iqio::set_last_error(err);
     return rc;
 }
-
-}  // extern "C"

@@ -115,6 +115,8 @@ def _load() -> C.CDLL:
     lib.iqgpu_chain_get_kernel_times.argtypes = [vp, C.POINTER(C.c_double), u32p, C.c_int]
     lib.iqgpu_chain_process.argtypes = [vp, vp, sz, u32p, sz, vp, sz, C.POINTER(sz), u32p]
     lib.iqgpu_chain_process_device.argtypes = [vp, vp, sz, u32p, sz, vp, sz, C.POINTER(sz), u32p, vp]
+    lib.iqgpu_chain_process_multi.argtypes = [C.POINTER(vp), sz, vp, sz, u32p, sz, C.POINTER(vp), C.POINTER(sz),
+                                              C.POINTER(sz), C.POINTER(u32p)]
     lib.iqgpu_chain_predict_output.argtypes = [vp, sz, C.POINTER(sz)]
     lib.iqgpu_chain_read_tap.argtypes = [vp, C.c_int, vp, sz, C.POINTER(sz)]
     lib.iqgpu_chain_get_filter_taps.argtypes = [vp, vp, C.c_uint32, u32p]
@@ -139,6 +141,9 @@ def _load() -> C.CDLL:
     lib.iqgpu_agc_digital_advance.argtypes = [C.POINTER(AgcStateC), C.c_float, C.c_double, vp, vp, sz, vp]
     lib.iqgpu_rawfile_run.restype = C.c_int
     lib.iqgpu_rawfile_run.argtypes = [C.POINTER(ChainConfigC), C.c_int, C.c_char_p, C.c_char_p, sz, C.POINTER(RawfileStatsC)]
+    lib.iqgpu_rawfile_run_channels.restype = C.c_int
+    lib.iqgpu_rawfile_run_channels.argtypes = [C.POINTER(ChainConfigC), sz, C.c_int, C.c_char_p, C.POINTER(C.c_char_p), sz,
+                                               C.POINTER(RawfileStatsC)]
     lib.iqgpu_rawfile_last_error.restype = C.c_char_p
     lib.iqgpu_wav_probe.argtypes = [C.c_char_p, C.POINTER(WavInfoC)]
     lib.iqgpu_wav_parse_auxi.argtypes = [C.c_char_p, sz, C.POINTER(WavInfoC)]
@@ -149,8 +154,12 @@ def _load() -> C.CDLL:
     lib.iqgpu_wav_build_header.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint64, vp, sz]
     lib.iqgpu_wavfile_run.argtypes = [C.POINTER(ChainConfigC), C.c_int, C.c_char_p, C.c_int, C.c_char_p, C.c_int,
                                       C.c_float, sz, C.POINTER(RawfileStatsC), C.POINTER(WavInfoC)]
+    lib.iqgpu_wavfile_run_channels.argtypes = [C.POINTER(ChainConfigC), sz, C.c_int, C.c_char_p, C.c_int,
+                                               C.POINTER(C.c_char_p), C.POINTER(C.c_int), C.POINTER(C.c_float), sz,
+                                               C.POINTER(RawfileStatsC), C.POINTER(WavInfoC)]
     for name in ("iqgpu_wav_probe", "iqgpu_wav_parse_auxi", "iqgpu_wav_parse_filename",
-                 "iqgpu_wav_center_target_shift", "iqgpu_wav_build_header", "iqgpu_wavfile_run"):
+                 "iqgpu_wav_center_target_shift", "iqgpu_wav_build_header", "iqgpu_wavfile_run",
+                 "iqgpu_wavfile_run_channels"):
         getattr(lib, name).restype = C.c_int
     lib.iqgpu_ubench_fp32_peak.restype = C.c_int
     lib.iqgpu_ubench_fp32_peak.argtypes = [C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]
@@ -162,6 +171,7 @@ def _load() -> C.CDLL:
                                       C.POINTER(C.c_float), C.POINTER(C.c_float)]
     for name in ("iqgpu_chain_reset", "iqgpu_chain_restart", "iqgpu_chain_get_info", "iqgpu_chain_set_option",
                  "iqgpu_chain_set_iq_factors", "iqgpu_chain_process", "iqgpu_chain_process_device",
+                 "iqgpu_chain_process_multi",
                  "iqgpu_chain_predict_output", "iqgpu_chain_read_tap", "iqgpu_chain_get_filter_taps",
                  "iqgpu_chain_get_halfband_taps", "iqgpu_chain_get_arb_taps", "iqgpu_chain_seek",
                  "iqgpu_chain_halo_frames", "iqgpu_chain_resampler_outputs_after",
@@ -412,6 +422,31 @@ class Chain:
         return out
 
 
+def process_channels(chains: Sequence[Chain], raw: np.ndarray, chunk_frames: Optional[Sequence[int]] = None,
+                     return_chunk_counts: bool = False):
+    """Several channels out of one host buffer: every chain processes the same input, which crosses PCIe once per
+    sub-train (iqgpu_chain_process_multi).  Returns one output array per chain, as Chain.process would (with
+    return_chunk_counts, one (output, per-chunk counts) pair per chain)."""
+    chains = list(chains)
+    K = len(chains)
+    raw = np.ascontiguousarray(raw)
+    n_frames = raw.nbytes // chains[0].cfg.in_bytes if K else 0
+    outs = [np.zeros(ch.out_capacity_frames(n_frames) * ch.cfg.out_bytes, dtype=np.uint8) for ch in chains]
+    cptr, ncz, keep = chains[0]._chunks(chunk_frames) if K else (None, 0, None)
+    nchunks = ncz if chunk_frames is not None else (n_frames + 16383) // 16384
+    counts = [np.zeros(max(1, nchunks), dtype=np.uint32) for _ in chains]
+    handles = (C.c_void_p * max(1, K))(*[ch._h for ch in chains])
+    out_ptrs = (C.c_void_p * max(1, K))(*[o.ctypes.data for o in outs])
+    caps = (C.c_size_t * max(1, K))(*[o.nbytes for o in outs])
+    nout = (C.c_size_t * max(1, K))()
+    count_ptrs = (C.POINTER(C.c_uint32) * max(1, K))(*[c.ctypes.data_as(C.POINTER(C.c_uint32)) for c in counts])
+    _check(lib.iqgpu_chain_process_multi(handles, K, raw.ctypes.data, n_frames, cptr, ncz, out_ptrs, caps, nout,
+                                         count_ptrs))
+    res = [o[: nout[k] * ch.cfg.out_bytes].view(NUMPY_DTYPE[ch.cfg.output_format])
+           for k, (o, ch) in enumerate(zip(outs, chains))]
+    return [(r, c[:nchunks]) for r, c in zip(res, counts)] if return_chunk_counts else res
+
+
 def convert_block_to_cf32(raw: np.ndarray, fmt_code: int, n_frames: int, gain: float) -> np.ndarray:
     raw = np.ascontiguousarray(raw)
     out = np.zeros(n_frames, dtype=np.complex64)
@@ -466,6 +501,23 @@ def rawfile_run(cfg: ChainConfig, in_path: str, out_path: str, device: int = 0, 
     return st
 
 
+def _paths(paths: Sequence[str]):
+    return (C.c_char_p * max(1, len(paths)))(*[os.fsencode(p) for p in paths])
+
+
+def rawfile_run_channels(cfgs: Sequence[ChainConfig], in_path: str, out_paths: Sequence[str], device: int = 0,
+                         train_chunks: int = 0) -> list[RawfileStatsC]:
+    """Several channels out of one raw I/Q file: read once, one chain per config, one output file per channel.
+    Returns one stats record per channel."""
+    K = len(cfgs)
+    if len(out_paths) != K:
+        raise ValueError("one output path per configuration")
+    cs = (ChainConfigC * max(1, K))(*[c.to_c() for c in cfgs])
+    st = (RawfileStatsC * max(1, K))()
+    _io_check(lib.iqgpu_rawfile_run_channels(cs, K, device, os.fsencode(in_path), _paths(out_paths), train_chunks, st))
+    return list(st)[:K]
+
+
 def _io_check(rc: int) -> None:
     if rc != 0:
         raise IqGpuError(rc, lib.iqgpu_rawfile_last_error().decode("utf-8", "replace"))
@@ -511,3 +563,24 @@ def wavfile_run(cfg: ChainConfig, in_path: str, out_path: str, in_container: int
                                out_container, center_target_hz, train_chunks, C.byref(st), C.byref(info))
     _io_check(rc)
     return st, info
+
+
+def wavfile_run_channels(cfgs: Sequence[ChainConfig], in_path: str, out_paths: Sequence[str],
+                         in_container: int = CONTAINER_WAV, out_containers: Sequence[int] | int = CONTAINER_WAV,
+                         center_targets_hz: Optional[Sequence[float]] = None, device: int = 0,
+                         train_chunks: int = 0) -> tuple[list[RawfileStatsC], WavInfoC]:
+    """wavfile_run with several channels out of one input: a WAV input gives every channel its format and rate, a
+    non-zero centre target turns the file's centre frequency into that channel's shift.  Returns one stats record per
+    channel and the probe of the input."""
+    K = len(cfgs)
+    if isinstance(out_containers, int):
+        out_containers = [out_containers] * K
+    if len(out_paths) != K or len(out_containers) != K or (center_targets_hz is not None and len(center_targets_hz) != K):
+        raise ValueError("one output path, container and centre target per configuration")
+    cs = (ChainConfigC * max(1, K))(*[c.to_c() for c in cfgs])
+    conts = (C.c_int * max(1, K))(*out_containers)
+    targets = (C.c_float * max(1, K))(*center_targets_hz) if center_targets_hz is not None else None
+    st, info = (RawfileStatsC * max(1, K))(), WavInfoC()
+    _io_check(lib.iqgpu_wavfile_run_channels(cs, K, device, os.fsencode(in_path), in_container, _paths(out_paths), conts,
+                                             targets, train_chunks, st, C.byref(info)))
+    return list(st)[:K], info
