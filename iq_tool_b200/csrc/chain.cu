@@ -16,10 +16,12 @@
 #include <cstring>
 #include <string>
 #include <exception>
+#include <memory>
 #include <new>
 #include <vector>
 
 #include "../../include/iqgpu.h"
+#include "cuda_owned.hpp"
 #include "design.hpp"
 #include "kernels.hpp"
 
@@ -60,35 +62,32 @@ bool is_complex_format(int fmt) { return fmt >= IQGPU_FMT_CU8 && fmt <= IQGPU_FM
 // cf32 stream segment with history head-room.  New data of a call is written at base+pos; the
 // previous `hist` samples sit right below it.
 struct DevStream {
-    float2* base = nullptr;
-    size_t cap = 0, hist = 0, pos = 0, max_n = 0, slack = 0;   // slack: readable (zeroable) room kept beyond the new data
-    int alloc(size_t hist_, size_t max_n_, size_t slack_ = 0)
+    DeviceArray<float2> buf;
+    size_t hist = 0, pos = 0, max_n = 0, slack = 0;   // slack: readable (zeroable) room kept beyond the new data
+    cudaError_t alloc(size_t hist_, size_t max_n_, size_t slack_ = 0)
     {
         hist = (hist_ + 3) & ~(size_t)3;
         max_n = std::max(max_n_, hist) + 4;
         slack = slack_;
-        cap = hist + 2 * max_n + slack;
-        cudaError_t e = cudaMalloc(&base, cap * sizeof(float2));
-        if (e != cudaSuccess) return -1;
-        return 0;
+        return buf.alloc(hist + 2 * max_n + slack);
     }
-    void release() { if (base) cudaFree(base); base = nullptr; }
     cudaError_t reset(cudaStream_t st)
     {
         pos = hist;
-        return hist ? cudaMemsetAsync(base, 0, hist * sizeof(float2), st) : cudaSuccess;
+        return hist ? cudaMemsetAsync(buf.data(), 0, hist * sizeof(float2), st) : cudaSuccess;
     }
     // stream discontinuity that keeps the newest `keep` samples where they are and clears the history below them
     cudaError_t reset_keep_tail(cudaStream_t st, size_t keep)
     {
         if (keep >= hist) return cudaSuccess;
-        return cudaMemsetAsync(base + pos - hist, 0, (hist - keep) * sizeof(float2), st);
+        return cudaMemsetAsync(buf.data() + pos - hist, 0, (hist - keep) * sizeof(float2), st);
     }
     // make room for n new samples; returns pointer to the first new sample
     cudaError_t begin(size_t n, cudaStream_t st, float2** p)
     {
         if (n > max_n) return cudaErrorInvalidValue;
-        if (pos + n + slack > cap) {
+        float2* base = buf.data();
+        if (pos + n + slack > buf.size()) {
             // move the history to the front (ranges cannot overlap: pos - hist >= hist)
             cudaError_t e = cudaMemcpyAsync(base, base + pos - hist, hist * sizeof(float2), cudaMemcpyDeviceToDevice, st);
             if (e != cudaSuccess) return e;
@@ -98,33 +97,31 @@ struct DevStream {
         return cudaSuccess;
     }
     void commit(size_t n) { pos += n; }
-    float2* cur() const { return base + pos; }
 };
 
 struct TapBuf {
-    float2* p = nullptr;
-    size_t cap = 0, len = 0;
+    DeviceArray<float2> buf;
+    size_t len = 0;
     cudaError_t append(const float2* src, size_t n, cudaStream_t st)
     {
-        if (len + n > cap) {
-            size_t ncap = std::max(cap * 2, len + n + 1024);
-            float2* np = nullptr;
-            cudaError_t e = cudaMalloc(&np, ncap * sizeof(float2));
+        if (len + n > buf.size()) {
+            DeviceArray<float2> nb;
+            cudaError_t e = nb.alloc(std::max(buf.size() * 2, len + n + 1024));
             if (e != cudaSuccess) return e;
             if (len) {
-                e = cudaMemcpyAsync(np, p, len * sizeof(float2), cudaMemcpyDeviceToDevice, st);
+                e = cudaMemcpyAsync(nb.data(), buf.data(), len * sizeof(float2), cudaMemcpyDeviceToDevice, st);
                 if (e != cudaSuccess) return e;
                 cudaStreamSynchronize(st);
             }
-            if (p) cudaFree(p);
-            p = np; cap = ncap;
+            buf = std::move(nb);
         }
-        cudaError_t e = cudaMemcpyAsync(p + len, src, n * sizeof(float2), cudaMemcpyDeviceToDevice, st);
+        cudaError_t e = cudaMemcpyAsync(buf.data() + len, src, n * sizeof(float2), cudaMemcpyDeviceToDevice, st);
         len += n;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = len = 0; }
 };
+
+struct FusedDelete { void operator()(FusedFront* f) const { fused_destroy(f); } };
 
 }  // namespace
 
@@ -171,113 +168,104 @@ struct iqgpu_chain {
     uint32_t launches = 0;
 
     // ---- device state ----
-    cudaStream_t stream = nullptr, h2d = nullptr, d2h = nullptr;
+    Stream stream, h2d, d2h;
     // second compute stream: the DC pre-pass of sub-train k+1 (HBM bound) runs underneath the fused front
     // kernel of sub-train k (issue bound); ordered with events
-    cudaStream_t aux = nullptr;
-    cudaEvent_t ev_pre[2] = {nullptr, nullptr}, ev_front[2] = {nullptr, nullptr}, ev_call = nullptr, ev_reset = nullptr;
+    Stream aux;
+    Event ev_pre[2], ev_front[2], ev_call, ev_reset;
     cudaStream_t reset_stream = nullptr;   // stream a not yet consumed reset was queued on
     int order_after_reset(cudaStream_t st);
-    uint32_t* seg_pin[2] = {nullptr, nullptr};    // pinned staging of the chunk table (digital AGC)
-    size_t seg_pin_cap[2] = {0, 0};
-    cudaEvent_t ev_seg[2] = {nullptr, nullptr};
+    PinnedArray<uint32_t> seg_pin[2];   // pinned staging of the chunk table (digital AGC)
+    Event ev_seg[2];
     int seg_pin_slot = 0;
+    template <typename Fill> int stage_chunk_table(uint32_t* dst, size_t n_chunks, cudaStream_t st, Fill fill);
     // chunk tables of lower shards (iqgpu_chain_agc_advance_device), kept per (first frame, frames): a shard plan is
     // replayed step after step, and the table is closed form in those two numbers
-    struct PrefixTab { uint64_t first = 0, frames = 0; uint32_t* d_seg = nullptr; size_t nch = 0; };
+    struct PrefixTab { uint64_t first = 0, frames = 0; DeviceArray<uint32_t> d_seg; };
     std::vector<PrefixTab> prefix_tabs;
     bool front_recorded[2] = {false, false};
     int dc_slot = 0;                    // table slot of the sub-train run_subtrain is about to launch
     bool dc_prepared = false;           // ... and whether its pre-pass was issued on `aux`
     cudaStream_t last_stream = nullptr;   // stream of the most recent process call
-    float* d_lut = nullptr;
-    double2* d_dc_carry = nullptr;
-    float2* d_dc_ref = nullptr;          // dc_mode 1: liquid's v0 {re, im} in fp32
-    double2 *d_run_sums = nullptr, *d_run_start = nullptr;
-    double* d_scan_ws = nullptr;
-    size_t max_runs = 0;
-    std::vector<float*> d_hb_taps;  // per design index
-    float* d_bank = nullptr;
-    float* d_fir_taps = nullptr;
+    DeviceArray<float> d_lut;
+    DeviceArray<double2> d_dc_carry;
+    DeviceArray<float2> d_dc_ref;        // dc_mode 1: liquid's v0 {re, im} in fp32
+    DeviceArray<double2> d_run_sums, d_run_start;
+    DeviceArray<double> d_scan_ws;
+    std::vector<DeviceArray<float>> d_hb_taps;  // per design index
+    DeviceArray<float> d_bank;
+    DeviceArray<float> d_fir_taps;
     std::vector<float> h_fir_taps;      // host copy (kernel-parameter taps)
     unsigned fir_taps_padded = 0;
-    float2 *d_fft_H = nullptr, *d_fft_tw = nullptr, *d_fft_scratch = nullptr;
-    size_t fft_scratch_bytes = 0;
-    cudaError_t ensure_fft_scratch(size_t blocks, cudaStream_t st)
+    DeviceArray<float2> d_fft_H, d_fft_tw, d_fft_scratch;
+    cudaError_t ensure_fft_scratch(size_t blocks, unsigned block, cudaStream_t st)
     {
-        const size_t need = fftfilt_scratch_bytes(blocks, filt.block);
-        if (need <= fft_scratch_bytes) return cudaSuccess;
-        cudaStreamSynchronize(st);
-        cudaFree(d_fft_scratch);
-        d_fft_scratch = nullptr; fft_scratch_bytes = 0;
-        cudaError_t e = cudaMalloc(&d_fft_scratch, need + need / 2);
-        if (e == cudaSuccess) fft_scratch_bytes = need + need / 2;
-        return e;
+        const size_t need = fftfilt_scratch_bytes(blocks, block) / sizeof(float2);
+        return d_fft_scratch.grow(need, need + need / 2, [st] { return cudaStreamSynchronize(st); });
     }
+    int fft_block_pass(const float2* src, size_t n, DevStream& out, cudaStream_t st, const float2** y, size_t* ny);
     // in-chain I/Q optimiser (SURVEY 8(f) rank 3): gate on the sample clock, passes on the device, factors applied from the
     // next sub-train on
     bool iq_optimize = false;
     double iq_interval_ms = 500.0;          // IQ_CORRECTION_INTERVAL_MS, include/constants.h:159
     uint32_t iq_seed = 20261017u;
     double iq_last_attempt_s = -1e18;       // sample-clock time of the last probe
-    IqOptState* d_iq_state = nullptr;
-    IqOptState* h_iq_state = nullptr;       // pinned
-    float2* d_iq_probe = nullptr;
-    size_t iq_probe_cap = 0;
-    cudaEvent_t ev_iq = nullptr, ev_iq_probe = nullptr;
+    DeviceArray<IqOptState> d_iq_state;
+    PinnedArray<IqOptState> h_iq_state;
+    DeviceArray<float2> d_iq_probe;         // 1024 frames per probe
+    Event ev_iq, ev_iq_probe;
     bool iq_pending = false;
     int iq_sync_state();
     int iq_push_state(cudaStream_t st);
     int iq_run_probes(const void* d_rawp, const float2* pre_out, uint64_t N0, const uint32_t* chunks, size_t n_chunks, int slot,
                       cudaStream_t st);
-    AgcState* d_agc = nullptr;
-    uint32_t* d_seg_start = nullptr;
-    float *d_seg_peak = nullptr, *d_seg_gain = nullptr;
-    size_t max_segs = 0;
-    float2* d_agc_scratch = nullptr;
-    size_t agc_scratch_cap = 0;
-    void* d_agc_quiet = nullptr;        // digital AGC: workspace of the grid-wide quiet test (state-only advance)
-    size_t agc_quiet_bytes = 0;
-    void* d_agc_ws = nullptr;           // RMS-AGC time-parallel workspace (block end states + sweep flags)
-    size_t agc_ws_bytes = 0;
+    DeviceArray<AgcState> d_agc;
+    DeviceArray<uint32_t> d_seg_start;  // one entry more than the chunks of d_seg_peak / d_seg_gain
+    DeviceArray<float> d_seg_peak, d_seg_gain;
+    DeviceArray<float2> d_agc_scratch;
+    DeviceArray<unsigned char> d_agc_quiet;     // digital AGC: workspace of the grid-wide quiet test (state-only advance)
+    cudaError_t ensure_agc_quiet(size_t n_chunks, cudaStream_t st)
+    {
+        const size_t need = agc_quiet_workspace_bytes(n_chunks);
+        return d_agc_quiet.grow(need, need * 2, [st] { return cudaStreamSynchronize(st); });
+    }
+    DeviceArray<unsigned char> d_agc_ws;        // RMS-AGC time-parallel workspace (block end states + sweep flags)
     // RMS AGC of the last call when it was one sub-train: input, parameters and (in d_agc_scratch / d_agc_ws) output and
     // checkpoints, which iqgpu_chain_agc_rms_resume_device re-runs from a later start state (time shards)
     const float2* rms_src = nullptr;
     size_t rms_n = 0;
     PostParams rms_qp{};
     bool rms_ready = false, rms_fresh = false;
-    AgcRmsResume* d_rms_resume = nullptr;
+    DeviceArray<AgcRmsResume> d_rms_resume;
     // d_rms_rerun[0]: {g, y2'} the last call started from (its rms_g / rms_y2), [1]: the state of a re-run of that call
     // (which so leaves d_agc alone); rms_resume_max: the latest resume frame since the call or its last re-run.  A resume
     // in front of that frame first re-runs the call (iqgpu_chain_agc_rms_resume_device).
-    AgcState* d_rms_rerun = nullptr;
+    DeviceArray<AgcState> d_rms_rerun;
     size_t rms_resume_max = 0;
     // streams: s_in = pre output; s_stage[d] = output of executed halfband stage d; s_rs = resampler
     // output; s_f = post-filter output (or pre-filter output when the filter is pre-resample)
     DevStream s_in, s_pref, s_arb_in, s_rs, s_f;
     std::vector<DevStream> s_stage;
     TapBuf tap[3];
-    FusedFront* fused = nullptr;
+    std::unique_ptr<FusedFront, FusedDelete> fused;
     int num_sms = 148;
-    // host-path staging
-    void* d_raw[2] = {nullptr, nullptr};
-    void* d_out[2] = {nullptr, nullptr};
-    size_t d_raw_bytes = 0, d_out_bytes = 0;
-    cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr}, ev_d2h[2] = {nullptr, nullptr};
+    // host-path staging (bytes)
+    DeviceArray<char> d_raw[2], d_out[2];
+    Event ev_h2d[2], ev_done[2], ev_d2h[2];
     bool buffers_ready = false;
 
     // optional per-kernel-class device timing (CUDA events on the launch stream)
     bool time_kernels = false;
-    struct TimedSpan { int cls; cudaEvent_t a, b; };
+    struct TimedSpan { int cls; Event a, b; };
     std::vector<TimedSpan> spans;
-    std::vector<cudaEvent_t> ev_pool;
+    std::vector<Event> ev_pool;
     double class_ms[IQGPU_KCLASS_COUNT] = {0};
     uint32_t class_launches[IQGPU_KCLASS_COUNT] = {0};
-    cudaEvent_t get_event()
+    Event get_event()
     {
-        cudaEvent_t e = nullptr;
-        if (!ev_pool.empty()) { e = ev_pool.back(); ev_pool.pop_back(); }
-        else cudaEventCreate(&e);
+        Event e;
+        if (!ev_pool.empty()) { e = std::move(ev_pool.back()); ev_pool.pop_back(); }
+        else create(e, cudaEventDefault);
         return e;
     }
     void span_begin(int cls, cudaStream_t st)
@@ -286,7 +274,7 @@ struct iqgpu_chain {
         if (!time_kernels) return;
         TimedSpan sp{cls, get_event(), get_event()};
         cudaEventRecord(sp.a, st);
-        spans.push_back(sp);
+        spans.push_back(std::move(sp));
     }
     void span_end(cudaStream_t st)
     {
@@ -299,7 +287,7 @@ struct iqgpu_chain {
             float ms = 0.f;
             if (cudaEventSynchronize(sp.b) == cudaSuccess && cudaEventElapsedTime(&ms, sp.a, sp.b) == cudaSuccess)
                 class_ms[sp.cls] += ms;
-            ev_pool.push_back(sp.a); ev_pool.push_back(sp.b);
+            ev_pool.push_back(std::move(sp.a)); ev_pool.push_back(std::move(sp.b));
         }
         spans.clear();
     }
@@ -338,43 +326,14 @@ struct iqgpu_chain {
     } pend;
 };
 
+// the members free their resources after this body, once nothing runs on the chain's streams any more
 iqgpu_chain::~iqgpu_chain()
 {
     if (plan_only) return;
     cudaSetDevice(device);
     if (stream) cudaStreamSynchronize(stream);
-    fused_destroy(fused);
+    if (aux) cudaStreamSynchronize(aux);
     collect_spans();
-    for (auto e : ev_pool) cudaEventDestroy(e);
-    for (auto* t : d_hb_taps) cudaFree(t);
-    cudaFree(d_lut); cudaFree(d_dc_carry); cudaFree(d_dc_ref); cudaFree(d_run_sums); cudaFree(d_run_start); cudaFree(d_scan_ws); cudaFree(d_bank);
-    cudaFree(d_fir_taps); cudaFree(d_fft_H); cudaFree(d_fft_tw); cudaFree(d_fft_scratch); cudaFree(d_agc); cudaFree(d_seg_start);
-    cudaFree(d_seg_peak); cudaFree(d_seg_gain); cudaFree(d_agc_scratch); cudaFree(d_agc_ws);
-    cudaFree(d_iq_state); cudaFree(d_iq_probe); cudaFree(d_agc_quiet); cudaFree(d_rms_resume); cudaFree(d_rms_rerun);
-    if (h_iq_state) cudaFreeHost(h_iq_state);
-    if (ev_iq) cudaEventDestroy(ev_iq);
-    if (ev_iq_probe) cudaEventDestroy(ev_iq_probe);
-    for (auto& t : prefix_tabs) cudaFree(t.d_seg);
-    s_in.release(); s_pref.release(); s_arb_in.release(); s_rs.release(); s_f.release();
-    for (auto& s : s_stage) s.release();
-    for (auto& t : tap) t.release();
-    for (int i = 0; i < 2; i++) {
-        cudaFree(d_raw[i]); cudaFree(d_out[i]);
-        if (ev_h2d[i]) cudaEventDestroy(ev_h2d[i]);
-        if (ev_done[i]) cudaEventDestroy(ev_done[i]);
-        if (ev_d2h[i]) cudaEventDestroy(ev_d2h[i]);
-    }
-    for (int i = 0; i < 2; i++) {
-        if (ev_pre[i]) cudaEventDestroy(ev_pre[i]);
-        if (ev_front[i]) cudaEventDestroy(ev_front[i]);
-    }
-    if (ev_call) cudaEventDestroy(ev_call);
-    if (ev_reset) cudaEventDestroy(ev_reset);
-    for (int i = 0; i < 2; i++) { if (ev_seg[i]) cudaEventDestroy(ev_seg[i]); if (seg_pin[i]) cudaFreeHost(seg_pin[i]); }
-    if (aux) { cudaStreamSynchronize(aux); cudaStreamDestroy(aux); }
-    if (stream) cudaStreamDestroy(stream);
-    if (h2d) cudaStreamDestroy(h2d);
-    if (d2h) cudaStreamDestroy(d2h);
 }
 
 static bool filter_is_fft(const FilterPlan& f)
@@ -440,38 +399,27 @@ int iqgpu_chain::init_device()
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(IQGPU_ENODEVICE, "no CUDA device available");
     if (device >= ndev) return fail(IQGPU_EINVAL, "device index out of range");
     CK(cudaSetDevice(device));
-    CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&h2d, cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&d2h, cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&aux, cudaStreamNonBlocking));
-    CK(cudaEventCreateWithFlags(&ev_call, cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&ev_reset, cudaEventDisableTiming));
-    for (int i = 0; i < 2; i++) {
-        CK(cudaEventCreateWithFlags(&ev_pre[i], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ev_front[i], cudaEventDisableTiming));
-    }
-    for (int i = 0; i < 2; i++) {
-        CK(cudaEventCreateWithFlags(&ev_h2d[i], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ev_done[i], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ev_d2h[i], cudaEventDisableTiming));
-    }
+    for (Stream* s : {&stream, &h2d, &d2h, &aux}) CK(create(*s));
+    for (Event* e : {&ev_call, &ev_reset, &ev_pre[0], &ev_pre[1], &ev_front[0], &ev_front[1], &ev_seg[0], &ev_seg[1], &ev_h2d[0],
+                     &ev_h2d[1], &ev_done[0], &ev_done[1], &ev_d2h[0], &ev_d2h[1]})
+        CK(create(*e));
     // constant tables
     float lut[1024];
     nco_sine_table(lut);
-    CK(cudaMalloc(&d_lut, sizeof(lut)));
-    CK(cudaMemcpy(d_lut, lut, sizeof(lut), cudaMemcpyHostToDevice));
-    CK(cudaMalloc(&d_dc_carry, sizeof(double2)));
-    CK(cudaMalloc(&d_dc_ref, sizeof(float2)));
-    CK(cudaMalloc(&d_agc, sizeof(AgcState)));
-    if (agc_mode == 2) CK(cudaMalloc(&d_rms_rerun, 2 * sizeof(AgcState)));
+    CK(d_lut.alloc(1024));
+    CK(cudaMemcpy(d_lut.data(), lut, sizeof(lut), cudaMemcpyHostToDevice));
+    CK(d_dc_carry.alloc(1));
+    CK(d_dc_ref.alloc(1));
+    CK(d_agc.alloc(1));
+    if (agc_mode == 2) CK(d_rms_rerun.alloc(2));
     if (!rs.passthrough) {
-        d_hb_taps.resize(rs.num_halfband, nullptr);
+        d_hb_taps.resize(rs.num_halfband);
         for (unsigned i = 0; i < rs.num_halfband; i++) {
-            CK(cudaMalloc(&d_hb_taps[i], rs.stages[i].h1.size() * sizeof(float)));
-            CK(cudaMemcpy(d_hb_taps[i], rs.stages[i].h1.data(), rs.stages[i].h1.size() * sizeof(float), cudaMemcpyHostToDevice));
+            CK(d_hb_taps[i].alloc(rs.stages[i].h1.size()));
+            CK(cudaMemcpy(d_hb_taps[i].data(), rs.stages[i].h1.data(), rs.stages[i].h1.size() * sizeof(float), cudaMemcpyHostToDevice));
         }
-        CK(cudaMalloc(&d_bank, rs.bank.size() * sizeof(float)));
-        CK(cudaMemcpy(d_bank, rs.bank.data(), rs.bank.size() * sizeof(float), cudaMemcpyHostToDevice));
+        CK(d_bank.alloc(rs.bank.size()));
+        CK(cudaMemcpy(d_bank.data(), rs.bank.data(), rs.bank.size() * sizeof(float), cudaMemcpyHostToDevice));
     }
     {
         cudaDeviceProp prop{};
@@ -489,7 +437,7 @@ int iqgpu_chain::init_device()
         }
         if (ok && fused_supported(cfg.input_format, rd)) {
             std::string ferr;
-            fused = fused_create(cfg.input_format, rd, nco_pre, d_bank, num_sms, ferr);
+            fused.reset(fused_create(cfg.input_format, rd, nco_pre, d_bank.data(), num_sms, ferr));
             if (!fused) return fail(IQGPU_ECUDA, ferr);
         }
     }
@@ -504,8 +452,8 @@ int iqgpu_chain::init_device()
             if (cplx) { h[2 * (pad + i)] = t.real(); h[2 * (pad + i) + 1] = t.imag(); }
             else h[pad + i] = t.real();
         }
-        CK(cudaMalloc(&d_fir_taps, h.size() * sizeof(float)));
-        CK(cudaMemcpy(d_fir_taps, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
+        CK(d_fir_taps.alloc(h.size()));
+        CK(cudaMemcpy(d_fir_taps.data(), h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
         h_fir_taps = h;
     }
     if (filter_is_fir(filt) && filt.post_resample && filt.taps.size() >= 512 && filt.taps.size() <= 8192 &&
@@ -520,15 +468,14 @@ int iqgpu_chain::init_device()
         std::vector<float2> tw(fft_twiddle_entries(nfft)), hpad(nfft, make_float2(0.f, 0.f));
         fft_fill_twiddles(nfft, tw.data());
         for (size_t i = 0; i < filt.taps.size(); i++) hpad[i] = make_float2(filt.taps[i].real(), filt.taps[i].imag());
-        float2* d_h = nullptr;
-        CK(cudaMalloc(&d_fft_tw, tw.size() * sizeof(float2)));
-        CK(cudaMalloc(&d_fft_H, nfft * sizeof(float2)));
-        CK(cudaMalloc(&d_h, nfft * sizeof(float2)));
-        CK(cudaMemcpy(d_fft_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(d_h, hpad.data(), nfft * sizeof(float2), cudaMemcpyHostToDevice));
-        CK(launch_fft_forward(d_h, nfft, d_fft_tw, d_fft_H, stream));
+        DeviceArray<float2> d_h;
+        CK(d_fft_tw.alloc(tw.size()));
+        CK(d_fft_H.alloc(nfft));
+        CK(d_h.alloc(nfft));
+        CK(cudaMemcpy(d_fft_tw.data(), tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(d_h.data(), hpad.data(), nfft * sizeof(float2), cudaMemcpyHostToDevice));
+        CK(launch_fft_forward(d_h.data(), nfft, d_fft_tw.data(), d_fft_H.data(), stream));
         CK(cudaStreamSynchronize(stream));
-        cudaFree(d_h);
     }
     return IQGPU_OK;
 }
@@ -589,14 +536,14 @@ int iqgpu_chain::ensure_buffers()
     if (post_filter && s_f.alloc(0, rs_max + 2 * (size_t)std::max<unsigned>(filt.block, fir_fft_block)) != 0)
         return fail(IQGPU_ENOMEM, "device allocation failed (s_f)");
 
-    max_runs = n / 128 + 2;
-    CK(cudaMalloc(&d_run_sums, max_runs * sizeof(double2)));
-    CK(cudaMalloc(&d_scan_ws, dc_scan_workspace_doubles(max_runs) * sizeof(double)));
-    CK(cudaMalloc(&d_run_start, max_runs * sizeof(double2)));
-    max_segs = n / std::max<uint32_t>(1, std::min<uint32_t>(chunk_frames, 1024)) + 8;
-    CK(cudaMalloc(&d_seg_start, (max_segs + 1) * sizeof(uint32_t)));
-    CK(cudaMalloc(&d_seg_peak, max_segs * sizeof(float)));
-    CK(cudaMalloc(&d_seg_gain, max_segs * sizeof(float)));
+    const size_t max_runs = n / 128 + 2;
+    CK(d_run_sums.alloc(max_runs));
+    CK(d_scan_ws.alloc(dc_scan_workspace_doubles(max_runs)));
+    CK(d_run_start.alloc(max_runs));
+    const size_t max_segs = n / std::max<uint32_t>(1, std::min<uint32_t>(chunk_frames, 1024)) + 8;
+    CK(d_seg_start.alloc(max_segs + 1));
+    CK(d_seg_peak.alloc(max_segs));
+    CK(d_seg_gain.alloc(max_segs));
     buffers_ready = true;
     return reset_state();
 }
@@ -627,21 +574,21 @@ int iqgpu_chain::reset_state(bool keep_fft_remainder)
     cudaStream_t S = last_stream ? last_stream : stream;
     dc_prepared = false;
     front_recorded[0] = front_recorded[1] = false;
-    CK(cudaMemsetAsync(d_dc_carry, 0, sizeof(double2), S));
-    CK(cudaMemsetAsync(d_dc_ref, 0, sizeof(float2), S));
+    CK(cudaMemsetAsync(d_dc_carry.data(), 0, sizeof(double2), S));
+    CK(cudaMemsetAsync(d_dc_ref.data(), 0, sizeof(float2), S));
     AgcState a{};
     a.locked = 0; a.gain = 1.0f; a.seen = 0; a.last_strong = 0.0;
     a.peak_mem = (agc_mode == 1) ? 0.05f : 0.001f;   // agc.c:66,78
     a.rms_g = 1.0f; a.rms_y2 = 1.0f;                  // agc.c:58-62 (set_signal_level then set_gain(1))
-    agc_state_init_kernel<<<1, 1, 0, S>>>(d_agc, a);
+    agc_state_init_kernel<<<1, 1, 0, S>>>(d_agc.data(), a);
     CK(cudaGetLastError());
-    if (fused) CK(fused_reset(fused, S));
-    if (s_in.base) CK((keep && pre_fft) ? s_in.reset_keep_tail(S, keep) : s_in.reset(S));
-    if (s_pref.base) CK(s_pref.reset(S));
-    if (s_arb_in.base) CK(s_arb_in.reset(S));
-    for (auto& s : s_stage) if (s.base) CK(s.reset(S));
+    if (fused) CK(fused_reset(fused.get(), S));
+    if (s_in.buf.data()) CK((keep && pre_fft) ? s_in.reset_keep_tail(S, keep) : s_in.reset(S));
+    if (s_pref.buf.data()) CK(s_pref.reset(S));
+    if (s_arb_in.buf.data()) CK(s_arb_in.reset(S));
+    for (auto& s : s_stage) if (s.buf.data()) CK(s.reset(S));
     CK((keep && post_fft) ? s_rs.reset_keep_tail(S, keep) : s_rs.reset(S));
-    if (s_f.base) CK(s_f.reset(S));
+    if (s_f.buf.data()) CK(s_f.reset(S));
     CK(cudaEventRecord(ev_reset, S));
     reset_stream = S;
     return IQGPU_OK;
@@ -661,7 +608,7 @@ PreParams iqgpu_chain::pre_params(uint64_t N0) const
     pp.format = cfg.input_format; pp.gain = cfg.gain;
     pp.dc_enable = dc.enable; pp.dc_c = dc.c; pp.dc_a = dc.one_minus_c;
     pp.iq_enable = cfg.iq_correction_enable; pp.iq_magp1 = 1.0f + iq_mag; pp.iq_phase = iq_phase;
-    pp.nco_enable = nco_pre; pp.nco_dtheta = nco_dtheta; pp.nco_sign = nco_sign; pp.nco_table = d_lut;
+    pp.nco_enable = nco_pre; pp.nco_dtheta = nco_dtheta; pp.nco_sign = nco_sign; pp.nco_table = d_lut.data();
     pp.nco_theta0 = (uint32_t)((uint64_t)(uint32_t)N0 * nco_dtheta);
     return pp;
 }
@@ -674,7 +621,7 @@ int iqgpu_chain::prepare_dc(int slot, const void* d_rawp, uint64_t N0, size_t n,
     if (front_recorded[slot]) CK(cudaStreamWaitEvent(aux, ev_front[slot], 0));
     const PreParams pp = pre_params(N0);
     uint32_t l = 0;
-    CK(fused_prepare_dc(fused, slot, d_rawp, (int64_t)N0, n, pp, d_dc_carry, &l, aux));
+    CK(fused_prepare_dc(fused.get(), slot, d_rawp, (int64_t)N0, n, pp, d_dc_carry.data(), &l, aux));
     prepass_launches += l;                      // 0 when the front kernel carries the DC state itself (no pre-pass)
     CK(cudaEventRecord(ev_pre[slot], aux));
     return IQGPU_OK;
@@ -693,23 +640,23 @@ int iqgpu_chain::iq_sync_state()
     if (!iq_pending) return IQGPU_OK;
     CK(cudaEventSynchronize(ev_iq));
     iq_pending = false;
-    iq_mag = h_iq_state->mag; iq_phase = h_iq_state->phase;
+    iq_mag = h_iq_state.data()->mag; iq_phase = h_iq_state.data()->phase;
     return IQGPU_OK;
 }
 
 int iqgpu_chain::iq_push_state(cudaStream_t st)
 {
-    if (!d_iq_state) {
-        CK(cudaMalloc(&d_iq_state, sizeof(IqOptState)));
-        CK(cudaMallocHost(&h_iq_state, sizeof(IqOptState)));
-        CK(cudaEventCreateWithFlags(&ev_iq, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ev_iq_probe, cudaEventDisableTiming));
-        memset(h_iq_state, 0, sizeof(IqOptState));
-        h_iq_state->seed = iq_seed;
+    if (!d_iq_state.data()) {       // first use; d_iq_state comes last, so that a set-up that failed is redone as a whole
+        CK(h_iq_state.alloc(1));
+        memset(h_iq_state.data(), 0, sizeof(IqOptState));
+        CK(create(ev_iq));
+        CK(create(ev_iq_probe));
+        CK(d_iq_state.alloc(1));
     }
     { int rc_ = iq_sync_state(); if (rc_) return rc_; }
-    h_iq_state->mag = iq_mag; h_iq_state->phase = iq_phase; h_iq_state->seed = iq_seed;
-    CK(cudaMemcpyAsync(d_iq_state, h_iq_state, sizeof(IqOptState), cudaMemcpyHostToDevice, st));
+    IqOptState* h = h_iq_state.data();
+    h->mag = iq_mag; h->phase = iq_phase; h->seed = iq_seed;
+    CK(cudaMemcpyAsync(d_iq_state.data(), h, sizeof(IqOptState), cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));          // h_iq_state is also the read-back buffer
     return IQGPU_OK;
 }
@@ -727,29 +674,26 @@ int iqgpu_chain::iq_run_probes(const void* d_rawp, const float2* pre_out, uint64
         const double t = (double)pos / (double)in_rate;
         if (chunks[c] >= 1024 && (t - iq_last_attempt_s) * 1000.0 >= iq_interval_ms) {       // pipeline.c:469, iq_correct.c:157-162
             bool ok = true;
-            if (!pre_out && dc.enable && !fused_dc_state_at(fused, slot, (int64_t)N0, (int64_t)pos)) ok = false;
+            if (!pre_out && dc.enable && !fused_dc_state_at(fused.get(), slot, (int64_t)N0, (int64_t)pos)) ok = false;
             if (ok) { pos_list.push_back(pos); iq_last_attempt_s = t; }
         }
         pos += chunks[c];
     }
     if (pos_list.empty()) return IQGPU_OK;
-    if (!d_iq_state) { int rc_ = iq_push_state(st); if (rc_) return rc_; }
-    if (pos_list.size() > iq_probe_cap) {
-        CK(cudaStreamSynchronize(st));
-        if (aux) CK(cudaStreamSynchronize(aux));
-        cudaFree(d_iq_probe);
-        iq_probe_cap = pos_list.size() * 2 + 8;
-        CK(cudaMalloc(&d_iq_probe, iq_probe_cap * 1024 * sizeof(float2)));
-    }
+    if (!d_iq_state.data()) { int rc_ = iq_push_state(st); if (rc_) return rc_; }
+    CK(d_iq_probe.grow(pos_list.size() * 1024, (pos_list.size() * 2 + 8) * 1024, [&] {
+        const cudaError_t e = cudaStreamSynchronize(st);
+        return e != cudaSuccess ? e : cudaStreamSynchronize(aux);
+    }));
     if (iq_pending) CK(cudaStreamWaitEvent(st, ev_iq, 0));      // the previous train's passes still read the probe buffer
     for (size_t i = 0; i < pos_list.size(); i++) {
         const uint64_t p0 = pos_list[i];
-        float2* dst = d_iq_probe + i * 1024;
+        float2* dst = d_iq_probe.data() + i * 1024;
         if (pre_out) {
             CK(cudaMemcpyAsync(dst, pre_out + (p0 - N0), 1024 * sizeof(float2), cudaMemcpyDeviceToDevice, st));
         } else {
             const PreParams pp = pre_params(p0);
-            const double2* v = dc.enable ? fused_dc_state_at(fused, slot, (int64_t)N0, (int64_t)p0) : nullptr;
+            const double2* v = dc.enable ? fused_dc_state_at(fused.get(), slot, (int64_t)N0, (int64_t)p0) : nullptr;
             CK(launch_pre(reinterpret_cast<const char*>(d_rawp) + (p0 - N0) * in_bps, 1024, pp, 1024, v, dst, st));
             launches++;
         }
@@ -757,11 +701,43 @@ int iqgpu_chain::iq_run_probes(const void* d_rawp, const float2* pre_out, uint64
     // the passes themselves run on the second stream: the post kernels of this sub-train do not wait for them
     CK(cudaEventRecord(ev_iq_probe, st));
     CK(cudaStreamWaitEvent(aux, ev_iq_probe, 0));
-    CK(launch_iq_optimize_train(d_iq_probe, (int)pos_list.size(), d_iq_state, aux));
+    CK(launch_iq_optimize_train(d_iq_probe.data(), (int)pos_list.size(), d_iq_state.data(), aux));
     launches++;
-    CK(cudaMemcpyAsync(h_iq_state, d_iq_state, sizeof(IqOptState), cudaMemcpyDeviceToHost, aux));
+    CK(cudaMemcpyAsync(h_iq_state.data(), d_iq_state.data(), sizeof(IqOptState), cudaMemcpyDeviceToHost, aux));
     CK(cudaEventRecord(ev_iq, aux));
     iq_pending = true;
+    return IQGPU_OK;
+}
+
+// FFT block filter over the fft_rem frames that wait in front of `src` and the n new ones: the whole blocks go to `out`
+// (*y: first output sample, *ny: their count), the rest waits for the next call
+int iqgpu_chain::fft_block_pass(const float2* src, size_t n, DevStream& out, cudaStream_t st, const float2** y, size_t* ny)
+{
+    const uint32_t B = filt.block, tot = fft_rem + (uint32_t)n, blocks = tot / B;
+    float2* yo = nullptr;
+    CK(out.begin((size_t)blocks * B, st, &yo));
+    if (blocks) {
+        CK(ensure_fft_scratch(blocks, B, st));
+        CK(launch_fftfilt(src - fft_rem, blocks, B, d_fft_H.data(), d_fft_tw.data(), yo, d_fft_scratch.data(), &launches, st));
+    }
+    out.commit((size_t)blocks * B);
+    fft_rem = tot - blocks * B;
+    *y = yo; *ny = (size_t)blocks * B;
+    return IQGPU_OK;
+}
+
+// copies a chunk table of n_chunks + 1 entries, written by fill(), to `dst` on `st` through pinned staging: an async copy
+// from pageable memory would first drain the stream.  Two slots, each reused once its previous copy has finished.
+template <typename Fill>
+int iqgpu_chain::stage_chunk_table(uint32_t* dst, size_t n_chunks, cudaStream_t st, Fill fill)
+{
+    const size_t need = n_chunks + 1;
+    const int sl = seg_pin_slot ^= 1;
+    CK(cudaEventSynchronize(ev_seg[sl]));
+    CK(seg_pin[sl].grow(need, need * 2, no_drain));
+    fill(seg_pin[sl].data());
+    CK(cudaMemcpyAsync(dst, seg_pin[sl].data(), need * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(ev_seg[sl], st));
     return IQGPU_OK;
 }
 
@@ -805,7 +781,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
         const bool fold_ok = post_filter && filter_is_fir(filt) && !fir_via_fft && !record_taps &&
                              fir_can_fold_dc(fir_taps_padded, filt.impl == IQGPU_FILTER_IMPL_FIR_ASYM, !h_fir_taps.empty());
         dc_fold.corr = nullptr;
-        CK(fused_launch(fused, d_rawp, (int64_t)N0, n, pp, d_dc_carry, (int64_t)O0, (size_t)(O1 - O0), y_rs, &launches, dc_slot, st,
+        CK(fused_launch(fused.get(), d_rawp, (int64_t)N0, n, pp, d_dc_carry.data(), (int64_t)O0, (size_t)(O1 - O0), y_rs, &launches, dc_slot, st,
                         fold_ok ? &dc_fold : nullptr));
         span_end(st);
         { int rc_iq = iq_run_probes(d_rawp, nullptr, N0, chunks, n_chunks, dc_slot, st); if (rc_iq) return rc_iq; }
@@ -828,7 +804,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
             CK(launch_pre(d_rawp, n, p1, run_len, nullptr, x_in, st));
             span_end(st);
             span_begin(IQGPU_KCLASS_DC_SCAN, st);
-            CK(launch_dc_reference(x_in, n, dc.c, d_dc_ref, st));
+            CK(launch_dc_reference(x_in, n, dc.c, d_dc_ref.data(), st));
             span_end(st);
             launches += 2;
             if (pp.iq_enable || pp.nco_enable) {
@@ -840,19 +816,20 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
                 launches++;
             }
         } else {
-        if (dc.enable) {
-            const size_t n_runs = (n + run_len - 1) / run_len;
-            if (n_runs > max_runs) return fail(IQGPU_EINVAL, "internal: run table too small");
-            span_begin(IQGPU_KCLASS_DC_SCAN, st);
-            CK(launch_dc_run_sums(d_rawp, n, pp, run_len, d_run_sums, st));
-            CK(launch_dc_scan(d_run_sums, n_runs, run_len, n, dc.c, d_dc_carry, d_run_start, d_scan_ws, st));
+            if (dc.enable) {
+                const size_t n_runs = (n + run_len - 1) / run_len;
+                if (n_runs > d_run_sums.size()) return fail(IQGPU_EINVAL, "internal: run table too small");
+                span_begin(IQGPU_KCLASS_DC_SCAN, st);
+                CK(launch_dc_run_sums(d_rawp, n, pp, run_len, d_run_sums.data(), st));
+                CK(launch_dc_scan(d_run_sums.data(), n_runs, run_len, n, dc.c, d_dc_carry.data(), d_run_start.data(),
+                                  d_scan_ws.data(), st));
+                span_end(st);
+                launches += 2;
+            }
+            span_begin(IQGPU_KCLASS_PRE, st);
+            CK(launch_pre(d_rawp, n, pp, run_len, d_run_start.data(), x_in, st));
             span_end(st);
-            launches += 2;
-        }
-        span_begin(IQGPU_KCLASS_PRE, st);
-        CK(launch_pre(d_rawp, n, pp, run_len, d_run_start, x_in, st));
-        span_end(st);
-        launches++;
+            launches++;
         }
         s_in.commit(n);
         if (record_tap0) CK(tap[0].append(x_in, n, st));
@@ -866,24 +843,16 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
             if (filter_is_fir(filt)) {
                 float2* y = nullptr;
                 CK(s_pref.begin(n, st, &y));
-                CK(launch_fir(x_in, n, d_fir_taps, fir_taps_padded, filt.impl == IQGPU_FILTER_IMPL_FIR_ASYM, y, st, h_fir_taps.data()));
+                CK(launch_fir(x_in, n, d_fir_taps.data(), fir_taps_padded, filt.impl == IQGPU_FILTER_IMPL_FIR_ASYM, y, st, h_fir_taps.data()));
                 launches++;
                 s_pref.commit(n);
                 rs_src = y;
                 // the reference probes buffer A after the whole pre chain, i.e. behind a pre-resample FIR (pipeline.c:466-472)
                 { int rc_iq = iq_run_probes(d_rawp, y, N0, chunks, n_chunks, 0, st); if (rc_iq) return rc_iq; }
             } else {
-                const uint32_t tot = fft_rem + (uint32_t)n, blocks = tot / filt.block;
-                float2* y = nullptr;
-                CK(s_pref.begin((size_t)blocks * filt.block, st, &y));
-                if (blocks) {
-                    CK(ensure_fft_scratch(blocks, st));
-                    CK(launch_fftfilt(x_in - fft_rem, blocks, filt.block, d_fft_H, d_fft_tw, y, d_fft_scratch, &launches, st));
-                }
-                s_pref.commit((size_t)blocks * filt.block);
                 rs_pos0 = N0 + fft_rem_carry - fft_rem;
-                fft_rem = tot - blocks * filt.block;
-                rs_src = y; rs_n = (size_t)blocks * filt.block;
+                int rc = fft_block_pass(x_in, n, s_pref, st, &rs_src, &rs_n);
+                if (rc) return rc;
             }
         }
 
@@ -903,7 +872,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
                     const uint64_t k0 = P0 >> (d + 1), k1 = P1 >> (d + 1);
                     float2* y = nullptr;
                     CK(s_stage[d].begin((size_t)(k1 - k0), st, &y));
-                    CK(launch_halfband_decim(src, (int64_t)a0, d_hb_taps[g], rs.stages[g].m, (int64_t)k0, (size_t)(k1 - k0),
+                    CK(launch_halfband_decim(src, (int64_t)a0, d_hb_taps[g].data(), rs.stages[g].m, (int64_t)k0, (size_t)(k1 - k0),
                                              (d + 1 == S) ? rs.zeta : 1.0f, y, st));
                     launches++;
                     s_stage[d].commit((size_t)(k1 - k0));
@@ -913,7 +882,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
                 const uint64_t O0 = arb_outputs_after(K0, rs.step), O1 = arb_outputs_after(K1, rs.step);
                 const unsigned __int128 Pph = (unsigned __int128)O0 * rs.step;
                 CK(s_rs.begin((size_t)(O1 - O0), st, &y_rs));
-                CK(launch_arb(src, (int64_t)K0, d_bank, rs.step, (int64_t)(uint64_t)(Pph >> 24), (uint32_t)(Pph & 0xffffffu),
+                CK(launch_arb(src, (int64_t)K0, d_bank.data(), rs.step, (int64_t)(uint64_t)(Pph >> 24), (uint32_t)(Pph & 0xffffffu),
                               (size_t)(O1 - O0), y_rs, st));
                 launches++;
                 post_n = (size_t)(O1 - O0);
@@ -923,7 +892,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
                 float2* y = nullptr;
                 size_t cnt = (size_t)(O1 - O0);
                 if (S == 0) CK(s_rs.begin(cnt, st, &y)); else CK(s_arb_in.begin(cnt, st, &y));
-                CK(launch_arb(rs_src, (int64_t)P0, d_bank, rs.step, (int64_t)(uint64_t)(Pph >> 24), (uint32_t)(Pph & 0xffffffu), cnt, y, st));
+                CK(launch_arb(rs_src, (int64_t)P0, d_bank.data(), rs.step, (int64_t)(uint64_t)(Pph >> 24), (uint32_t)(Pph & 0xffffffu), cnt, y, st));
                 launches++;
                 if (S == 0) y_rs = y; else s_arb_in.commit(cnt);
                 const float2* src = y;
@@ -931,7 +900,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
                 for (unsigned s = 0; s < S; s++) {
                     float2* yo = nullptr;
                     if (s + 1 == S) CK(s_rs.begin(2 * cnt, st, &yo)); else CK(s_stage[s].begin(2 * cnt, st, &yo));
-                    CK(launch_halfband_interp(src, (int64_t)a0, d_hb_taps[s], rs.stages[s].m, (int64_t)a0, cnt, yo, st));
+                    CK(launch_halfband_interp(src, (int64_t)a0, d_hb_taps[s].data(), rs.stages[s].m, (int64_t)a0, cnt, yo, st));
                     launches++;
                     if (s + 1 == S) y_rs = yo; else s_stage[s].commit(2 * cnt);
                     src = yo; a0 *= 2; cnt *= 2;
@@ -942,8 +911,8 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
             post_src = y_rs;
             span_end(st);
         } else if (post_filter) {
-            // passthrough + post filter never happens (no_resample keeps the filter pre-resample), but keep the
-            // stream contract: copy into s_rs so the filter finds its history.
+            // passthrough + post filter: the filter-only module chain of a decimating configuration (IQGPU_STAGE_FILTER
+            // without IQGPU_STAGE_RESAMPLER).  Copy into s_rs, where the filter finds its history.
             float2* y = nullptr;
             CK(s_rs.begin(rs_n, st, &y));
             CK(cudaMemcpyAsync(y, rs_src, rs_n * sizeof(float2), cudaMemcpyDeviceToDevice, st));
@@ -965,14 +934,9 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
             if (blocks) {
                 if (blocks * B > post_n)
                     CK(cudaMemsetAsync(const_cast<float2*>(post_src) + post_n, 0, (blocks * B - post_n) * sizeof(float2), st));
-                const size_t need = fftfilt_scratch_bytes(blocks, (unsigned)B);
-                if (need > fft_scratch_bytes) {
-                    CK(cudaStreamSynchronize(st));
-                    cudaFree(d_fft_scratch); d_fft_scratch = nullptr; fft_scratch_bytes = 0;
-                    CK(cudaMalloc(&d_fft_scratch, need + need / 2));
-                    fft_scratch_bytes = need + need / 2;
-                }
-                CK(launch_fftfilt(post_src, blocks, (unsigned)B, d_fft_H, d_fft_tw, y, d_fft_scratch, &launches, st));
+                CK(ensure_fft_scratch(blocks, (unsigned)B, st));
+                CK(launch_fftfilt(post_src, blocks, (unsigned)B, d_fft_H.data(), d_fft_tw.data(), y, d_fft_scratch.data(), &launches,
+                                  st));
             }
             s_f.commit(post_n);
             post_src = y;
@@ -985,7 +949,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
             float2* y = nullptr;
             CK(s_f.begin(post_n, st, &y));
             const bool folding = use_fused && dc_fold.corr != nullptr;
-            CK(launch_fir(post_src, post_n, d_fir_taps, fir_taps_padded, cplx, y, st, h_fir_taps.data(),
+            CK(launch_fir(post_src, post_n, d_fir_taps.data(), fir_taps_padded, cplx, y, st, h_fir_taps.data(),
                           fir_wrote_output ? cfg.output_format : 0, fir_wrote_output ? d_outp : nullptr,
                           folding ? &dc_fold : nullptr));
             launches++;
@@ -999,16 +963,8 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
             s_f.commit(post_n);
             post_src = y;
         } else {
-            const uint32_t tot = fft_rem + (uint32_t)post_n, blocks = tot / filt.block;
-            float2* y = nullptr;
-            CK(s_f.begin((size_t)blocks * filt.block, st, &y));
-            if (blocks) {
-                CK(ensure_fft_scratch(blocks, st));
-                CK(launch_fftfilt(post_src - fft_rem, blocks, filt.block, d_fft_H, d_fft_tw, y, d_fft_scratch, &launches, st));
-            }
-            s_f.commit((size_t)blocks * filt.block);
-            fft_rem = tot - blocks * filt.block;
-            post_src = y; post_n = (size_t)blocks * filt.block;
+            int rc = fft_block_pass(post_src, post_n, s_f, st, &post_src, &post_n);
+            if (rc) return rc;
         }
         span_end(st);
     }
@@ -1017,7 +973,7 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
     // ---------------- K5: post NCO + AGC + convert ----------------
     PostParams qp{};
     qp.format = cfg.output_format;
-    qp.nco_enable = nco_post; qp.nco_dtheta = nco_dtheta; qp.nco_sign = nco_sign; qp.nco_table = d_lut;
+    qp.nco_enable = nco_post; qp.nco_dtheta = nco_dtheta; qp.nco_sign = nco_sign; qp.nco_table = d_lut.data();
     qp.nco_theta0 = (uint32_t)((uint64_t)(uint32_t)n_nco_post * nco_dtheta);
     qp.agc_mode = agc_mode; qp.agc_target = agc_target; qp.agc_alpha = agc_alpha; qp.target_rate = target_rate;
     pend.active = true;
@@ -1027,29 +983,12 @@ int iqgpu_chain::run_subtrain(const void* d_rawp, size_t n, const uint32_t* chun
         // pass 1 of the digital AGC: per-chunk peaks (agc.c:117-124).  Everything after this is a
         // function of the peaks and the carried AGC state only.
         span_begin(IQGPU_KCLASS_POST, st);
-        if (n_chunks > max_segs) {
-            CK(cudaStreamSynchronize(st));
-            cudaFree(d_seg_start); cudaFree(d_seg_peak); cudaFree(d_seg_gain);
-            max_segs = n_chunks * 2;
-            CK(cudaMalloc(&d_seg_start, (max_segs + 1) * sizeof(uint32_t)));
-            CK(cudaMalloc(&d_seg_peak, max_segs * sizeof(float)));
-            CK(cudaMalloc(&d_seg_gain, max_segs * sizeof(float)));
-        }
-        {
-            // pinned staging (two slots guarded by events): an async copy from pageable memory would first drain the stream
-            const size_t need = (n_chunks + 1) * sizeof(uint32_t);
-            const int sl = seg_pin_slot ^= 1;
-            if (need > seg_pin_cap[sl]) {
-                if (seg_pin[sl]) { CK(cudaEventSynchronize(ev_seg[sl])); CK(cudaFreeHost(seg_pin[sl])); seg_pin[sl] = nullptr; }
-                CK(cudaMallocHost(&seg_pin[sl], need * 2));
-                seg_pin_cap[sl] = need * 2;
-                if (!ev_seg[sl]) CK(cudaEventCreateWithFlags(&ev_seg[sl], cudaEventDisableTiming));
-            } else CK(cudaEventSynchronize(ev_seg[sl]));
-            memcpy(seg_pin[sl], seg.data(), need);
-            CK(cudaMemcpyAsync(d_seg_start, seg_pin[sl], need, cudaMemcpyHostToDevice, st));
-            CK(cudaEventRecord(ev_seg[sl], st));
-        }
-        CK(launch_agc_peaks(post_src, post_n, qp, d_seg_start, n_chunks, d_seg_peak, st));
+        auto drain = [st] { return cudaStreamSynchronize(st); };
+        CK(d_seg_start.grow(n_chunks + 1, n_chunks * 2 + 1, drain));
+        CK(d_seg_peak.grow(n_chunks, n_chunks * 2, drain));
+        CK(d_seg_gain.grow(n_chunks, n_chunks * 2, drain));
+        { int rc = stage_chunk_table(d_seg_start.data(), n_chunks, st, [&](uint32_t* t) { std::copy(seg.begin(), seg.end(), t); }); if (rc) return rc; }
+        CK(launch_agc_peaks(post_src, post_n, qp, d_seg_start.data(), n_chunks, d_seg_peak.data(), st));
         span_end(st);
         launches += 1;
         pend.peaks_done = true;
@@ -1077,7 +1016,7 @@ int iqgpu_chain::run_back(void* d_outp, size_t skip_chunks, size_t* out_frames, 
     if (record_taps && post_n) {
         // reserve room in the tap buffer and let the post kernel write straight into it
         CK(tap[2].append(post_src, post_n, st));
-        tap2 = tap[2].p + tap[2].len - post_n;
+        tap2 = tap[2].buf.data() + tap[2].len - post_n;
     }
     if (post_n && fir_wrote_output) {
         fir_wrote_output = false;        // the FIR epilogue already produced the final stream (run_subtrain)
@@ -1086,41 +1025,22 @@ int iqgpu_chain::run_back(void* d_outp, size_t skip_chunks, size_t* out_frames, 
         if (agc_mode == 1) {
             if (skip_chunks) {
                 const std::vector<float> ones(skip_chunks, 1.0f);
-                CK(cudaMemcpyAsync(d_seg_gain, ones.data(), skip_chunks * sizeof(float), cudaMemcpyHostToDevice, st));
+                CK(cudaMemcpyAsync(d_seg_gain.data(), ones.data(), skip_chunks * sizeof(float), cudaMemcpyHostToDevice, st));
             }
-            {
-                const size_t qneed = agc_quiet_workspace_bytes(n_chunks);
-                if (qneed > agc_quiet_bytes) {
-                    CK(cudaStreamSynchronize(st));
-                    cudaFree(d_agc_quiet);
-                    d_agc_quiet = nullptr; agc_quiet_bytes = 0;
-                    CK(cudaMalloc(&d_agc_quiet, qneed * 2));
-                    agc_quiet_bytes = qneed * 2;
-                }
-            }
-            CK(launch_agc_digital_scan(d_seg_start + skip_chunks, n_chunks - skip_chunks, d_seg_peak + skip_chunks, qp, d_agc,
-                                       d_seg_gain + skip_chunks, st, d_agc_quiet));
-            CK(launch_post(post_src, post_n, qp, d_seg_start, n_chunks, d_seg_gain, 0, tap2, d_outp, st));
+            CK(ensure_agc_quiet(n_chunks, st));
+            CK(launch_agc_digital_scan(d_seg_start.data() + skip_chunks, n_chunks - skip_chunks, d_seg_peak.data() + skip_chunks, qp,
+                                       d_agc.data(), d_seg_gain.data() + skip_chunks, st, d_agc_quiet.data()));
+            CK(launch_post(post_src, post_n, qp, d_seg_start.data(), n_chunks, d_seg_gain.data(), 0, tap2, d_outp, st));
             launches += 2;
         } else if (agc_mode == 2) {
-            if (post_n > agc_scratch_cap) {
-                CK(cudaStreamSynchronize(st));
-                cudaFree(d_agc_scratch);
-                agc_scratch_cap = post_n + post_n / 2 + 1024;
-                CK(cudaMalloc(&d_agc_scratch, agc_scratch_cap * sizeof(float2)));
-            }
-            float2* y = d_agc_scratch;
+            auto drain = [st] { return cudaStreamSynchronize(st); };
+            CK(d_agc_scratch.grow(post_n, post_n + post_n / 2 + 1024, drain));
+            float2* y = d_agc_scratch.data();
             const size_t ws_need = agc_rms_workspace_bytes(post_n, qp.agc_alpha);
-            if (ws_need > agc_ws_bytes) {
-                CK(cudaStreamSynchronize(st));
-                cudaFree(d_agc_ws);
-                d_agc_ws = nullptr; agc_ws_bytes = 0;
-                CK(cudaMalloc(&d_agc_ws, ws_need * 2));
-                agc_ws_bytes = ws_need * 2;
-            }
+            CK(d_agc_ws.grow(ws_need, ws_need * 2, drain));
             static_assert(offsetof(AgcState, rms_y2) == offsetof(AgcState, rms_g) + sizeof(float), "{g, y2'} must be adjacent");
-            CK(cudaMemcpyAsync(&d_rms_rerun->rms_g, &d_agc->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-            CK(launch_agc_rms(post_src, post_n, qp, d_agc, y, d_agc_ws, st));
+            CK(cudaMemcpyAsync(&d_rms_rerun.data()->rms_g, &d_agc.data()->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+            CK(launch_agc_rms(post_src, post_n, qp, d_agc.data(), y, d_agc_ws.data(), st));
             CK(launch_post(y, post_n, qp, nullptr, 0, nullptr, 1, tap2, d_outp, st));
             launches += 2;
             rms_src = post_src; rms_n = post_n; rms_qp = qp; rms_ready = true; rms_fresh = true; rms_resume_max = 0;
@@ -1156,7 +1076,7 @@ void* iqgpu_host_alloc(size_t bytes)
 void iqgpu_host_free(void* p) { if (p) cudaFreeHost(p); }
 size_t iqgpu_get_bytes_per_sample(int format) { return bytes_per_sample(format); }
 
-static int chain_create_impl(const iqgpu_chain_config* cfgp, int device, iqgpu_chain** out, iqgpu_chain*& in_flight)
+static int chain_create_impl(const iqgpu_chain_config* cfgp, int device, iqgpu_chain** out)
 {
     if (!cfgp || !out) return fail(IQGPU_EINVAL, "null argument");
     *out = nullptr;
@@ -1165,8 +1085,7 @@ static int chain_create_impl(const iqgpu_chain_config* cfgp, int device, iqgpu_c
         return fail(IQGPU_EINVAL, "unhandled input format");       // sample_convert.c:207
     if (!is_complex_format(g.output_format) || !bytes_per_sample(g.output_format))
         return fail(IQGPU_EINVAL, "unhandled output format");      // sample_convert.c:304
-    iqgpu_chain* c = new iqgpu_chain();
-    in_flight = c;                  // the caller frees it if a design step throws
+    std::unique_ptr<iqgpu_chain> c(new iqgpu_chain());
     c->cfg = g;
     c->device = device;
     c->plan_only = device < 0;
@@ -1175,32 +1094,31 @@ static int chain_create_impl(const iqgpu_chain_config* cfgp, int device, iqgpu_c
     c->in_bps = bytes_per_sample(g.input_format);
     c->out_bps = bytes_per_sample(g.output_format);
     std::string err;
-    auto bail = [&](int code, const std::string& m) { in_flight = nullptr; delete c; return fail(code, m); };
-    if (c->in_rate <= 0) return bail(IQGPU_EINVAL, "input sample rate must be positive");
+    if (c->in_rate <= 0) return fail(IQGPU_EINVAL, "input sample rate must be positive");
     // setup.c:91-113
     if (g.no_resample) c->target_rate = (double)c->in_rate;
     c->ratio = (float)(c->target_rate / (double)c->in_rate);
     if (!std::isfinite(c->ratio) || c->ratio < 0.001f || c->ratio > 1000.0f)
-        return bail(IQGPU_EINVAL, "resampling ratio invalid or outside the acceptable range");
+        return fail(IQGPU_EINVAL, "resampling ratio invalid or outside the acceptable range");
     c->dc = design_dc(g.dc_block_enable != 0, c->in_rate);
-    if (g.dc_block_enable && c->dc.alpha <= 0.0f) return bail(IQGPU_EINVAL, "DC block alpha invalid");
+    if (g.dc_block_enable && c->dc.alpha <= 0.0f) return fail(IQGPU_EINVAL, "DC block alpha invalid");
     c->iq_mag = g.iq_mag; c->iq_phase = g.iq_phase;
     // frequency_shift.c:24-84
     // AppResources.nco_shift_hz is a double (frequency_shift.c:32-33 widens the float CLI argument, input_wav.c:614-628
     // stores centre - (double)target): no float round trip here, callers that emulate --freq-shift cast themselves
     const double shift = g.freq_shift_hz;
     if (g.shift_after_resample && std::fabs(shift) < 1e-9)
-        return bail(IQGPU_EINVAL, "--shift-after-resample used without an effective frequency shift");
+        return fail(IQGPU_EINVAL, "--shift-after-resample used without an effective frequency shift");
     if (std::fabs(shift) >= 1e-9) {
         const double rate = g.shift_after_resample ? c->target_rate : (double)c->in_rate;
-        if (std::fabs(shift) > 5.0 * rate) return bail(IQGPU_EINVAL, "frequency shift exceeds the sanity limit");
+        if (std::fabs(shift) > 5.0 * rate) return fail(IQGPU_EINVAL, "frequency shift exceeds the sanity limit");
         c->nco_dtheta = nco_dtheta_for_shift(shift, rate);
         c->nco_sign = shift >= 0 ? 1.0f : -1.0f;
         c->nco_pre = !g.shift_after_resample;
         c->nco_post = g.shift_after_resample != 0;
     }
-    if (!design_resampler(c->ratio, 60.0f, g.no_resample != 0, c->rs, err)) return bail(IQGPU_EINVAL, err);
-    if (!design_filter(g, c->in_rate, c->target_rate, c->filt, err)) return bail(IQGPU_EINVAL, err);
+    if (!design_resampler(c->ratio, 60.0f, g.no_resample != 0, c->rs, err)) return fail(IQGPU_EINVAL, err);
+    if (!design_filter(g, c->in_rate, c->target_rate, c->filt, err)) return fail(IQGPU_EINVAL, err);
     // agc.c:21-84
     if (g.agc_enable && g.agc_profile != IQGPU_AGC_OFF) {
         if (g.agc_profile == IQGPU_AGC_DIGITAL) {
@@ -1223,15 +1141,14 @@ static int chain_create_impl(const iqgpu_chain_config* cfgp, int device, iqgpu_c
         if (!(m & IQGPU_STAGE_AGC)) c->agc_mode = 0;
         if (!(m & IQGPU_STAGE_RESAMPLER)) {
             c->rs = ResamplerPlan();
-            if (!design_resampler(1.0f, 60.0f, true, c->rs, err)) return bail(IQGPU_EINVAL, err);
+            if (!design_resampler(1.0f, 60.0f, true, c->rs, err)) return fail(IQGPU_EINVAL, err);
         }
     }
     if (!c->plan_only) {
         int rc = c->init_device();
-        if (rc != IQGPU_OK) { std::string m = g_err; in_flight = nullptr; delete c; return fail(rc, m); }
+        if (rc != IQGPU_OK) return rc;
     }
-    in_flight = nullptr;
-    *out = c;
+    *out = c.release();
     return IQGPU_OK;
 }
 
@@ -1239,15 +1156,12 @@ static int chain_create_impl(const iqgpu_chain_config* cfgp, int device, iqgpu_c
 // fit memory, a length that went negative before its cast ...) is refused like any other invalid configuration.
 int iqgpu_chain_create(const iqgpu_chain_config* cfgp, int device, iqgpu_chain** out)
 {
-    iqgpu_chain* in_flight = nullptr;
     try {
-        return chain_create_impl(cfgp, device, out, in_flight);
+        return chain_create_impl(cfgp, device, out);
     } catch (const std::bad_alloc&) {
-        delete in_flight;
         if (out) *out = nullptr;
         return fail(IQGPU_ENOMEM, "out of host memory while designing the chain");
     } catch (const std::exception& e) {
-        delete in_flight;
         if (out) *out = nullptr;
         return fail(IQGPU_EINVAL, std::string("configuration cannot be designed: ") + e.what());
     }
@@ -1278,7 +1192,7 @@ int iqgpu_chain_set_option(iqgpu_chain* c, const char* key, int64_t value)
     }
     if (k == "iq_optimize") { c->iq_optimize = value != 0; return IQGPU_OK; }
     if (k == "iq_optimize_interval_ms") { if (value < 0) return fail(IQGPU_EINVAL, "negative interval"); c->iq_interval_ms = (double)value; return IQGPU_OK; }
-    if (k == "iq_optimize_seed") { c->iq_seed = (uint32_t)value; if (c->d_iq_state) return c->iq_push_state(c->last_stream ? c->last_stream : c->stream); return IQGPU_OK; }
+    if (k == "iq_optimize_seed") { c->iq_seed = (uint32_t)value; if (c->d_iq_state.data()) return c->iq_push_state(c->last_stream ? c->last_stream : c->stream); return IQGPU_OK; }
     if (k == "dc_mode") {
         if (c->buffers_ready) return fail(IQGPU_EINVAL, "option must be set before the first process call");
         if (value != 0 && value != 1) return fail(IQGPU_EINVAL, "dc_mode: 0 (exact arithmetic) or 1 (reference fp32 state rounding)");
@@ -1317,7 +1231,7 @@ int iqgpu_chain_get_kernel_times(iqgpu_chain* c, double* ms, uint32_t* launches,
 int iqgpu_chain_set_iq_factors(iqgpu_chain* c, float mag, float phase)
 {
     if (!c) return fail(IQGPU_EINVAL, "null chain");
-    if (c->d_iq_state) {
+    if (c->d_iq_state.data()) {
         int rc = c->iq_sync_state();
         if (rc) return rc;
         c->iq_mag = mag; c->iq_phase = phase;
@@ -1333,8 +1247,8 @@ int iqgpu_chain_get_iq_state(iqgpu_chain* c, float* mag, float* phase, uint64_t*
     if (!c->plan_only) { CK(cudaSetDevice(c->device)); int rc = c->iq_sync_state(); if (rc) return rc; }
     if (mag) *mag = c->iq_mag;
     if (phase) *phase = c->iq_phase;
-    if (passes) *passes = c->h_iq_state ? c->h_iq_state->passes : 0;
-    if (attempts) *attempts = c->h_iq_state ? c->h_iq_state->attempts : 0;
+    if (passes) *passes = c->h_iq_state.data() ? c->h_iq_state.data()->passes : 0;
+    if (attempts) *attempts = c->h_iq_state.data() ? c->h_iq_state.data()->attempts : 0;
     return IQGPU_OK;
 }
 
@@ -1358,13 +1272,13 @@ int iqgpu_chain_get_info(iqgpu_chain* c, iqgpu_chain_info* o)
     o->frames_out_total = c->n_out;
     o->fused_front = c->fused_used ? 1 : 0;
     o->kernel_launches = c->launches;
-    o->halo_frames = c->fused ? fused_halo_frames(c->fused) : (uint32_t)c->rs.halo_input_frames;
-    if (!c->plan_only && c->d_agc) {
+    o->halo_frames = c->fused ? fused_halo_frames(c->fused.get()) : (uint32_t)c->rs.halo_input_frames;
+    if (!c->plan_only && c->d_agc.data()) {
         AgcState a{};
         cudaSetDevice(c->device);
         if (c->last_stream) cudaStreamSynchronize(c->last_stream);
         cudaStreamSynchronize(c->stream);
-        if (cudaMemcpy(&a, c->d_agc, sizeof(a), cudaMemcpyDeviceToHost) == cudaSuccess) {
+        if (cudaMemcpy(&a, c->d_agc.data(), sizeof(a), cudaMemcpyDeviceToHost) == cudaSuccess) {
             o->agc_locked = a.locked; o->agc_gain = a.gain; o->agc_peak_memory = a.peak_mem; o->agc_samples_seen = a.seen;
         }
     }
@@ -1537,7 +1451,7 @@ int iqgpu_chain_pending_chunk_peaks(iqgpu_chain* c, float* peaks, uint32_t* coun
     if (peaks) {
         if (c->pend.peaks_done) {
             CK(cudaSetDevice(c->device));
-            CK(cudaMemcpyAsync(peaks, c->d_seg_peak, c->pend.n_chunks * sizeof(float), cudaMemcpyDeviceToHost, c->last_stream));
+            CK(cudaMemcpyAsync(peaks, c->d_seg_peak.data(), c->pend.n_chunks * sizeof(float), cudaMemcpyDeviceToHost, c->last_stream));
             CK(cudaStreamSynchronize(c->last_stream));
         } else std::fill(peaks, peaks + c->pend.n_chunks, 0.0f);
     }
@@ -1559,7 +1473,7 @@ int iqgpu_chain_pending_chunk_peaks_device(iqgpu_chain* c, size_t skip_chunks, f
     if (st != c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
     if (!live) return IQGPU_OK;
     if (c->pend.peaks_done)
-        CK(cudaMemcpyAsync(dev_peaks, c->d_seg_peak + skip_chunks, live * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        CK(cudaMemcpyAsync(dev_peaks, c->d_seg_peak.data() + skip_chunks, live * sizeof(float), cudaMemcpyDeviceToDevice, st));
     else CK(cudaMemsetAsync(dev_peaks, 0, live * sizeof(float), st));
     return IQGPU_OK;
 }
@@ -1581,49 +1495,33 @@ int iqgpu_chain_agc_advance_device(iqgpu_chain* c, const float* dev_peaks, uint6
     const size_t nch = (size_t)((n_frames + c->chunk_frames - 1) / c->chunk_frames);
     const uint32_t* d_seg = nullptr;
     for (const auto& t : c->prefix_tabs)
-        if (t.first == first_frame && t.frames == n_frames) { d_seg = t.d_seg; break; }
+        if (t.first == first_frame && t.frames == n_frames) { d_seg = t.d_seg.data(); break; }
     if (!d_seg) {
-        const size_t need = (nch + 1) * sizeof(uint32_t);
-        const int sl = c->seg_pin_slot ^= 1;
-        if (need > c->seg_pin_cap[sl]) {
-            if (c->seg_pin[sl]) { CK(cudaEventSynchronize(c->ev_seg[sl])); CK(cudaFreeHost(c->seg_pin[sl])); c->seg_pin[sl] = nullptr; }
-            CK(cudaMallocHost(&c->seg_pin[sl], need * 2));
-            c->seg_pin_cap[sl] = need * 2;
-            if (!c->ev_seg[sl]) CK(cudaEventCreateWithFlags(&c->ev_seg[sl], cudaEventDisableTiming));
-        } else if (c->ev_seg[sl]) CK(cudaEventSynchronize(c->ev_seg[sl]));
-        uint32_t* seg = c->seg_pin[sl];
-        uint64_t before = chain_outputs_after(c, first_frame);
-        seg[0] = 0;
-        for (size_t k = 0; k < nch; k++) {
-            const uint64_t end = std::min<uint64_t>(first_frame + n_frames, first_frame + (uint64_t)(k + 1) * c->chunk_frames);
-            const uint64_t after = chain_outputs_after(c, end);
-            seg[k + 1] = seg[k] + (uint32_t)(after - before);       // the scan uses differences only: wrap-around is harmless
-            before = after;
-        }
         if (c->prefix_tabs.size() >= 16) {                          // rare: a new plan; drop the oldest table once it is idle
             CK(cudaStreamSynchronize(st));
-            cudaFree(c->prefix_tabs.front().d_seg);
             c->prefix_tabs.erase(c->prefix_tabs.begin());
         }
         iqgpu_chain::PrefixTab t;
-        t.first = first_frame; t.frames = n_frames; t.nch = nch;
-        CK(cudaMalloc(&t.d_seg, need));
-        CK(cudaMemcpyAsync(t.d_seg, seg, need, cudaMemcpyHostToDevice, st));
-        CK(cudaEventRecord(c->ev_seg[sl], st));
-        c->prefix_tabs.push_back(t);
-        d_seg = t.d_seg;
+        t.first = first_frame; t.frames = n_frames;
+        CK(t.d_seg.alloc(nch + 1));
+        rc = c->stage_chunk_table(t.d_seg.data(), nch, st, [&](uint32_t* seg) {
+            uint64_t before = chain_outputs_after(c, first_frame);
+            seg[0] = 0;
+            for (size_t k = 0; k < nch; k++) {
+                const uint64_t end = std::min<uint64_t>(first_frame + n_frames, first_frame + (uint64_t)(k + 1) * c->chunk_frames);
+                const uint64_t after = chain_outputs_after(c, end);
+                seg[k + 1] = seg[k] + (uint32_t)(after - before);   // the scan uses differences only: wrap-around is harmless
+                before = after;
+            }
+        });
+        if (rc) return rc;
+        d_seg = t.d_seg.data();
+        c->prefix_tabs.push_back(std::move(t));
     }
     PostParams qp{};
     qp.agc_mode = c->agc_mode; qp.agc_target = c->agc_target; qp.agc_alpha = c->agc_alpha; qp.target_rate = c->target_rate;
-    const size_t qneed = agc_quiet_workspace_bytes(nch);
-    if (qneed > c->agc_quiet_bytes) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(c->d_agc_quiet);
-        c->d_agc_quiet = nullptr; c->agc_quiet_bytes = 0;
-        CK(cudaMalloc(&c->d_agc_quiet, qneed * 2));
-        c->agc_quiet_bytes = qneed * 2;
-    }
-    CK(launch_agc_digital_scan(d_seg, nch, dev_peaks, qp, c->d_agc, nullptr, st, c->d_agc_quiet));
+    CK(c->ensure_agc_quiet(nch, st));
+    CK(launch_agc_digital_scan(d_seg, nch, dev_peaks, qp, c->d_agc.data(), nullptr, st, c->d_agc_quiet.data()));
     return IQGPU_OK;
 }
 
@@ -1651,7 +1549,7 @@ int iqgpu_chain_get_agc_state(iqgpu_chain* c, iqgpu_agc_state* s)
     if (c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
     CK(cudaStreamSynchronize(c->stream));
     AgcState a{};
-    CK(cudaMemcpy(&a, c->d_agc, sizeof(a), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&a, c->d_agc.data(), sizeof(a), cudaMemcpyDeviceToHost));
     s->locked = (uint32_t)a.locked; s->gain = a.gain; s->peak_memory = a.peak_mem; s->samples_seen = a.seen;
     s->last_strong_s = a.last_strong;
     return IQGPU_OK;
@@ -1666,11 +1564,11 @@ int iqgpu_chain_set_agc_state(iqgpu_chain* c, const iqgpu_agc_state* s)
     if (rc) return rc;
     cudaStream_t st = c->last_stream ? c->last_stream : c->stream;
     AgcState a{};
-    CK(cudaMemcpyAsync(&a, c->d_agc, sizeof(a), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&a, c->d_agc.data(), sizeof(a), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     a.locked = (int)s->locked; a.gain = s->gain; a.peak_mem = s->peak_memory; a.seen = s->samples_seen;
     a.last_strong = s->last_strong_s;
-    CK(cudaMemcpyAsync(c->d_agc, &a, sizeof(a), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(c->d_agc.data(), &a, sizeof(a), cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));
     return IQGPU_OK;
 }
@@ -1685,7 +1583,7 @@ int iqgpu_chain_agc_rms_state_device(iqgpu_chain* c, float* dev_state, void* cud
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
     if (c->last_stream && st != c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
     static_assert(offsetof(AgcState, rms_y2) == offsetof(AgcState, rms_g) + sizeof(float), "{g, y2'} must be adjacent");
-    CK(cudaMemcpyAsync(dev_state, &c->d_agc->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(dev_state, &c->d_agc.data()->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
     return IQGPU_OK;
 }
 
@@ -1705,7 +1603,7 @@ int iqgpu_chain_agc_rms_resume_device(iqgpu_chain* c, size_t first_output, const
     if (c->last_stream && st != c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
     c->last_stream = st;
     if (first_output == c->rms_n) {            // at the end of the call: no output changes, the end state is the given one
-        agc_rms_set_end_kernel<<<1, 1, 0, st>>>(c->d_agc, reinterpret_cast<const float2*>(dev_state), dev_changed);
+        agc_rms_set_end_kernel<<<1, 1, 0, st>>>(c->d_agc.data(), reinterpret_cast<const float2*>(dev_state), dev_changed);
         CK(cudaGetLastError());
         c->rms_fresh = true;                    // the trajectory in memory no longer ends in the end state
         c->launches += 1;
@@ -1715,7 +1613,7 @@ int iqgpu_chain_agc_rms_resume_device(iqgpu_chain* c, size_t first_output, const
         if (dev_changed) CK(cudaMemsetAsync(dev_changed, 0, sizeof(int), st));
         return IQGPU_OK;
     }
-    if (!c->d_rms_resume) CK(cudaMalloc(&c->d_rms_resume, sizeof(AgcRmsResume)));
+    if (!c->d_rms_resume.data()) CK(c->d_rms_resume.alloc(1));
     // A resume compares its trajectory with the checkpoints of the one in memory and stops where the two meet.  Behind an
     // earlier resume's frame that trajectory is the earlier resume's, while the rows in front of the frame still hold the
     // call's own: a resume in front of it would meet the call's trajectory and stop, and leave the earlier resume's
@@ -1724,17 +1622,17 @@ int iqgpu_chain_agc_rms_resume_device(iqgpu_chain* c, size_t first_output, const
     // converts the whole call again.  Resumes at the same or a later frame, the time-shard hand-over, need none of this.
     const bool rerun = first_output < c->rms_resume_max;
     if (rerun) {
-        AgcState* s = c->d_rms_rerun + 1;         // [0] keeps the start state for the next re-run
-        CK(cudaMemcpyAsync(&s->rms_g, &c->d_rms_rerun->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-        CK(launch_agc_rms(c->rms_src, c->rms_n, c->rms_qp, s, c->d_agc_scratch, c->d_agc_ws, st));
+        AgcState* s = c->d_rms_rerun.data() + 1;         // [0] keeps the start state for the next re-run
+        CK(cudaMemcpyAsync(&s->rms_g, &c->d_rms_rerun.data()->rms_g, 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        CK(launch_agc_rms(c->rms_src, c->rms_n, c->rms_qp, s, c->d_agc_scratch.data(), c->d_agc_ws.data(), st));
     }
-    CK(launch_agc_rms_resume(c->rms_src, c->rms_n, c->rms_qp, c->d_agc, c->d_agc_scratch, c->d_agc_ws, first_output,
-                             reinterpret_cast<const float2*>(dev_state), c->d_rms_resume, c->rms_fresh || rerun, dev_changed,
+    CK(launch_agc_rms_resume(c->rms_src, c->rms_n, c->rms_qp, c->d_agc.data(), c->d_agc_scratch.data(), c->d_agc_ws.data(), first_output,
+                             reinterpret_cast<const float2*>(dev_state), c->d_rms_resume.data(), c->rms_fresh || rerun, dev_changed,
                              st));
     c->rms_fresh = false;
     c->rms_resume_max = rerun ? first_output : std::max(c->rms_resume_max, first_output);
-    if (rerun) CK(launch_post(c->d_agc_scratch, c->rms_n, c->rms_qp, nullptr, 0, nullptr, 1, nullptr, dev_out, st));
-    else CK(launch_convert_range(c->d_agc_scratch, c->d_rms_resume, c->cfg.output_format, dev_out, st));
+    if (rerun) CK(launch_post(c->d_agc_scratch.data(), c->rms_n, c->rms_qp, nullptr, 0, nullptr, 1, nullptr, dev_out, st));
+    else CK(launch_convert_range(c->d_agc_scratch.data(), c->d_rms_resume.data(), c->cfg.output_format, dev_out, st));
     c->launches += rerun ? 3 : 2;
     return IQGPU_OK;
 }
@@ -1747,7 +1645,7 @@ int iqgpu_chain_get_agc_rms_state(iqgpu_chain* c, float* g, float* y2)
     if (c->last_stream) CK(cudaStreamSynchronize(c->last_stream));
     CK(cudaStreamSynchronize(c->stream));
     AgcState a{};
-    CK(cudaMemcpy(&a, c->d_agc, sizeof(a), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&a, c->d_agc.data(), sizeof(a), cudaMemcpyDeviceToHost));
     *g = a.rms_g; *y2 = a.rms_y2;
     return IQGPU_OK;
 }
@@ -1846,28 +1744,13 @@ int iqgpu_chain_process_multi(iqgpu_chain* const* chains, size_t K, const void* 
             return fail(IQGPU_ECAPACITY, chan(k) + "output buffer too small");
     }
     // staging slots sized for one sub-train: the raw input in channel 0's, each channel's output in its own
+    // (the previous call ended with a synchronisation: nothing still uses the slots)
     const size_t raw_need = (sub + 16) * c0->in_bps;
-    if (c0->d_raw_bytes < raw_need) {
-        c0->d_raw_bytes = 0;
-        for (int i = 0; i < 2; i++) {
-            cudaFree(c0->d_raw[i]);
-            c0->d_raw[i] = nullptr;
-            CK(cudaMalloc(&c0->d_raw[i], raw_need));
-        }
-        c0->d_raw_bytes = raw_need;
-    }
+    for (auto& r : c0->d_raw) CK(r.grow(raw_need, raw_need, no_drain));
     for (size_t k = 0; k < K; k++) {
         iqgpu_chain* c = chains[k];
         const size_t out_need = c->max_out_for(sub) * c->out_bps;
-        if (c->d_out_bytes < out_need) {
-            c->d_out_bytes = 0;
-            for (int i = 0; i < 2; i++) {
-                cudaFree(c->d_out[i]);
-                c->d_out[i] = nullptr;
-                CK(cudaMalloc(&c->d_out[i], out_need));
-            }
-            c->d_out_bytes = out_need;
-        }
+        for (auto& o : c->d_out) CK(o.grow(out_need, out_need, no_drain));
         rc = c->order_after_reset(c->stream);
         if (rc) return rc;
         c->last_stream = c->stream;
@@ -1885,7 +1768,7 @@ int iqgpu_chain_process_multi(iqgpu_chain* const* chains, size_t K, const void* 
         // which follows that channel's compute on the slot's previous contents
         if (used[slot])
             for (size_t k = 0; k < K; k++) CK(cudaStreamWaitEvent(c0->h2d, chains[k]->ev_d2h[slot], 0));
-        CK(cudaMemcpyAsync(c0->d_raw[slot], (const char*)raw_in + in_off * c0->in_bps, n * c0->in_bps, cudaMemcpyHostToDevice, c0->h2d));
+        CK(cudaMemcpyAsync(c0->d_raw[slot].data(), (const char*)raw_in + in_off * c0->in_bps, n * c0->in_bps, cudaMemcpyHostToDevice, c0->h2d));
         CK(cudaEventRecord(c0->ev_h2d[slot], c0->h2d));
         for (size_t k = 0; k < K; k++) {
             iqgpu_chain* c = chains[k];
@@ -1893,14 +1776,14 @@ int iqgpu_chain_process_multi(iqgpu_chain* const* chains, size_t K, const void* 
             size_t produced = 0;
             c->dc_slot = 0; c->dc_prepared = false;      // host path is PCIe bound: DC pre-pass inline on the compute stream
             uint32_t* pc = per_chunk_out ? per_chunk_out[k] : nullptr;
-            rc = c->run_subtrain(c0->d_raw[slot], n, chunks.data() + ci, cj - ci, c->d_out[slot], &produced,
+            rc = c->run_subtrain(c0->d_raw[slot].data(), n, chunks.data() + ci, cj - ci, c->d_out[slot].data(), &produced,
                                  pc ? pc + ci : nullptr, c->stream);
             if (rc) return rc;
             launches[k] += c->launches;
             CK(cudaEventRecord(c->ev_done[slot], c->stream));
             CK(cudaStreamWaitEvent(c->d2h, c->ev_done[slot], 0));
             if (produced)
-                CK(cudaMemcpyAsync((char*)out[k] + out_off[k], c->d_out[slot], produced * c->out_bps, cudaMemcpyDeviceToHost, c->d2h));
+                CK(cudaMemcpyAsync((char*)out[k] + out_off[k], c->d_out[slot].data(), produced * c->out_bps, cudaMemcpyDeviceToHost, c->d2h));
             CK(cudaEventRecord(c->ev_d2h[slot], c->d2h));
             out_off[k] += produced * c->out_bps; total[k] += produced;
         }
@@ -1929,7 +1812,7 @@ int iqgpu_chain_read_tap(iqgpu_chain* c, int tapi, float* host_cf32, size_t capa
     *frames = n;
     if (host_cf32) {
         if (n > capacity_frames) return fail(IQGPU_ECAPACITY, "tap buffer too small");
-        if (n) CK(cudaMemcpy(host_cf32, c->tap[tapi].p, n * sizeof(float2), cudaMemcpyDeviceToHost));
+        if (n) CK(cudaMemcpy(host_cf32, c->tap[tapi].buf.data(), n * sizeof(float2), cudaMemcpyDeviceToHost));
     }
     return IQGPU_OK;
 }

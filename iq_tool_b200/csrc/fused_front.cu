@@ -18,8 +18,10 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <vector>
 
+#include "cuda_owned.hpp"
 #include "device_common.cuh"
 #include "fused_front2.cuh"
 #include "kernels.hpp"
@@ -27,14 +29,12 @@
 namespace iqgpu {
 
 struct FusedFront {
-    float2* d_tail[2] = {nullptr, nullptr};
+    DeviceArray<float2> d_tail[2];
     int tail_cur = 0;
     // DC pre-pass products, double buffered so that the (HBM-bound) pre-pass of the next sub-train can
     // run on a second stream underneath the (issue-bound) front kernel of the current one
-    double2* d_dc_table[2] = {nullptr, nullptr};
-    double2* d_dc_sums[2] = {nullptr, nullptr};
-    double* d_dc_ws[2] = {nullptr, nullptr};
-    size_t dc_cap[2] = {0, 0};
+    DeviceArray<double2> d_dc_table[2], d_dc_sums[2];
+    DeviceArray<double> d_dc_ws[2];
     bool dc_ready[2] = {false, false};  // slot holds the table of the sub-train about to be launched
     int num_sms = 148;
     int format = 0;
@@ -45,15 +45,14 @@ struct FusedFront {
     float v2_zeta = 1.f;
     uint32_t v2_step = 0;
     int H_tail = 0;                     // cf32 tail length of the plan
-    float2* d_bank_image = nullptr;     // polyphase bank in the v2 shared-memory layout (w2_bank_row)
-    float2* d_bank_image_q = nullptr;   // ... and in the layout of the four-output variant (w2_qbank_chunk, rotation arb_tz)
+    DeviceArray<float2> d_bank_image;   // polyphase bank in the v2 shared-memory layout (w2_bank_row)
+    DeviceArray<float2> d_bank_image_q; // ... and in the layout of the four-output variant (w2_qbank_chunk, rotation arb_tz)
     int arb_tz = 0, arb_b2 = 0, arb_b3 = 0, arb_skew_sh = 31;
     bool arb_quad_ok = false;
     // local DC state (fused_front2.cuh, DC == 2): per-warp records, per-stretch corrections, row gains of the polyphase stage
-    W2DcStretch* d_dc_stretch = nullptr;
-    W2DcCorr* d_dc_corr = nullptr;
-    size_t dc_stretch_cap = 0;
-    float* d_dc_G = nullptr;
+    DeviceArray<W2DcStretch> d_dc_stretch;
+    DeviceArray<W2DcCorr> d_dc_corr;
+    DeviceArray<float> d_dc_G;
     float dc_G_for_c = -1.f;            // pole the gains were computed for
     double dc_atot = 1.0;
     std::vector<float> h_bank;          // host copy of the 256 x 14 polyphase bank
@@ -153,31 +152,27 @@ bool fused_supported(int format, const ResamplerDesc& r)
 
 FusedFront* fused_create(int format, const ResamplerDesc& r, bool nco, const float* d_bank, int num_sms, std::string& err)
 {
-    FusedFront* f = new FusedFront();
+    std::unique_ptr<FusedFront> f(new FusedFront());
     f->format = format;
     f->num_sms = num_sms;
-    if (!v2_setup(f, r, nco)) { err = "fused front: no compiled plan fits this cascade"; delete f; return nullptr; }
-    if (cudaMalloc(&f->d_tail[0], (size_t)f->H_tail * sizeof(float2)) != cudaSuccess ||
-        cudaMalloc(&f->d_tail[1], (size_t)f->H_tail * sizeof(float2)) != cudaSuccess) {
+    if (!v2_setup(f.get(), r, nco)) { err = "fused front: no compiled plan fits this cascade"; return nullptr; }
+    if (f->d_tail[0].alloc(f->H_tail) != cudaSuccess || f->d_tail[1].alloc(f->H_tail) != cudaSuccess) {
         err = "fused front: device allocation failed";
-        fused_destroy(f);
         return nullptr;
     }
     // lay the bank out the way the kernel reads it, so one TMA bulk copy stages it per CTA
     std::vector<float> hb(256 * 14);
     std::vector<float2> img(W2_BANK_F2, make_float2(0.f, 0.f));
     if (cudaMemcpy(hb.data(), d_bank, hb.size() * sizeof(float), cudaMemcpyDeviceToHost) != cudaSuccess ||
-        cudaMalloc(&f->d_bank_image, img.size() * sizeof(float2)) != cudaSuccess) {
+        f->d_bank_image.alloc(img.size()) != cudaSuccess) {
         err = "fused front: bank image allocation failed";
-        fused_destroy(f);
         return nullptr;
     }
     f->h_bank = hb;
     for (int idx = 0; idx < 256; idx++)
         for (int i = 0; i < 7; i++) img[w2_bank_row(idx) + i] = make_float2(hb[idx * 14 + 2 * i], hb[idx * 14 + 2 * i + 1]);
-    if (cudaMemcpy(f->d_bank_image, img.data(), img.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) {
+    if (cudaMemcpy(f->d_bank_image.data(), img.data(), img.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) {
         err = "fused front: bank image upload failed";
-        fused_destroy(f);
         return nullptr;
     }
     // four-output variant: rows of 16 floats, rotated / chunk-permuted for this rate (fused_front2.cuh)
@@ -194,34 +189,24 @@ FusedFront* fused_create(int format, const ResamplerDesc& r, bool nco, const flo
             for (unsigned j = 0; j < 4; j++)
                 for (unsigned t = 0; t < 4; t++)
                     if (4 * j + t < 14) q[w2_qbank_chunk(idx, (unsigned)f->arb_tz, j) + t] = hb[idx * 14 + 4 * j + t];
-        if (cudaMalloc(&f->d_bank_image_q, q.size() * sizeof(float)) != cudaSuccess ||
-            cudaMemcpy(f->d_bank_image_q, q.data(), q.size() * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess) {
+        if (f->d_bank_image_q.alloc(q.size() / 2) != cudaSuccess ||
+            cudaMemcpy(f->d_bank_image_q.data(), q.data(), q.size() * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess) {
             err = "fused front: bank image upload failed";
-            fused_destroy(f);
             return nullptr;
         }
     }
-    return f;
+    return f.release();
 }
 
-void fused_destroy(FusedFront* f)
-{
-    if (!f) return;
-    cudaFree(f->d_tail[0]); cudaFree(f->d_tail[1]);
-    for (int i = 0; i < 2; i++) { cudaFree(f->d_dc_table[i]); cudaFree(f->d_dc_sums[i]); cudaFree(f->d_dc_ws[i]); }
-    cudaFree(f->d_bank_image);
-    cudaFree(f->d_bank_image_q);
-    cudaFree(f->d_dc_stretch); cudaFree(f->d_dc_corr); cudaFree(f->d_dc_G);
-    delete f;
-}
+void fused_destroy(FusedFront* f) { delete f; }
 
 cudaError_t fused_reset(FusedFront* f, cudaStream_t st)
 {
     f->tail_cur = 0;
     f->dc_ready[0] = f->dc_ready[1] = false;
-    cudaError_t e = cudaMemsetAsync(f->d_tail[0], 0, (size_t)f->H_tail * sizeof(float2), st);
+    cudaError_t e = cudaMemsetAsync(f->d_tail[0].data(), 0, (size_t)f->H_tail * sizeof(float2), st);
     if (e != cudaSuccess) return e;
-    return cudaMemsetAsync(f->d_tail[1], 0, (size_t)f->H_tail * sizeof(float2), st);
+    return cudaMemsetAsync(f->d_tail[1].data(), 0, (size_t)f->H_tail * sizeof(float2), st);
 }
 
 uint32_t fused_halo_frames(const FusedFront* f)
@@ -234,11 +219,11 @@ uint32_t fused_halo_frames(const FusedFront* f)
 // state, frame not on a tick boundary)
 const double2* fused_dc_state_at(const FusedFront* f, int slot, int64_t n0, int64_t pos)
 {
-    if (slot < 0 || slot > 1 || !f->d_dc_table[slot] || pos < n0) return nullptr;
+    if (slot < 0 || slot > 1 || !f->d_dc_table[slot].data() || pos < n0) return nullptr;
     const int64_t A0 = (n0 / W2_T0) * W2_T0;
     if ((pos - A0) % W2_T0) return nullptr;
     const size_t idx = (size_t)((pos - A0) / W2_T0);
-    return idx < f->dc_cap[slot] ? f->d_dc_table[slot] + idx : nullptr;
+    return idx < f->d_dc_table[slot].size() ? f->d_dc_table[slot].data() + idx : nullptr;
 }
 
 __global__ void dc_rewind_kernel(double2* carry, double c, long long k)
@@ -254,25 +239,23 @@ static cudaError_t fused_dc_prepass(FusedFront* f, int slot, const void* raw, lo
 {
     const size_t nv = (size_t)(N1 - A0);
     const size_t n_runs = (nv + 511) / 512;          // one table entry per 512-frame tick
-    if (n_runs + 2 > f->dc_cap[slot]) {
-        cudaDeviceSynchronize();        // rare (first use / larger sub-train): nothing may still read the old buffers
-        cudaFree(f->d_dc_table[slot]); cudaFree(f->d_dc_sums[slot]); cudaFree(f->d_dc_ws[slot]);
-        f->d_dc_table[slot] = nullptr; f->d_dc_sums[slot] = nullptr; f->d_dc_ws[slot] = nullptr;
-        f->dc_cap[slot] = n_runs * 2 + 16;
-        cudaError_t e = cudaMalloc(&f->d_dc_table[slot], f->dc_cap[slot] * sizeof(double2));
-        if (e != cudaSuccess) return e;
-        e = cudaMalloc(&f->d_dc_sums[slot], f->dc_cap[slot] * sizeof(double2));
-        if (e != cudaSuccess) return e;
-        e = cudaMalloc(&f->d_dc_ws[slot], dc_scan_workspace_doubles(f->dc_cap[slot]) * sizeof(double));
-        if (e != cudaSuccess) return e;
-    }
+    // rare (first use / larger sub-train): nothing may still read the old buffers
+    auto drain = [] { return cudaDeviceSynchronize(); };
+    const size_t cap = n_runs * 2 + 16;
+    cudaError_t e = f->d_dc_table[slot].grow(n_runs + 2, cap, drain);
+    if (e == cudaSuccess) e = f->d_dc_sums[slot].grow(n_runs + 2, cap, drain);
+    // the scan's workspace covers the table
+    const size_t ws = dc_scan_workspace_doubles(f->d_dc_table[slot].size());
+    if (e == cudaSuccess) e = f->d_dc_ws[slot].grow(ws, ws, drain);
+    if (e != cudaSuccess) return e;
     const size_t bps = (pre.format == IQGPU_FMT_CS8 || pre.format == IQGPU_FMT_CU8) ? 2 : (pre.format == IQGPU_FMT_CF32 ? 8 : 4);
     const long long back = n0 - A0;
     const char* vraw = reinterpret_cast<const char*>(raw) - back * (long long)bps;
     if (back) dc_rewind_kernel<<<1, 1, 0, st>>>(d_carry, (double)pre.dc_c, back);
-    cudaError_t e = launch_dc_tick_sums(vraw, nv, (size_t)back, pre, f->d_dc_sums[slot], st);
+    e = launch_dc_tick_sums(vraw, nv, (size_t)back, pre, f->d_dc_sums[slot].data(), st);
     if (e != cudaSuccess) return e;
-    return launch_dc_scan(f->d_dc_sums[slot], n_runs, 512, nv, pre.dc_c, d_carry, f->d_dc_table[slot], f->d_dc_ws[slot], st, 512);
+    return launch_dc_scan(f->d_dc_sums[slot].data(), n_runs, 512, nv, pre.dc_c, d_carry, f->d_dc_table[slot].data(),
+                          f->d_dc_ws[slot].data(), st, 512);
 }
 
 // DC pre-pass of the sub-train [n0, n0+n) into table slot `slot`, on stream `st` (which may differ from the
@@ -287,7 +270,7 @@ static bool v2_dc_local(const PreParams& pre)
 // gains of the cascade for the sequence c^n (see fused_front2.cuh): Atot over the halfband stages, G per polyphase row
 static cudaError_t v2_dc_gains(FusedFront* f, float c, cudaStream_t st)
 {
-    if (f->dc_G_for_c == c && f->d_dc_G) return cudaSuccess;
+    if (f->dc_G_for_c == c && f->d_dc_G.data()) return cudaSuccess;
     double mu = (double)c, atot = 1.0;
     int k = 0;
     for (int d = 0; d < f->v2_S; d++) {
@@ -306,11 +289,11 @@ static cudaError_t v2_dc_gains(FusedFront* f, float c, cudaStream_t st)
         G[idx] = (float)g;
     }
     cudaError_t e = cudaSuccess;
-    if (!f->d_dc_G) e = cudaMalloc(&f->d_dc_G, 256 * sizeof(float));
+    if (!f->d_dc_G.data()) e = f->d_dc_G.alloc(256);
     if (e != cudaSuccess) return e;
     e = cudaStreamSynchronize(st);           // first use / new pole only
     if (e != cudaSuccess) return e;
-    e = cudaMemcpy(f->d_dc_G, G.data(), 256 * sizeof(float), cudaMemcpyHostToDevice);
+    e = cudaMemcpy(f->d_dc_G.data(), G.data(), 256 * sizeof(float), cudaMemcpyHostToDevice);
     if (e == cudaSuccess) f->dc_G_for_c = c;
     return e;
 }
@@ -354,13 +337,13 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     if (dc_slot < 0 || dc_slot > 1) dc_slot = 0;
     Fused2Args A{};
     A.raw = raw; A.n0 = n0; A.N1 = n0 + (long long)n;
-    A.tail_in = f->d_tail[f->tail_cur];
-    A.tail_out = f->d_tail[f->tail_cur ^ 1];
+    A.tail_in = f->d_tail[f->tail_cur].data();
+    A.tail_out = f->d_tail[f->tail_cur ^ 1].data();
     A.H_tail = f->H_tail;
     A.pre = pre;
     A.dc = make_dc_dev16(pre.dc_enable ? pre.dc_c : 0.f, pre.dc_a);
     A.A0 = (n0 / W2_T0) * W2_T0;                 // the tick that contains n0 starts the DC table
-    A.bank_image = f->d_bank_image;
+    A.bank_image = f->d_bank_image.data();
     A.O0 = O0; A.O1 = O0 + (long long)n_out; A.y = y;
     A.step = f->v2_step; A.zeta = f->v2_zeta;
     A.lut_sh = 4; A.lut_mask = 0;
@@ -399,7 +382,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     cudaError_t e;
     if ((long long)n < f->H_tail) {
         const size_t keep = (size_t)f->H_tail - n;
-        e = cudaMemcpyAsync(f->d_tail[f->tail_cur ^ 1], f->d_tail[f->tail_cur] + n, keep * sizeof(float2),
+        e = cudaMemcpyAsync(f->d_tail[f->tail_cur ^ 1].data(), f->d_tail[f->tail_cur].data() + n, keep * sizeof(float2),
                             cudaMemcpyDeviceToDevice, st);
         if (e != cudaSuccess) return e;
     }
@@ -408,20 +391,13 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     if (dc_local) {
         e = v2_dc_gains(f, pre.dc_c, st);
         if (e != cudaSuccess) return e;
-        if ((size_t)warps_needed > f->dc_stretch_cap) {
-            e = cudaStreamSynchronize(st);
-            if (e != cudaSuccess) return e;
-            cudaFree(f->d_dc_stretch); cudaFree(f->d_dc_corr);
-            f->d_dc_stretch = nullptr; f->d_dc_corr = nullptr;
-            f->dc_stretch_cap = (size_t)warps_needed + 64;
-            e = cudaMalloc(&f->d_dc_stretch, f->dc_stretch_cap * sizeof(W2DcStretch));
-            if (e != cudaSuccess) return e;
-            e = cudaMalloc(&f->d_dc_corr, f->dc_stretch_cap * sizeof(W2DcCorr));
-            if (e != cudaSuccess) return e;
-        }
+        auto drain = [st] { return cudaStreamSynchronize(st); };
+        e = f->d_dc_stretch.grow((size_t)warps_needed, (size_t)warps_needed + 64, drain);
+        if (e == cudaSuccess) e = f->d_dc_corr.grow((size_t)warps_needed, (size_t)warps_needed + 64, drain);
+        if (e != cudaSuccess) return e;
         const double c = (double)pre.dc_c;
         A.dc_carry = d_dc_carry;
-        A.dc_stretch = f->d_dc_stretch;
+        A.dc_stretch = f->d_dc_stretch.data();
         A.dc_lnc = log(c);
         A.dc_c512 = pow(c, 512.0);
         geo.n_stretch = (int)warps_needed;
@@ -439,7 +415,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
             if (launches) *launches += 2;
         }
         f->dc_ready[dc_slot] = false;
-        A.dc_table = f->d_dc_table[dc_slot];
+        A.dc_table = f->d_dc_table[dc_slot].data();
         A.dc_table_shift = 9;
     }
     const int dc = dc_local ? 2 : (pre.dc_enable ? 1 : 0);
@@ -459,7 +435,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     A.arb_tz = f->arb_tz; A.arb_b2 = f->arb_b2; A.arb_b3 = f->arb_b3;
     auto set_mode = [&](int m) {
         A.arb_pairs = m;
-        A.bank_image = (m == 2) ? f->d_bank_image_q : f->d_bank_image;
+        A.bank_image = (m == 2) ? f->d_bank_image_q.data() : f->d_bank_image.data();
         A.arb_skew_sh = (m == 2) ? f->arb_skew_sh : 31;
     };
     if (const char* force = getenv("IQGPU_ARB_PAIRS")) {
@@ -469,8 +445,8 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     if (f->arb_pairs < 0 && n >= ((size_t)1 << 22)) {
         // time the variants on this launch (same inputs, same outputs: every run overwrites the last with equal bits)
         const int nmodes = f->arb_quad_ok ? 3 : 2;
-        cudaEvent_t ev[4];
-        for (auto& x : ev) cudaEventCreate(&x);
+        Event ev[4];
+        for (auto& x : ev) create(x, cudaEventDefault);
         float ms[3] = {0.f, 0.f, 0.f};
         set_mode(1); e = go(A);                          // untimed: caches, clocks, TMA descriptors warm for all candidates
         cudaEventRecord(ev[0], st);
@@ -490,7 +466,6 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
                 fprintf(stderr, "iqgpu: polyphase stage: one output per lane %.3f ms, two %.3f ms, four %.3f ms -> mode %d (tz %d, B2 %d, B3 %d, skew %d)\n",
                         ms[0], ms[1], ms[2], best, f->arb_tz, f->arb_b2, f->arb_b3, f->arb_skew_sh);
         }
-        for (auto& x : ev) cudaEventDestroy(x);
         if (launches) *launches += (uint32_t)nmodes;
         if (e == cudaSuccess && A.arb_pairs != f->arb_pairs) { set_mode(f->arb_pairs); e = go(A); if (launches) *launches += 1; }
     } else {
@@ -499,14 +474,15 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     }
     if (launches) *launches += 1;
     if (dc_local && e == cudaSuccess) {
-        w2_dc_scan_kernel<<<1, 1024, 0, st>>>(f->d_dc_stretch, geo, f->d_dc_corr, d_dc_carry);
+        w2_dc_scan_kernel<<<1, 1024, 0, st>>>(f->d_dc_stretch.data(), geo, f->d_dc_corr.data(), d_dc_carry);
         // a consumer that adds the term to the resampled stream itself leaves only the cf32 tail to this pass
         const long long O1c = fold ? A.O0 : A.O1;
-        if (fold) *fold = DcFold{f->d_dc_corr, f->d_dc_G, geo, A.O0, A.step, f->v2_S};
+        if (fold) *fold = DcFold{f->d_dc_corr.data(), f->d_dc_G.data(), geo, A.O0, A.step, f->v2_S};
         const long long work = (O1c - A.O0) + f->H_tail;
         const int cgrid = (int)std::min<long long>((work + 255) / 256, 148LL * 16);
-        w2_dc_correct_kernel<<<std::max(cgrid, 1), 256, 0, st>>>(y, A.O0, O1c, A.step, f->v2_S, geo, f->d_dc_corr, f->d_dc_G,
-                                                               f->d_tail[f->tail_cur ^ 1], A.N1 - f->H_tail, A.n0, A.N1);
+        w2_dc_correct_kernel<<<std::max(cgrid, 1), 256, 0, st>>>(y, A.O0, O1c, A.step, f->v2_S, geo, f->d_dc_corr.data(),
+                                                               f->d_dc_G.data(), f->d_tail[f->tail_cur ^ 1].data(), A.N1 - f->H_tail,
+                                                               A.n0, A.N1);
         e = cudaGetLastError();
         if (launches) *launches += 2;
     }

@@ -12,6 +12,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/iqgpu.h"
+#include "cuda_owned.hpp"
 #include "fft_core.cuh"
 #include "kernels.hpp"
 
@@ -198,22 +199,20 @@ float iq_direction_host(unsigned seed, unsigned long long pass, unsigned k) { re
 cudaError_t iq_optimize_device(const float* host_block1024, const float* host_dirs50, float* mag, float* phase,
                                float* avg_power, float* power_range, int* optimized)
 {
-    float2* d_block = nullptr;
-    float* d_dirs = nullptr;
-    IqOptResult* d_out = nullptr;
-    cudaError_t e;
-    if ((e = cudaMalloc(&d_block, IQ_NFFT * sizeof(float2))) != cudaSuccess) return e;
-    if ((e = cudaMalloc(&d_dirs, 2 * IQ_PASSES * sizeof(float))) != cudaSuccess) { cudaFree(d_block); return e; }
-    if ((e = cudaMalloc(&d_out, sizeof(IqOptResult))) != cudaSuccess) { cudaFree(d_block); cudaFree(d_dirs); return e; }
+    DeviceArray<float2> d_block;
+    DeviceArray<float> d_dirs;
+    DeviceArray<IqOptResult> d_out;
+    cudaError_t e = d_block.alloc(IQ_NFFT);
+    if (e == cudaSuccess) e = d_dirs.alloc(2 * IQ_PASSES);
+    if (e == cudaSuccess) e = d_out.alloc(1);
     IqOptResult r{};
-    e = cudaMemcpy(d_block, host_block1024, IQ_NFFT * sizeof(float2), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(d_dirs, host_dirs50, 2 * IQ_PASSES * sizeof(float), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(d_block.data(), host_block1024, IQ_NFFT * sizeof(float2), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(d_dirs.data(), host_dirs50, 2 * IQ_PASSES * sizeof(float), cudaMemcpyHostToDevice);
     if (e == cudaSuccess) {
-        iq_optimize_kernel<<<1, IQ_THREADS, sizeof(IqShared)>>>(d_block, d_dirs, *mag, *phase, d_out);
+        iq_optimize_kernel<<<1, IQ_THREADS, sizeof(IqShared)>>>(d_block.data(), d_dirs.data(), *mag, *phase, d_out.data());
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = cudaMemcpy(&r, d_out, sizeof(r), cudaMemcpyDeviceToHost);
-    cudaFree(d_block); cudaFree(d_dirs); cudaFree(d_out);
+    if (e == cudaSuccess) e = cudaMemcpy(&r, d_out.data(), sizeof(r), cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) return e;
     *mag = r.mag; *phase = r.phase;
     if (avg_power) *avg_power = r.avg_power;
