@@ -123,7 +123,8 @@ typedef struct {
     uint32_t fused_front;           /* 1 when the fused convert+mix+resample kernel is in use */
     uint32_t kernel_launches;       /* kernels launched by the last process call */
     uint32_t halo_frames;           /* raw-input halo the fused front re-reads per train */
-    uint32_t reserved;
+    uint32_t polyphase_variant;     /* outputs per lane of the fused front's polyphase stage in its last launch (1, 2
+                                       or 4; 0 before the fused front has run) */
 } iqgpu_chain_info;
 
 typedef struct iqgpu_chain iqgpu_chain;
@@ -236,7 +237,13 @@ int  iqgpu_chain_get_arb_taps(iqgpu_chain *c, float *taps, uint32_t capacity, ui
  *      pre-resample FFT filter (interpolating or no_resample chains) is refused.  The RMS AGC
  *      starts from its reset state; iqgpu_chain_agc_rms_resume_device hands the state over.
  *      The halo covers the resampler's history, a FIR's taps, two FFT blocks (2n / ratio frames)
- *      and 16 time constants of the DC blocker (the only approximate term). ------------------- */
+ *      and 16 time constants of the DC blocker (the only approximate term).
+ *      Stream positions are limited to IQGPU_MAX_STREAM_POSITION (2^62) input frames, and the
+ *      resampled output index to the same bound (an interpolating chain reaches it first): a seek
+ *      to first_frame >= 2^62, or one whose output index would pass it, and a process call or an
+ *      iqgpu_chain_agc_advance_device range that would carry either past it are refused with
+ *      IQGPU_EINVAL before any work is queued. -------------------------------------------------- */
+#define IQGPU_MAX_STREAM_POSITION (1ull << 62)
 int  iqgpu_chain_seek(iqgpu_chain *c, uint64_t first_frame, uint64_t *out_first_frame);
 int  iqgpu_chain_halo_frames(iqgpu_chain *c, size_t *halo_frames);
 /* closed form: chain output frames after `frames_in` input frames since a restart — the resampler's

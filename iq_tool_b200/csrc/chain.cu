@@ -1271,6 +1271,7 @@ int iqgpu_chain_get_info(iqgpu_chain* c, iqgpu_chain_info* o)
     o->frames_in_total = c->n_in;
     o->frames_out_total = c->n_out;
     o->fused_front = c->fused_used ? 1 : 0;
+    o->polyphase_variant = c->fused ? fused_polyphase_variant(c->fused.get()) : 0;
     o->kernel_launches = c->launches;
     o->halo_frames = c->fused ? fused_halo_frames(c->fused.get()) : (uint32_t)c->rs.halo_input_frames;
     if (!c->plan_only && c->d_agc.data()) {
@@ -1283,6 +1284,19 @@ int iqgpu_chain_get_info(iqgpu_chain* c, iqgpu_chain_info* o)
         }
     }
     return IQGPU_OK;
+}
+
+// the supported stream range (include/iqgpu.h): `n_frames` more frames from the chain's position keep the input position
+// and the resampled output index within IQGPU_MAX_STREAM_POSITION
+static int check_stream_range(const iqgpu_chain* c, uint64_t from, uint64_t n_frames)
+{
+    const uint64_t lim = IQGPU_MAX_STREAM_POSITION;
+    bool ok = from <= lim && n_frames <= lim - from;
+    if (ok && !c->rs.passthrough && c->rs.is_interp)
+        ok = arb_outputs_after(from + n_frames, c->rs.step) <= (lim >> c->rs.num_halfband);
+    if (ok) return IQGPU_OK;
+    return fail(IQGPU_EINVAL, "stream position beyond IQGPU_MAX_STREAM_POSITION (2^62 input frames or output frames): from " +
+                                  std::to_string(from) + ", " + std::to_string(n_frames) + " frames");
 }
 
 static int build_chunks(iqgpu_chain* c, size_t n_frames, const uint32_t* chunk_frames, size_t n_chunks,
@@ -1341,6 +1355,7 @@ int iqgpu_chain_process_device(iqgpu_chain* c, const void* dev_raw_in, size_t n_
     if (c->plan_only) return fail(IQGPU_ENODEVICE, "chain was created without a device (plan only)");
     *out_frames = 0;
     if (n_frames == 0) return IQGPU_OK;
+    { int rc_r = check_stream_range(c, c->n_in, n_frames); if (rc_r) return rc_r; }
     if (!dev_raw_in || !dev_out) return fail(IQGPU_EINVAL, "null buffer");
     CK(cudaSetDevice(c->device));
     int rc = c->ensure_buffers();
@@ -1420,6 +1435,7 @@ int iqgpu_chain_process_device_begin(iqgpu_chain* c, const void* dev_raw_in, siz
     if (c->plan_only) return fail(IQGPU_ENODEVICE, "chain was created without a device (plan only)");
     if (n_frames == 0 || !dev_raw_in) return fail(IQGPU_EINVAL, "empty input");
     if (c->pend.active) return fail(IQGPU_EINVAL, "a begun call is still pending (call process_device_finish)");
+    { int rc_r = check_stream_range(c, c->n_in, n_frames); if (rc_r) return rc_r; }
     CK(cudaSetDevice(c->device));
     int rc = c->ensure_buffers();
     if (rc) return rc;
@@ -1483,6 +1499,7 @@ int iqgpu_chain_agc_advance_device(iqgpu_chain* c, const float* dev_peaks, uint6
     if (!c) return fail(IQGPU_EINVAL, "null argument");
     if (c->plan_only) return fail(IQGPU_ENODEVICE, "plan-only chain");
     if (c->agc_mode != 1) return fail(IQGPU_EINVAL, "the chain has no digital AGC");
+    { int rc_r = check_stream_range(c, first_frame, n_frames); if (rc_r) return rc_r; }
     if (n_frames == 0) return IQGPU_OK;
     if (!dev_peaks) return fail(IQGPU_EINVAL, "null buffer");
     if (first_frame % c->chunk_frames) return fail(IQGPU_EINVAL, "first_frame must be chunk aligned");
@@ -1717,6 +1734,7 @@ int iqgpu_chain_process_multi(iqgpu_chain* const* chains, size_t K, const void* 
         if (c->cfg.input_rate_hz != c0->cfg.input_rate_hz) return bad(k, "input_rate_hz differs from channel 0's");
         if (!chunk_frames && c->chunk_frames != c0->chunk_frames) return bad(k, "chunk_frames option differs from channel 0's");
         if (c->pend.active) return bad(k, "a begun process_device call is still pending (call process_device_finish)");
+        if (check_stream_range(c, c->n_in, n_frames)) return bad(k, iqgpu_last_error());
     }
     for (size_t k = 0; k < K; k++)
         if (chains[k]->plan_only) return fail(IQGPU_ENODEVICE, "chain was created without a device (plan only)");
@@ -1868,6 +1886,7 @@ int iqgpu_chain_outputs_after(iqgpu_chain* c, uint64_t frames_in, uint64_t* fram
 int iqgpu_chain_seek(iqgpu_chain* c, uint64_t first_frame, uint64_t* out_first_frame)
 {
     if (!c) return fail(IQGPU_EINVAL, "null chain");
+    { int rc_r = check_stream_range(c, first_frame, 1); if (rc_r) return rc_r; }
     if (filter_is_fft(c->filt) && !c->filt.post_resample)
         return fail(IQGPU_EINVAL, "seek is not supported with a pre-resample FFT filter: its blocks are cut from the input "
                                   "stream behind the remainder that filter_reset carries into the next stream (F5), a "

@@ -233,15 +233,16 @@ __device__ __forceinline__ f32x2_t add2(f32x2_t a, f32x2_t b)
 // h * {x.re, x.im} + {acc.re, acc.im}
 __device__ __forceinline__ f32x2_t fma2s(float h, f32x2_t x, f32x2_t acc) { return fma2(pk2(h, h), x, acc); }
 
-// The closed-form DC term of the warp-streaming front for output sample `o` (absolute index), which belongs to stretch
-// w = (nk - B0) / L_full (nk = the input frame its polyphase window ends at).  ONE definition, used by the in-memory pass
-// (w2_dc_correct_kernel) and by consumers that add the term while they load the stream (fir_param_kernel): same bits.
-__device__ __forceinline__ long long dc_fold_frame(unsigned long long o, uint32_t step, int S)
+// The closed-form DC term of the warp-streaming front for output sample `o` (absolute index, o >= g.O0), which belongs to
+// stretch w = (nk - B0) / L_full (nk = the input frame its polyphase window ends at).  ONE definition, used by the in-memory
+// pass (w2_dc_correct_kernel) and by consumers that add the term while they load the stream (fir_param_kernel): same bits.
+// Dp = o * step - g.pos.p_base (mod 2^64, ArbBase): exact, where o * step itself wraps from input frame 2^(40+S) on.
+__device__ __forceinline__ long long dc_fold_frame(unsigned long long Dp, const W2DcGeom& g, int S)
 {
-    return (long long)(((unsigned long long)o * step) >> 24) << S;
+    return (g.pos.k_base + (long long)(Dp >> 24)) << S;
 }
-// Pp = o * step (the caller may carry it from sample to sample), since = nk - (first frame of stretch w's warm-up): below
-// 2^31 for any stretch a launch can make (fused_launch_v2 checks)
+// Pp = o * step, or o * step - p_base (the caller may carry it from sample to sample; the row bits are the same),
+// since = nk - (first frame of stretch w's warm-up): below 2^31 for any stretch a launch can make (fused_launch_v2 checks)
 __device__ __forceinline__ float2 dc_fold_add_at(float2 v, unsigned long long Pp, int since, float lnc, const W2DcCorr& c,
                                                  const float* __restrict__ sG)
 {
@@ -252,10 +253,10 @@ __device__ __forceinline__ float2 dc_fold_add_at(float2 v, unsigned long long Pp
     v.y = fmaf(c.c_out.y, e, v.y);
     return v;
 }
-__device__ __forceinline__ float2 dc_fold_add(float2 v, unsigned long long o, uint32_t step, long long nk, long long w,
+__device__ __forceinline__ float2 dc_fold_add(float2 v, unsigned long long Dp, long long nk, long long w,
                                               const W2DcGeom& g, float lnc, const W2DcCorr& c, const float* __restrict__ sG)
 {
-    return dc_fold_add_at(v, o * step, (int)(nk - (g.B0 + w * g.L_full - g.warm_frames)), lnc, c, sG);
+    return dc_fold_add_at(v, Dp, (int)(nk - (g.B0 + w * g.L_full - g.warm_frames)), lnc, c, sG);
 }
 
 }  // namespace iqgpu

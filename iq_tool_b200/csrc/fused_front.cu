@@ -60,6 +60,7 @@ struct FusedFront {
     // faster depends on the rate of the arbitrary stage (bank conflicts of the window loads), so the first launch that is
     // large enough times both on its own data — the kernel is idempotent — and the choice sticks.
     int arb_pairs = -1;
+    int last_pairs = -1;                // the variant the last launch ran
     uint32_t lut_dtheta = 0;            // NCO table swizzle chosen for this phase increment
     unsigned lut_sh = 4, lut_mask = 0, lut_rot_sh = 4, lut_rot_c = 0;
     bool lut_picked = false;
@@ -217,6 +218,11 @@ uint32_t fused_halo_frames(const FusedFront* f)
 // DC blocker state v just before absolute frame `pos` of the sub-train that fused_launch() last ran from frame n0 with table
 // slot `slot` (device pointer into the tick table), or nullptr when the launch kept no table entry for that frame (local DC
 // state, frame not on a tick boundary)
+uint32_t fused_polyphase_variant(const FusedFront* f)
+{
+    return f->last_pairs < 0 ? 0u : (f->last_pairs == 2 ? 4u : (uint32_t)f->last_pairs + 1u);
+}
+
 const double2* fused_dc_state_at(const FusedFront* f, int slot, int64_t n0, int64_t pos)
 {
     if (slot < 0 || slot > 1 || !f->d_dc_table[slot].data() || pos < n0) return nullptr;
@@ -346,6 +352,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     A.bank_image = f->d_bank_image.data();
     A.O0 = O0; A.O1 = O0 + (long long)n_out; A.y = y;
     A.step = f->v2_step; A.zeta = f->v2_zeta;
+    A.arb_pos = arb_base((unsigned long long)O0, f->v2_step);
     A.lut_sh = 4; A.lut_mask = 0;
     A.arb_skew_sh = 31;
     if (pre.nco_enable) {
@@ -408,6 +415,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
         geo.warm_frames = (long long)f->v2_warm_sup * sup_frames;
         geo.pad_frames = (A.sup_last + 1) * sup_frames - A.N1;
         geo.lnc = A.dc_lnc; geo.alpha = (double)pre.dc_a; geo.atot = f->dc_atot;
+        geo.O0 = A.O0; geo.pos = A.arb_pos;
     } else if (pre.dc_enable) {
         if (!f->dc_ready[dc_slot]) {
             e = fused_dc_prepass(f, dc_slot, raw, n0, A.N1, pre, d_dc_carry, A.A0, st);
@@ -435,6 +443,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
     A.arb_tz = f->arb_tz; A.arb_b2 = f->arb_b2; A.arb_b3 = f->arb_b3;
     auto set_mode = [&](int m) {
         A.arb_pairs = m;
+        f->last_pairs = m;
         A.bank_image = (m == 2) ? f->d_bank_image_q.data() : f->d_bank_image.data();
         A.arb_skew_sh = (m == 2) ? f->arb_skew_sh : 31;
     };
@@ -477,7 +486,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
         w2_dc_scan_kernel<<<1, 1024, 0, st>>>(f->d_dc_stretch.data(), geo, f->d_dc_corr.data(), d_dc_carry);
         // a consumer that adds the term to the resampled stream itself leaves only the cf32 tail to this pass
         const long long O1c = fold ? A.O0 : A.O1;
-        if (fold) *fold = DcFold{f->d_dc_corr.data(), f->d_dc_G.data(), geo, A.O0, A.step, f->v2_S};
+        if (fold) *fold = DcFold{f->d_dc_corr.data(), f->d_dc_G.data(), geo, A.step, f->v2_S};
         const long long work = (O1c - A.O0) + f->H_tail;
         const int cgrid = (int)std::min<long long>((work + 255) / 256, 148LL * 16);
         w2_dc_correct_kernel<<<std::max(cgrid, 1), 256, 0, st>>>(y, A.O0, O1c, A.step, f->v2_S, geo, f->d_dc_corr.data(),
@@ -494,7 +503,7 @@ cudaError_t fused_launch(FusedFront* f, const void* raw, int64_t n0, size_t n, c
 cudaError_t fused_dc_correct_range(const DcFold& fold, float2* y, size_t first, size_t count, cudaStream_t st)
 {
     if (!fold.corr || count == 0) return cudaSuccess;
-    const long long Oa = fold.O0 + (long long)first;
+    const long long Oa = fold.geo.O0 + (long long)first;
     const int cgrid = (int)std::min<size_t>((count + 255) / 256, (size_t)148 * 16);
     w2_dc_correct_kernel<<<std::max(cgrid, 1), 256, 0, st>>>(y + first, Oa, Oa + (long long)count, fold.step, fold.S, fold.geo,
                                                            fold.corr, fold.G, nullptr, 0, 0, 0);

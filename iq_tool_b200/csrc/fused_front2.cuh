@@ -235,6 +235,7 @@ struct Fused2Args {
     double dc_c512, dc_lnc;             // c^512 and ln c in double (c = the float pole)
     const float2* bank_image;           // device, W2_BANK_F2 float2 in the w2_bank_row layout
     long long O0, O1;
+    ArbBase arb_pos;                    // polyphase position of O0 (kernels.hpp): k and row of every output o >= O0
     float2* y;
     long long sup_first, sup_last;      // absolute super-tick range of the call
     int sup_per_warp, warm_sup;
@@ -940,10 +941,12 @@ __device__ __forceinline__ void w2_arb_quad(const Fused2Args& A, const float2* _
     const unsigned tz = (unsigned)A.arb_tz;
     const float* __restrict__ bank = reinterpret_cast<const float*>(sbank);
     constexpr int NU = 15 + B3;                         // window entries: output 3 reaches index B3 + 1 + 13
+    const long long kA_rel = kA - A.arb_pos.k_base;
     for (long long o = oa + 4 * lane; o < ob; o += 128) {
-        const unsigned long long P0 = (unsigned long long)o * step, P1 = P0 + step, P2 = P1 + step, P3 = P2 + step;
+        // relative to the launch's base (ArbBase): P0..P3 never wrap, so the steps e1..e3 are right wherever o * step would
+        const unsigned long long P0 = (unsigned long long)o * step - A.arb_pos.p_base, P1 = P0 + step, P2 = P1 + step, P3 = P2 + step;
         const long long k0 = (long long)(P0 >> 24);
-        const int rel = (int)(k0 - kA);
+        const int rel = (int)(k0 - kA_rel);
         const bool e1 = ((long long)(P1 >> 24) - k0) != 1;
         const bool e2 = ((long long)(P2 >> 24) - k0) != B2;
         const bool e3 = ((long long)(P3 >> 24) - k0) != B3;
@@ -1007,8 +1010,9 @@ __device__ __forceinline__ void w2_arb(const Fused2Args& A, const float2* __rest
     using P = W2Plan<S>;
     const unsigned long long step = A.step;
     const unsigned long long kb = (unsigned long long)kA + P::flat_new;
-    // outputs of this run: o >= o_cur with o*step < kb << 24
-    const unsigned long long Dn = (kb << 24) - (unsigned long long)o_cur * step;      // in (0, (flat_new+2) << 24]
+    // outputs of this run: o >= o_cur with o*step < kb << 24.  Both products may wrap mod 2^64; their true difference lies
+    // in (0, (flat_new+2) << 24], so the difference mod 2^64 is exact.
+    const unsigned long long Dn = (kb << 24) - (unsigned long long)o_cur * step;
     // cnt = ceil(Dn / step): float estimate of the quotient (Dn < 2^34, step in [2^24, 2^25]: off by at most one),
     // then an exact remainder fix-up without loops
     unsigned cnt = (unsigned)__fdividef((float)Dn, (float)step);
@@ -1030,10 +1034,13 @@ __device__ __forceinline__ void w2_arb(const Fused2Args& A, const float2* __rest
         }
         return;
     }
+    // o * step relative to the launch's base (ArbBase, o >= oa >= O0): exact k and row at any stream position
+    const long long kA_rel = kA - A.arb_pos.k_base;
+    const unsigned long long p_base = A.arb_pos.p_base;
     if (!A.arb_pairs) {
     for (long long o = oa + lane; o < ob; o += 32) {
-        const unsigned long long Pp = (unsigned long long)o * step;
-        const int rel = (int)((long long)(Pp >> 24) - kA);
+        const unsigned long long Pp = (unsigned long long)o * step - p_base;
+        const int rel = (int)((long long)(Pp >> 24) - kA_rel);
         const unsigned idx = (unsigned)(Pp >> 16) & 0xffu;
         const float2* __restrict__ w = flat + rel + (W2_ARB_HIST - 13);
         const float2* __restrict__ b = sbank + w2_bank_row((int)idx);
@@ -1055,8 +1062,8 @@ __device__ __forceinline__ void w2_arb(const Fused2Args& A, const float2* __rest
     // which lines its taps up with the shared window: taps that fall outside the row are exact zeros, the order of the
     // non-zero terms is that of a single output, hence the same bits.
     for (long long o = oa + 2 * lane; o < ob; o += 64) {
-        const unsigned long long P0 = (unsigned long long)o * step, P1 = P0 + step;
-        const int rel = (int)((long long)(P0 >> 24) - kA);
+        const unsigned long long P0 = (unsigned long long)o * step - p_base, P1 = P0 + step;
+        const int rel = (int)((long long)(P0 >> 24) - kA_rel);
         const int d = (int)((P1 >> 24) - (P0 >> 24));
         const f32x2_t* __restrict__ w = reinterpret_cast<const f32x2_t*>(flat + rel + (W2_ARB_HIST - 13));
         const float2* __restrict__ b0 = sbank + w2_bank_row((int)((unsigned)(P0 >> 16) & 0xffu));
@@ -1148,11 +1155,14 @@ __global__ void __launch_bounds__(W2_MAX_WARPS * 32, 1) fused_front2_kernel(cons
     float2* flat = wsm + P::flat_off;
 
     const long long t_begin = (seg_first - A.warm_sup) * P::sup, t_emit = seg_first * P::sup, t_end = (seg_last + 1) * P::sup;
-    // first output of the first emitting run (exact), carried from run to run afterwards
+    // first output of the first emitting run, o_cur = ceil(k_emit 2^24 / step), carried from run to run afterwards; as an
+    // offset from O0: D = k_emit 2^24 - O0 step = (k_emit - k_base) 2^24 - (O0 step mod 2^24), within the call (any sign)
     long long o_cur;
     {
-        const unsigned long long k_emit = (unsigned long long)((t_emit * W2_T0) >> S);
-        o_cur = (long long)(((k_emit << 24) + A.step - 1) / A.step);
+        const long long k_emit = (t_emit * W2_T0) >> S;
+        const long long step = (long long)A.step;
+        const long long D = ((k_emit - A.arb_pos.k_base) << 24) - (long long)(((unsigned long long)A.O0 * A.step) & 0xffffffull);
+        o_cur = A.O0 + (D >= 0 ? (D + step - 1) / step : -((-D) / step));
     }
     double2 vloc = make_double2(0.0, 0.0);
     if (DC == 2 && gw == 0) {
@@ -1340,10 +1350,11 @@ __global__ void __launch_bounds__(256) w2_dc_correct_kernel(float2* __restrict__
     const long long n_tail = (N1 > t_lo) ? (N1 - t_lo) : 0;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_out + n_tail; i += stride) {
         if (i < n_out) {
-            const long long nk = dc_fold_frame((unsigned long long)(O0 + i), step, S);
+            const unsigned long long Dp = (unsigned long long)(O0 + i) * step - g.pos.p_base;
+            const long long nk = dc_fold_frame(Dp, g, S);
             const long long w = (nk - g.B0) / g.L_full;
             if (w <= 0) continue;
-            y[i] = dc_fold_add(y[i], (unsigned long long)(O0 + i), step, nk, w, g, lnc, corr[w], sG);
+            y[i] = dc_fold_add(y[i], Dp, nk, w, g, lnc, corr[w], sG);
         } else {
             const long long n = t_lo + (i - n_out);
             const long long w = (n - g.B0) / g.L_full;

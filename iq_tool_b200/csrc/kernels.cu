@@ -671,13 +671,14 @@ __global__ void __launch_bounds__(FIR_THREADS) fir_param_kernel(const float2* __
         // and first warm-up frame; all 64-bit work happens once per thread and tile
         long long w = -1, w_end = 0, w_from = 0;
         W2DcCorr cw{};
-        unsigned long long Pp = FOLD ? (unsigned long long)(F.O0 + wbase + t) * F.step : 0ull;
+        // (relative to the launch's polyphase base, ArbBase: exact for the samples g >= 0 the fold touches)
+        unsigned long long Pp = FOLD ? (unsigned long long)(F.geo.O0 + wbase + t) * F.step - F.geo.pos.p_base : 0ull;
         const unsigned long long dPp = (unsigned long long)FIR_THREADS * F.step;
         for (int j = t; j < FIR_TILE + tc - 1; j += FIR_THREADS, Pp += dPp) {
             const long long g = wbase + j;
             f32x2_t v = (g < (long long)n) ? *reinterpret_cast<const f32x2_t*>(x + g) : 0ull;
             if (FOLD && g >= 0 && g < (long long)n) {
-                const long long nk = (long long)(Pp >> 24) << F.S;
+                const long long nk = dc_fold_frame(Pp, F.geo, F.S);
                 if (w < 0 || nk >= w_end) {
                     if (w < 0) { w = (nk - F.geo.B0) / F.geo.L_full; w_end = F.geo.B0 + (w + 1) * F.geo.L_full; }
                     while (nk >= w_end) { w++; w_end += F.geo.L_full; }

@@ -173,18 +173,32 @@ struct ResamplerDesc {
 };
 // Local DC state of the warp-streaming front (fused_front2.cuh): every warp ran its stretch of the stream from v = 0, the
 // term it could not know is a decaying exponential per stretch that is added afterwards in closed form.
+// Polyphase position of the outputs o >= o_base of one launch.  P(o) = o * step needs up to 87 bits (positions below 2^62),
+// k(o) = P >> 24 is the input sample the window ends at, (P >> 16) & 255 the bank row.  With p_base = o_base * step mod 2^64
+// rounded down to a multiple of 2^24, D = o * step - p_base (mod 2^64) equals P(o) - k_base * 2^24 exactly while
+// (o - o_base) * step stays below 2^63 (any launch), so k(o) = k_base + (D >> 24) and the row is (D >> 16) & 255.
+struct ArbBase {
+    long long k_base;
+    unsigned long long p_base;
+};
+inline ArbBase arb_base(unsigned long long o_base, uint32_t step)
+{
+    const unsigned __int128 P = (unsigned __int128)o_base * step;
+    return ArbBase{(long long)(P >> 24), (unsigned long long)P & ~0xffffffull};
+}
 struct W2DcCorr { float2 c_out, c_pre; };      // -a V0 Atot (cascade output) and -a V0 (cascade input, for the cf32 tail)
 struct W2DcGeom {
     int n_stretch;
     long long B0, L_full, L_last, warm_frames, pad_frames;     // pad: zero frames between N1 and the end of the last tick
     double lnc, alpha, atot;
+    long long O0;              // first output of the launch and its polyphase position
+    ArbBase pos;
 };
 // what a consumer of the resampled stream needs to add that term itself to sample i (absolute output index O0 + i)
 struct DcFold {
     const W2DcCorr* corr;      // device: one record per stretch
     const float* G;            // device: 256 polyphase row gains
-    W2DcGeom geo;
-    long long O0;
+    W2DcGeom geo;              // geo.O0: the launch's first output
     uint32_t step;
     int S;
 };
@@ -194,6 +208,8 @@ FusedFront* fused_create(int format, const ResamplerDesc& r, bool nco, const flo
 void fused_destroy(FusedFront* f);
 cudaError_t fused_reset(FusedFront* f, cudaStream_t st);
 uint32_t fused_halo_frames(const FusedFront* f);
+// outputs per lane of the polyphase variant the last launch ran (1, 2 or 4; 0 before the first launch)
+uint32_t fused_polyphase_variant(const FusedFront* f);
 const double2* fused_dc_state_at(const FusedFront* f, int slot, int64_t n0, int64_t pos);
 // raw[0] has absolute index n0; produces outputs [O0, O0+n_out) into y; d_dc_carry is the DC state at n0
 // (updated to the state at n0+n).  *launches is incremented by the kernels launched.

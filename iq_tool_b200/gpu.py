@@ -34,7 +34,7 @@ class ChainInfoC(C.Structure):
         ("agc_gain", C.c_float), ("agc_peak_memory", C.c_float), ("agc_samples_seen", C.c_uint64),
         ("frames_in_total", C.c_uint64), ("frames_out_total", C.c_uint64),
         ("fused_front", C.c_uint32), ("kernel_launches", C.c_uint32), ("halo_frames", C.c_uint32),
-        ("reserved", C.c_uint32),
+        ("polyphase_variant", C.c_uint32),
     ]
 
 
